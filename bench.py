@@ -4,6 +4,7 @@
 Contract (see DESIGN.md "Measurement"):
   python bench.py --gpus N --steps K --warmup W            our arm (libxsparse_b200 through the C ABI)
   python bench.py --impl reference --gpus N ...            the reference's CPU algorithm (oracle port)
+  python bench.py --gpus 1 ... --dump-outputs DIR          also writes the CSC of the last timed step to DIR/*.npy
 
 A step = one full assembly of the workload: reset!, insertion of the whole (i,j,v) stream,
 flush! into a fresh CSC.  N=1 workload: BASELINE.json configs[1], the 3-D P1-FEM Laplacian on
@@ -219,6 +220,41 @@ def csc_digest(colptr, rowval, nzval):
     return hsh.hexdigest()
 
 
+DUMP_SAMPLE = 1 << 20  # rowval / nzval positions --dump-outputs keeps: 3 x 8 MiB beside the 16 MiB colptr of 128^3
+
+
+def fetch_csc_device(h, torch):
+    """The handle's CSC (colptr, rowval, nzval) copied into new tensors on the current CUDA device."""
+    nnz = h.nnz
+    cp = torch.empty(h.n + 1, dtype=torch.int64, device="cuda")
+    rv = torch.empty(nnz, dtype=torch.int64, device="cuda")
+    nz = torch.empty(nnz, dtype=torch.float64, device="cuda")
+    h.fetch_csc(cp, rv if nnz else None, nz if nnz else None)
+    h.synchronize()
+    return cp, rv, nz
+
+
+def csc_outputs(colptr, rowval, nzval, torch):
+    """What --dump-outputs writes of a CSC: colptr whole, rowval and nzval at DUMP_SAMPLE positions drawn with a
+    fixed seed (the same positions for the same nnz, listed in sample_index), all as float64, which holds every
+    index below 2^53 exactly."""
+    import numpy as np
+
+    nnz = rowval.numel()
+    pos = np.sort(np.random.default_rng(0).choice(nnz, min(nnz, DUMP_SAMPLE), replace=False))
+    at = torch.from_numpy(pos).to(rowval.device)
+    arrays = {"colptr": colptr, "sample_index": at, "rowval_sample": rowval[at], "nzval_sample": nzval[at]}
+    return {name: a.to(torch.float64).cpu().numpy() for name, a in arrays.items()}
+
+
+def write_outputs(path, arrays):
+    import numpy as np
+
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def host_threads():
     """Host threads the CPU legs may use: the cores this process is allowed on, capped at 64
     (every partition of the MT path owns a dense column map)."""
@@ -392,10 +428,15 @@ def run_ours(args):
     with ClockSampler(local) as clk:
         ms_step = timed_steps(h, step, args.steps)
         launches_timed = h.kernel_launches - launches0
+        # the result of the last timed step, taken before the untimed steps below can replace it
+        last = fetch_csc_device(h, torch) if args.dump_outputs else None
         # keep the sampler alive for at least a few samples on very short runs
         t_end = time.time() + max(0.0, 0.5 - ms_step * args.steps / 1e3)
         while time.time() < t_end:
             step()
+    if last is not None:
+        write_outputs(args.dump_outputs, csc_outputs(*last, torch))
+        del last
     nnz = h.nnz
     value = n_ins / (ms_step / 1e3)
     peak, peak_src = peaks()
@@ -774,8 +815,14 @@ def main():
                     help="N>1 only: fem = weak scaling of configs[1] (default, the bench line); fd400 = configs[4], "
                          "fdrand 400^3 sharded by node slab over the ranks (strong scaling, no e2e leg)")
     ap.add_argument("--fd-n", type=int, default=400, help="grid points per direction of --workload fd400")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="one GPU: write the CSC of the last timed step to DIR/*.npy (float64; colptr whole, rowval and "
+                         "nzval at a fixed seeded sample of positions) to compare two builds output for output")
     args = ap.parse_args()
-    args.steps = max(1, args.steps)
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1):
+        ap.error("--dump-outputs needs the single-GPU arm (--impl ours --gpus 1)")
     args.warmup = max(3, args.warmup) if args.impl == "ours" else max(0, args.warmup)
     if args.impl == "reference":
         run_reference(args)
