@@ -22,7 +22,7 @@ TRIPLET_DTYPE = np.dtype([("row", "<u4"), ("col", "<u4"), ("val", "<f8")])
 assert TRIPLET_DTYPE.itemsize == 16
 DETERMINISTIC, FAST = 0, 1
 COMBINE_SEED, COMBINE_ADD = 0, 1
-STRATEGY_AUTO, STRATEGY_FULLSORT, STRATEGY_COLSORT = 0, 1, 2
+STRATEGY_AUTO, STRATEGY_FULLSORT = 0, 1
 GROUPING_AUTO, GROUPING_OFF, GROUPING_ON = 0, 1, 2
 
 
@@ -134,9 +134,6 @@ SIGNATURES = {
     "xsb_stream_count_p1fem": (_i32, [_i64, _i64, _i64, C.POINTER(_i64)]),
     "xsb_stream_count_blockrd": (_i32, [_i64, _i64, _i64, _i32, C.POINTER(_i64)]),
     "xsb_debug_fetch_staged": (_i32, [_p, _i32, _p, _p, _p, _p, _i64, C.POINTER(_i64)]),
-    "xsb_debug_set_sort_variant": (_i32, [_i32]),
-    "xsb_debug_sort_selftest": (_i32, [_p, _i64, _i32, _i32, _i32, C.POINTER(C.c_float), C.POINTER(C.c_float),
-                                       C.POINTER(_i64), C.POINTER(_i32)]),
     "xsb_synchronize": (_i32, [_p]),
     "xsb_get_stream": (_i32, [_p, C.POINTER(_p)]),
     "xsb_timer_start": (_i32, [_p]),
@@ -240,11 +237,6 @@ class Handle:
             n = int(splits[rank + 1]) - int(splits[rank])
             self.n_ranks, self.rank = n_ranks, rank
         self._h = h
-        strat = os.environ.get("XSB_STRATEGY", "").lower()  # test/bench switch
-        if os.environ.get("XSB_GROUPING", "").lower() in ("off", "on"):
-            check(lib().xsb_set_grouping(h, GROUPING_OFF if os.environ["XSB_GROUPING"].lower() == "off" else GROUPING_ON), h)
-        if strat in ("fullsort", "colsort"):
-            check(lib().xsb_set_strategy(h, STRATEGY_FULLSORT if strat == "fullsort" else STRATEGY_COLSORT), h)
         self.m, self.n = int(m), int(n)
         self.idx_type, self.index_base, self.n_tid, self.device = idx_type, index_base, n_tid, device
         self.idx_dtype = np.int64 if idx_type == I64 else np.int32
@@ -484,12 +476,6 @@ class Handle:
             self._c(lib().xsb_debug_fetch_staged(self._h, tid, ptr(I), ptr(J), ptr(V), ptr(F), n, C.byref(c)))
         return I, J, V, F
 
-    def sort_selftest(self, n, nbits, variant=0, reps=3):
-        mh, mp, v, npass = C.c_float(0), C.c_float(0), _i64(0), _i32(0)
-        self._c(lib().xsb_debug_sort_selftest(self._h, n, nbits, variant, reps, C.byref(mh), C.byref(mp), C.byref(v),
-                                              C.byref(npass)))
-        return {"ms_histogram": mh.value, "ms_per_pass": mp.value, "violations": v.value, "passes": npass.value}
-
     def synchronize(self):
         self._c(lib().xsb_synchronize(self._h))
 
@@ -513,14 +499,14 @@ class Handle:
         self._c(lib().xsb_set_grouping(self._h, int(grouping)))
 
     def set_precount(self, on=True):
-        """Counting at insertion (default on): pack / emit kernels also take the grouping's per-chunk column histograms."""
+        """Grouping at insertion (default on): pack / emit kernels bring every chunk into column order and publish its runs."""
         self._c(lib().xsb_set_precount(self._h, 1 if on else 0))
 
     def set_preaggregation(self, on=True):
         self._c(lib().xsb_set_preaggregation(self._h, 1 if on else 0))
 
     def set_strategy(self, strategy):
-        """STRATEGY_AUTO (column sort + in-tile row ordering) or STRATEGY_FULLSORT ((col,row) sort)."""
+        """STRATEGY_AUTO (records grouped by column, duplicates folded per column) or STRATEGY_FULLSORT ((col,row) sort)."""
         self._c(lib().xsb_set_strategy(self._h, int(strategy)))
 
     def set_profiling(self, on=True):

@@ -301,7 +301,6 @@ struct xsb_matrix
     int grouping_misses = 0;          // consecutive flushes whose stream had no column locality
     int runs_misses = 0;              // consecutive flushes whose columns were too long / rich for the thread-per-column merge
     i64 stats_pairs = 0;
-    bool last_column_path = false;
     bool no_direct_fold = false; // the one-pass fold met columns it cannot take: park + compact instead
     int stats_direct = 0;
     i64 stats_preagg = 0;
@@ -420,13 +419,6 @@ struct xsb_matrix
 };
 
 namespace {
-
-// XSB_PREAGG=1 turns window pre-aggregation on for every handle's XSB_FAST flushes (A-B measurements);
-// the regular switch is xsb_set_preaggregation
-const bool g_preagg = []() {
-    const char *e = getenv("XSB_PREAGG");
-    return e && *e == '1';
-}();
 
 void set_err(xsb_matrix *h, const std::string &s)
 {
@@ -593,9 +585,9 @@ void check_exchange(xsb_matrix *h)
 // resident CSC untouched (apart from the in-place grouping of chunks, which keeps every entry's insertions in
 // stream order) -- when this flush has to take another path: a stream without column locality, a column too long
 // or too rich for one thread.
-bool runs_flush(xsb_matrix *h, int32_t mode, i64 n_ins, StageTimer *tp, int64_t *nnz_out)
+// The fold is an exact left fold in insertion order, so both summation modes take it alike.
+bool runs_flush(xsb_matrix *h, StageTimer *tp, int64_t *nnz_out)
 {
-    (void)mode; // the fold is an exact left fold in insertion order in both modes
     cudaStream_t s = h->stream;
     Stage &st = h->stage[0];
     const i64 count = st.count;
@@ -736,7 +728,6 @@ bool runs_flush(xsb_matrix *h, int32_t mode, i64 n_ins, StageTimer *tp, int64_t 
     h->clear_staging(false);
     if (nnz_new != nnz_old)
         h->drop_frozen();
-    (void)n_ins;
     *nnz_out = nnz_new;
     return true;
 }
@@ -779,13 +770,12 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
     h->stats_direct = 0;
     h->stats_preagg = 0;
     h->stats_precounted = 0;
-    if (combine == XSB_COMBINE_SEED && !(mode == XSB_FAST && (h->preagg || g_preagg)))
+    if (combine == XSB_COMBINE_SEED && !(mode == XSB_FAST && h->preagg))
     { // ---- the product path: grouped chunks, records never move, resident CSC merged column by column
         int64_t nnz_runs = 0;
         const i64 foreign_runs = h->foreign + h->n_pad;
-        if (runs_flush(h, mode, n_ins, tp, &nnz_runs))
+        if (runs_flush(h, tp, &nnz_runs))
         {
-            h->last_column_path = true;
             h->stats.n_inserted = n_ins - foreign_runs;
             h->stats.nnz_old = nnz_old;
             h->stats.nnz_new = nnz_runs;
@@ -877,7 +867,7 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
     // ---- XSB_FAST: accumulate-on-insert inside windows of the staged stream (xsb_preagg.cu); the
     // partial sums replace the staged records, the old entries ride in front of them as before
     bool preagged = false;
-    if (mode == XSB_FAST && !h->has_assign && !h->fixed_exchange && combine == XSB_COMBINE_SEED && (h->preagg || g_preagg) && h->preagg_misses < 2 &&
+    if (mode == XSB_FAST && !h->has_assign && !h->fixed_exchange && combine == XSB_COMBINE_SEED && h->preagg && h->preagg_misses < 2 &&
         n_ins >= 4096)
     {
         if (tp)
@@ -899,8 +889,7 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
     KeyLayout Lf = h->L; // layout the fold sees: partial sums are not tied to a partition
     if (preagged)
         Lf.tidbits = 0;
-    const size_t ws_bytes = std::max(std::max(sort_workspace_bytes((u64)total), reduce_workspace_bytes((u64)total, h->n)),
-                                     column_workspace_bytes((u64)total, h->n));
+    const size_t ws_bytes = std::max(sort_workspace_bytes((u64)total), reduce_workspace_bytes((u64)total, h->n));
     void *ws = h->dalloc(ws_bytes);
     // slab handles: records owned (and already received) by other ranks are still in the buffer.  The
     // grouping kernels skip them by their owner bits; every other path first drops them with one
@@ -966,7 +955,7 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
     i64 nnz_new = -1;
     SortPlan plan{};
     int passes_run = 0;
-    int path = 0; // 0: (col,row) sort + flat reduction, 1: column sort + in-tile row ordering, 2: column sort + hash fold
+    int path = 0; // 0: (col,row) sort + flat reduction, 2: column sort + hash fold, 3: grouping + hash fold
     if (h->strategy == XSB_STRATEGY_AUTO && colfold_supported(h->L, (u64)total, h->n))
     {
         // ---- sort by column only; the per-column kernel folds duplicates through a hash table
@@ -981,9 +970,8 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
             colfold_lists(cws, (u64)total, h->n, &nzcol, &nzstart, &totals);
             int pair_passes = 0;
             u64 npairs = 0;
-            grouped = group_by_column(s, A, B, (u64)total, h->n, h->L, gws, ws, nzcol, nzstart, totals, h->h_scal + 4,
-                                      h->d_scal + 4, h->lc, tp, &pair_passes, &npairs,
-                                      tomb ? h->L.ownershift() : -1, (u32)h->rank, pord, nullptr);
+            grouped = group_by_column(s, A, B, (u64)total, h->n, h->L, gws, ws, nzcol, nzstart, totals, h->h_scal + 4, h->lc,
+                                      tp, &pair_passes, &npairs, tomb ? h->L.ownershift() : -1, (u32)h->rank, pord);
             h->dfree(gws);
             h->stats_pairs = (i64)npairs;
             if (grouped)
@@ -1041,55 +1029,25 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
             nnz_new = (i64)read_scalar(h, 0);
             if ((u32)h->h_scal[7])
                 h->fold_hint = (u32)h->h_scal[7]; // distinct rows per column: picks the next flush's table size
-        }
-        if (direct)
-        {
-        }
-        else if ((u32)h->h_scal[6] == 0u)
-        {
-            const size_t rv_bytes = (h->isz() * (size_t)nnz_new + 15) & ~(size_t)15;
-            new_store_bytes = rv_bytes + 8 * (size_t)nnz_new;
-            new_store = h->dalloc(new_store_bytes);
-            new_rowval = new_store;
-            new_nzval = reinterpret_cast<double *>(static_cast<unsigned char *>(new_store) + rv_bytes);
-            colfold_compact(s, spare, (u64)total, h->n, h->idx64, h->base, new_colptr, new_rowval, new_nzval, cws,
-                            h->lc, tp);
-            h->dfree(spare); // back to the buffer cache
-        }
-        else
-        { // a group of columns too rich for the in-warp table: finish with the general sort (records are intact)
-            A = sorted;
-            B = spare;
-            path = 0;
+            if ((u32)h->h_scal[6] == 0u)
+            {
+                const size_t rv_bytes = (h->isz() * (size_t)nnz_new + 15) & ~(size_t)15;
+                new_store_bytes = rv_bytes + 8 * (size_t)nnz_new;
+                new_store = h->dalloc(new_store_bytes);
+                new_rowval = new_store;
+                new_nzval = reinterpret_cast<double *>(static_cast<unsigned char *>(new_store) + rv_bytes);
+                colfold_compact(s, spare, (u64)total, h->n, h->idx64, h->base, new_colptr, new_rowval, new_nzval, cws,
+                                h->lc, tp);
+                h->dfree(spare); // back to the buffer cache
+            }
+            else
+            { // a group of columns too rich for the in-warp table: finish with the general sort (records are intact)
+                A = sorted;
+                B = spare;
+                path = 0;
+            }
         }
         h->dfree(cws);
-    }
-    else if (h->strategy == XSB_STRATEGY_COLSORT && column_path_supported(h->L))
-    {
-        drop_foreign();
-        // ---- sort by column only; rows are ordered inside the reduce kernel (bitonic, per column)
-        plan = make_sort_plan(h->L.low + h->L.rowbits, h->L.colbits);
-        sorted = radix_sort_records(s, A, B, (u64)total, plan, ws, h->lc, tp);
-        passes_run += plan.npasses;
-        spare = (sorted == A) ? B : A;
-        new_rowval = spare;
-        new_nzval = reinterpret_cast<double *>(reinterpret_cast<unsigned char *>(spare) + 8 * (size_t)total);
-        column_reduce_emit_csc(s, sorted, (u64)total, h->L, combine, !h->has_assign, h->n, h->idx64, h->base,
-                               new_rowval, new_nzval, new_colptr, ws, h->d_scal + 0,
-                               reinterpret_cast<u32 *>(h->d_scal + 6), h->lc, tp);
-        XSB_CUDA(cudaMemcpyAsync(h->h_scal + 6, h->d_scal + 6, sizeof(u64), cudaMemcpyDeviceToHost, s));
-        nnz_new = (i64)read_scalar(h, 0);
-        if ((u32)h->h_scal[6] == 0u)
-        {
-            path = 1;
-            new_store = spare;
-            new_store_bytes = sizeof(Rec) * (size_t)total;
-        }
-        else
-        { // a column too long for the in-warp path: finish with the general sort (records are intact)
-            A = sorted;
-            B = spare;
-        }
     }
     if (path == 0)
     {
@@ -1108,7 +1066,6 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
         new_store_bytes = sizeof(Rec) * (size_t)total;
     }
     const bool column_path = path != 0;
-    h->last_column_path = column_path;
 
     if (tp)
         tp->begin(s);
@@ -1211,21 +1168,10 @@ Rec *begin_emit(xsb_matrix *h, int32_t tid, int32_t flavour, i64 count)
     return st.buf + st.front + st.count;
 }
 
-// XSB_PRECOUNT=0 switches grouping at insertion off for every handle (A-B measurements): the flush then
-// groups the chunks itself; XSB_RUNS=0 switches the whole grouped-chunk flush off (previous product path)
-const bool g_precount_off = []() {
-    const char *e = getenv("XSB_PRECOUNT");
-    return e && *e == '0';
-}();
-const bool g_runs_off = []() {
-    const char *e = getenv("XSB_RUNS");
-    return e && *e == '0';
-}();
-
 // may this handle's flush work on grouped chunks (xsb_runs.cu)?
 bool runs_eligible(const xsb_matrix *h)
 {
-    return !g_runs_off && h->n_tid == 1 && h->strategy == XSB_STRATEGY_AUTO && h->grouping != XSB_GROUPING_OFF &&
+    return h->n_tid == 1 && h->strategy == XSB_STRATEGY_AUTO && h->grouping != XSB_GROUPING_OFF &&
            (h->grouping == XSB_GROUPING_ON || (h->grouping_misses < 2 && h->runs_misses < 2));
 }
 
@@ -1234,7 +1180,7 @@ bool runs_eligible(const xsb_matrix *h)
 // say where the runs go, the id of the first chunk and the position of the first record.
 bool runs_begin(xsb_matrix *h, int32_t tid, i64 count, u32 chunks, RunTarget *rt, u32 *chunk0, u32 *pos0)
 {
-    if (!h->precount || g_precount_off || tid != 0 || !runs_eligible(h) || count <= 0)
+    if (!h->precount || tid != 0 || !runs_eligible(h) || count <= 0)
         return false;
     Stage &st = h->stage[0];
     if (h->runs.dead || st.count != h->runs.sorted_end)
@@ -2721,27 +2667,6 @@ int32_t xsb_debug_fetch_staged(xsb_matrix *h, int32_t tid, void *I, void *J, voi
     });
 }
 
-int32_t xsb_debug_set_sort_variant(int32_t variant)
-{
-    set_sort_variant(variant);
-    return get_sort_variant() == variant ? XSB_OK : XSB_EINVAL;
-}
-
-int32_t xsb_debug_sort_selftest(xsb_matrix *h, int64_t n, int32_t nbits, int32_t variant, int32_t reps,
-                                float *ms_histogram, float *ms_per_pass, int64_t *violations, int32_t *npasses)
-{
-    return guard(h, [&]() -> int32_t {
-        REQUIRE(h && ms_histogram && ms_per_pass && violations && npasses, XSB_EINVAL, "NULL argument");
-        REQUIRE(n >= 2 && nbits >= 1 && nbits <= 64 && reps >= 1, XSB_EINVAL, "bad self-test size");
-        u64 viol = 0;
-        int np = 0;
-        sort_selftest(h->stream, (u64)n, nbits, variant, reps, ms_histogram, ms_per_pass, &viol, &np);
-        *violations = (int64_t)viol;
-        *npasses = np;
-        return XSB_OK;
-    });
-}
-
 int32_t xsb_synchronize(xsb_matrix *h)
 {
     return guard(h, [&]() -> int32_t {
@@ -2781,7 +2706,7 @@ int32_t xsb_timer_stop(xsb_matrix *h, float *ms_out)
 
 int32_t xsb_set_strategy(xsb_matrix *h, int32_t strategy)
 {
-    if (!h || strategy < XSB_STRATEGY_AUTO || strategy > XSB_STRATEGY_COLSORT)
+    if (!h || (strategy != XSB_STRATEGY_AUTO && strategy != XSB_STRATEGY_FULLSORT))
         return XSB_EINVAL;
     h->strategy = strategy;
     return XSB_OK;

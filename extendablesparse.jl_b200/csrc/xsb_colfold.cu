@@ -20,7 +20,6 @@
 // table raises an overflow flag; the caller then finishes with the general (col,row) sort.
 #include "xsb_fold.cuh"
 #include "xsb_internal.h"
-#include <cstdlib>
 
 namespace xsb {
 
@@ -1094,17 +1093,6 @@ compact_entries_kernel(const Rec *__restrict__ tmp, const u32 *__restrict__ nzco
 // host side
 // ------------------------------------------------------------------------
 namespace {
-int env_int(const char *name, int dflt)
-{
-    const char *e = getenv(name);
-    return e && *e ? atoi(e) : dflt;
-}
-// tuning knobs (debugging and the tile-shape sweeps of tools/): XSB_THREAD_FOLD=0 keeps every
-// column on the warp kernel, XSB_THREAD_HBITS=4|5|6 fixes the per-thread table size
-const int g_thread_fold = env_int("XSB_THREAD_FOLD", 1);
-const int g_thread_hbits = env_int("XSB_THREAD_HBITS", 0);
-const int g_direct_fold = env_int("XSB_DIRECT_FOLD", 1); // 0: always park the entries and compact them
-
 struct CtArgs
 {
     const Rec *sorted;
@@ -1232,7 +1220,7 @@ void launch_direct_t(cudaStream_t stream, unsigned blocks, const Rec *sorted, in
 
 bool colfold_direct_supported(const KeyLayout &L, int combine, bool plain_adds)
 {
-    return g_thread_fold && g_direct_fold && plain_adds && L.tidbits == 0 && combine == 0;
+    return plain_adds && L.tidbits == 0 && combine == 0;
 }
 
 // One-pass variant of the fold for plain += streams: records grouped by column -> final rowval / nzval /
@@ -1273,11 +1261,9 @@ void colfold_direct(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
     if (timer)
         timer->begin(stream);
     const u64 avg = nrec / std::max<u64>(1, kmax);
-    int level = hint_maxd ? (hint_maxd <= 12 ? 0 : (hint_maxd <= 24 ? 1 : 2)) : (avg < 14 ? 0 : (avg < 40 ? 1 : 2));
+    const int level = hint_maxd ? (hint_maxd <= 12 ? 0 : (hint_maxd <= 24 ? 1 : 2)) : (avg < 14 ? 0 : (avg < 40 ? 1 : 2));
     // 13..16 distinct rows in the previous flush (P1 FEM: 15): the 32-slot table with 16 accumulators
-    const bool slim = level == 1 && hint_maxd != 0 && hint_maxd <= 16 && g_thread_hbits == 0;
-    if (g_thread_hbits >= 4 && g_thread_hbits <= 6)
-        level = g_thread_hbits - 4;
+    const bool slim = level == 1 && hint_maxd != 0 && hint_maxd <= 16;
     const u32 maxlen = (u32)std::max<u64>(256, 6 * avg);
 #define XSB_DIRECT(HB, TI)                                                                                              \
     launch_direct_t<HB, TI>(stream, blocks, sorted, L.low, L.rowbits, maxlen, nzcol, nzstart, totals, ncols, base,      \
@@ -1357,7 +1343,7 @@ void colfold_reduce(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
     // Groups of short columns hold many distinct entries per record (little duplication), and the
     // in-register sort of the distinct entries grows faster than linearly: keep such groups small.
     const u32 chunk = (nrec / std::max<u64>(1, std::min<u64>((u64)ncols, nrec)) >= 48) ? (u32)CF_PIECE : 128u;
-    if (simple && g_thread_fold)
+    if (simple)
     { // one thread per column, smallest table first; what a size cannot take is handed to the next
       // one through a list, the rest (and the long columns) to the warp kernel
         u32 *listA = reinterpret_cast<u32 *>(ws + l.off_list);
@@ -1368,9 +1354,7 @@ void colfold_reduce(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
         const u64 avg = nrec / std::max<u64>(1, kmax);
         // table size to start with: what the previous flush of this handle needed, else the mean
         // column length (a column cannot hold more distinct rows than records)
-        int level = hint_maxd ? (hint_maxd <= 12 ? 0 : (hint_maxd <= 24 ? 1 : 2)) : (avg < 14 ? 0 : (avg < 40 ? 1 : 2));
-        if (g_thread_hbits >= 4 && g_thread_hbits <= 6)
-            level = g_thread_hbits - 4;
+        const int level = hint_maxd ? (hint_maxd <= 12 ? 0 : (hint_maxd <= 24 ? 1 : 2)) : (avg < 14 ? 0 : (avg < 40 ? 1 : 2));
         CtArgs a{sorted, L.low, L.rowbits, (u32)std::max<u64>(256, 6 * avg), nzcol, nzstart, totals, tmp, cnt,
                  nullptr, nullptr, nullptr, nullptr, longlist, counters + 2, d_maxd};
         // (nothing but skipped records: one block that finds no column)
@@ -1392,15 +1376,6 @@ void colfold_reduce(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
         once.set(colfold_kernel<true, W, true>, (int)smem);
         colfold_kernel<true, W, true><<<kNumSM * 2, W * 32, smem, stream>>>(sorted, L, combine, chunk, nzcol, nzstart, tilek,
                                                                           ntiles, tmp, cnt, d_overflow, longlist, counters + 2);
-    }
-    else if (simple)
-    {
-        constexpr int W = 8;
-        const size_t smem = sizeof(WarpSpace<true>) * W;
-        static FuncAttrOnce once;
-        once.set(colfold_kernel<true, W, false>, (int)smem);
-        colfold_kernel<true, W, false><<<std::max(1u, (ntiles + W - 1) / W), W * 32, smem, stream>>>(
-            sorted, L, combine, chunk, nzcol, nzstart, tilek, ntiles, tmp, cnt, d_overflow, nullptr, nullptr);
     }
     else
     {

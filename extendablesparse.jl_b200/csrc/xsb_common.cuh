@@ -201,21 +201,13 @@ struct StageFlags
 {
     unsigned char *flags; // one byte per tile, relative to the first staged record; nullptr: not a slab handle
     i64 pos0;             // staged records ahead of out0
-    // Counting at insertion (xsb_group.cu, PreCounted::cols): when set, the producer also leaves the
-    // column id of every record it stages in cols[position in the batch] (kNotMine for a record another
-    // rank owns); the grouping's counting pass then reads 4 instead of 16 bytes per record.
-    u32 *cols = nullptr;
 };
-constexpr u32 kNotMine = 0xffffffffu;
 __device__ __forceinline__ void st_staged(Rec *p, const Rec &r, const KeyLayout &L, const StageFlags &sf,
                                           const Rec *out0)
 {
     st_rec(p, r);
-    const bool foreign = sf.flags != nullptr && L.owner(r.key) != (u32)L.self;
-    if (foreign)
+    if (sf.flags != nullptr && L.owner(r.key) != (u32)L.self)
         sf.flags[(sf.pos0 + (i64)(p - out0)) >> kRouteTileShift] = 1; // benign race: same value
-    if (sf.cols != nullptr)
-        sf.cols[p - out0] = foreign ? kNotMine : (u32)L.col(r.key);
 }
 
 // Decoupled look-back over per-tile totals (tiles are dispatched in index order): the calling WARP

@@ -28,8 +28,7 @@
 namespace xsb {
 
 __global__ void __launch_bounds__(GP_WARPS * 32, 5)
-group_count_kernel(const Rec *__restrict__ in, u64 nrec, int ownershift, u32 me, u32 chunk0, u32 nchunks,
-                   const u32 *__restrict__ cols, u32 cols_chunks, CountTarget ct)
+group_count_kernel(const Rec *__restrict__ in, u64 nrec, int ownershift, u32 me, u32 nchunks, CountTarget ct)
 {
     const int colshift = ct.colshift;
     const u32 colmask = ct.colmask;
@@ -37,7 +36,7 @@ group_count_kernel(const Rec *__restrict__ in, u64 nrec, int ownershift, u32 me,
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     CountSpace &ws = reinterpret_cast<CountSpace *>(smem_raw)[warp];
-    const u32 chunk = chunk0 + blockIdx.x * GP_WARPS + warp; // chunks below chunk0 were counted when they were staged
+    const u32 chunk = blockIdx.x * GP_WARPS + warp;
     if (chunk >= nchunks)
         return;
     const u32 lt = lanemask_lt();
@@ -49,41 +48,7 @@ group_count_kernel(const Rec *__restrict__ in, u64 nrec, int ownershift, u32 me,
     u32 d = 0;
     bool crowded = false;
     const Rec *rec = in + r0 + lane;
-    if (chunk < cols_chunks)
-    { // the producer of this chunk left the records' column ids in cols[]: 4 instead of 16 bytes per
-      // record (kNotMine: a record another rank owns, already sent)
-        const u32 *cp = cols + r0 + lane;
-        u32 c[4], nc[4];
-#pragma unroll
-        for (int i = 0; i < 4; ++i)
-            nc[i] = cp[i * 32];
-#pragma unroll 1
-        for (int g = 0; g < GP_NB && !crowded; g += 4)
-        {
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-            {
-                c[i] = nc[i];
-                if (g + 4 < GP_NB)
-                    nc[i] = cp[(g + 4 + i) * 32];
-            }
-            if (d > (u32)GP_DMAX - 96u)
-                crowded = true;
-            else if (ownershift < 0)
-            {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    count_batch<true>(ws, (u64)c[i] << colshift, true, colshift, colmask, lt, d);
-            }
-            else
-            {
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    count_batch<false>(ws, (u64)c[i] << colshift, c[i] != kNotMine, colshift, colmask, lt, d);
-            }
-        }
-    }
-    else if (cnt_here == (u32)GP_W && ownershift < 0)
+    if (cnt_here == (u32)GP_W && ownershift < 0)
     { // whole chunk, every record takes part: no validity bookkeeping
         u64 key[4], nkey[4];
 #pragma unroll
@@ -273,7 +238,7 @@ constexpr int PS_TILE = PS_THREADS * PS_IPT;
 __device__ __forceinline__ u64 pair_payload(const Rec &r) { return (u64)__double_as_longlong(r.val); }
 
 __global__ void __launch_bounds__(PS_THREADS)
-pair_tilesum_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, u64 *__restrict__ trec,
+pair_tilesum_kernel(const Rec *__restrict__ sp, u32 npairs, u64 *__restrict__ trec,
                     u32 *__restrict__ tnz)
 {
     __shared__ u64 s_w[PS_THREADS / 32];
@@ -287,7 +252,7 @@ pair_tilesum_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, u64 *
         {
             const Rec r = sp[j];
             rec += pair_payload(r) & 0xffffull;
-            heads += (j == 0 || (sp[j - 1].key >> chunkbits) != (r.key >> chunkbits)) ? 1 : 0;
+            heads += (j == 0 || sp[j - 1].key != r.key) ? 1 : 0;
         }
     }
     // packed: records << 24 | heads (a tile holds at most 2048 heads)
@@ -308,7 +273,7 @@ pair_tilesum_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, u64 *
 }
 
 __global__ void __launch_bounds__(PS_THREADS)
-pair_emit_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, const u64 *__restrict__ trec,
+pair_emit_kernel(const Rec *__restrict__ sp, u32 npairs, const u64 *__restrict__ trec,
                  const u32 *__restrict__ tnz, u32 *__restrict__ offs, u32 *__restrict__ nzcol,
                  u32 *__restrict__ nzstart)
 {
@@ -318,7 +283,7 @@ pair_emit_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, const u6
     u32 cnt[PS_IPT], col[PS_IPT], tidx[PS_IPT];
     bool head[PS_IPT];
     u64 sum = 0;
-    u32 prevcol = (b0 > 0 && b0 <= npairs) ? (u32)(sp[b0 - 1].key >> chunkbits) : 0xffffffffu;
+    u32 prevcol = (b0 > 0 && b0 <= npairs) ? (u32)sp[b0 - 1].key : 0xffffffffu;
 #pragma unroll
     for (int i = 0; i < PS_IPT; ++i)
     {
@@ -333,7 +298,7 @@ pair_emit_kernel(const Rec *__restrict__ sp, u32 npairs, int chunkbits, const u6
             const u64 pl = pair_payload(r);
             cnt[i] = (u32)(pl & 0xffffull);
             tidx[i] = (u32)(pl >> 16);
-            col[i] = (u32)(r.key >> chunkbits);
+            col[i] = (u32)r.key;
             head[i] = j == 0 || col[i] != prevcol;
             prevcol = col[i];
         }
@@ -804,31 +769,6 @@ GpLayout gp_layout(u64 nrec, i64 ncols)
 } // namespace
 
 size_t group_workspace_bytes(u64 nrec, i64 ncols) { return gp_layout(nrec, ncols).bytes; }
-size_t group_pair_capacity(u64 nrec) { return (size_t)gp_layout(nrec, 1).cap + 1; }
-
-CountTarget group_count_target(void *workspace, Rec *pairs, u64 cap_records, i64 ncols, const KeyLayout &L)
-{
-    const GpLayout l = gp_layout(cap_records, ncols);
-    unsigned char *ws = static_cast<unsigned char *>(workspace);
-    CountTarget ct{};
-    ct.pair_total = reinterpret_cast<u32 *>(ws + l.off_ticket);
-    ct.flags = ct.pair_total + 1;
-    ct.pairs = pairs;
-    ct.chunkcols = reinterpret_cast<u32 *>(ws + l.off_chunkcols);
-    ct.chunkinfo = reinterpret_cast<uint2 *>(ws + l.off_chunkinfo);
-    ct.cap = l.cap;
-    ct.colshift = L.low + L.rowbits;
-    ct.colmask = L.colbits >= 32 ? 0xffffffffu : ((1u << L.colbits) - 1u);
-    ct.chunkcnt = reinterpret_cast<unsigned short *>(ws + l.off_chunkcnt);
-    return ct;
-}
-
-void group_precount_reset(cudaStream_t stream, void *workspace, u64 cap_records, i64 ncols)
-{ // pair ticket and flags (gp_layout puts them first)
-    (void)cap_records;
-    (void)ncols;
-    XSB_CUDA(cudaMemsetAsync(workspace, 0, 256, stream));
-}
 int group_chunk_records() { return GP_W; }
 
 bool group_supported(const KeyLayout &L, u64 nrec, i64 ncols)
@@ -843,20 +783,13 @@ void colscan_scan_launch(cudaStream_t stream, u64 *trec, u32 *tnz, i64 nt, u64 *
 // sort before the scatter.  On success nzcol / nzstart / totals (workspace of xsb_colfold.cu) hold
 // the compact column list.  Returns false -- with `in` untouched and `out` undefined -- when the
 // stream has too many (chunk, column) pairs for this to pay off.
-// XSB_PAIRS=sort: always order the (chunk, column) pairs with the radix sort (A-B measurements)
-static const bool g_pairs_sort = []() {
-    const char *e = getenv("XSB_PAIRS");
-    return e && e[0] == 's';
-}();
 
 bool group_by_column(cudaStream_t stream, const Rec *in, Rec *out, u64 nrec, i64 ncols, const KeyLayout &L, void *workspace,
-                     void *sort_workspace, u32 *nzcol, u32 *nzstart, u64 *totals, u64 *h_scal_pinned, u64 *d_scal,
-                     LaunchCounter &lc, StageTimer *timer, int *pair_passes, u64 *npairs_out, int ownershift, u32 me,
-                     const ChunkOrder *order, const PreCounted *pre)
+                     void *sort_workspace, u32 *nzcol, u32 *nzstart, u64 *totals, u64 *h_scal_pinned, LaunchCounter &lc,
+                     StageTimer *timer, int *pair_passes, u64 *npairs_out, int ownershift, u32 me, const ChunkOrder *order)
 {
-    // pre: the producers of the first pre->counted_chunks chunks already appended their pairs
-    const GpLayout l = gp_layout(pre ? pre->cap_records : nrec, ncols);
-    unsigned char *ws = static_cast<unsigned char *>(pre ? pre->ws : workspace);
+    const GpLayout l = gp_layout(nrec, ncols);
+    unsigned char *ws = static_cast<unsigned char *>(workspace);
     u32 *pair_total = reinterpret_cast<u32 *>(ws + l.off_ticket);
     u32 *flags = pair_total + 1;
     uint2 *chunkinfo = reinterpret_cast<uint2 *>(ws + l.off_chunkinfo);
@@ -878,27 +811,22 @@ bool group_by_column(cudaStream_t stream, const Rec *in, Rec *out, u64 nrec, i64
     once[0].set(group_count_kernel, (int)(sizeof(CountSpace) * GP_WARPS));
     once[1].set(group_scatter_kernel, (int)(sizeof(ScatterSpace) * GP_WARPS));
     Rec *pairs_a = out;
-    Rec *pairs_b = pre ? pre->pairs : out + l.cap;
+    Rec *pairs_b = out + l.cap;
 
     // ---- pass 1
     if (timer)
         timer->begin(stream);
-    if (!pre || pre->counted_chunks == 0)
-        XSB_CUDA(cudaMemsetAsync(ws + l.off_ticket, 0, 256, stream)); // pair ticket, flags
+    XSB_CUDA(cudaMemsetAsync(ws + l.off_ticket, 0, 256, stream)); // pair ticket, flags
     // The bucketed pair path works on per-column arrays (12 bytes cleared + 12 bytes scanned per column and
     // flush); for a hypersparse flush (far more columns than records) the radix sort of the pairs is cheaper.
-    const bool try_buckets = !g_pairs_sort && (u64)ncols <= 8ull * nrec;
+    const bool try_buckets = (u64)ncols <= 8ull * nrec;
     if (try_buckets) // per-column totals and bucket cursors
         XSB_CUDA(cudaMemsetAsync(ws + l.off_colrec, 0, l.off_pstart - l.off_colrec, stream));
-    const int chunkbits = 0; // pair keys hold the column only
-    const u32 chunk0 = pre ? std::min(pre->counted_chunks, nchunks) : 0u;
-    if (chunk0 < nchunks)
     {
         CountTarget ct{pair_total, flags, pairs_b, chunkcols, chunkinfo, l.cap, colshift, colmask, chunkcnt};
-        const unsigned cblocks = (nchunks - chunk0 + GP_WARPS - 1) / GP_WARPS;
-        group_count_kernel<<<cblocks, GP_WARPS * 32, sizeof(CountSpace) * GP_WARPS, stream>>>(
-            in, nrec, ownershift, me, chunk0, nchunks, pre ? pre->cols : nullptr,
-            pre ? std::min(pre->cols_chunks, nchunks) : 0u, ct);
+        const unsigned cblocks = (nchunks + GP_WARPS - 1) / GP_WARPS;
+        group_count_kernel<<<cblocks, GP_WARPS * 32, sizeof(CountSpace) * GP_WARPS, stream>>>(in, nrec, ownershift, me,
+                                                                                              nchunks, ct);
         lc.add();
         XSB_CUDA(cudaGetLastError());
     }
@@ -970,13 +898,12 @@ bool group_by_column(cudaStream_t stream, const Rec *in, Rec *out, u64 nrec, i64
         if (timer)
             timer->begin(stream);
         const unsigned ptiles = (npairs + PS_TILE - 1) / PS_TILE;
-        pair_tilesum_kernel<<<ptiles, PS_THREADS, 0, stream>>>(sp, npairs, chunkbits, trec, tnz);
+        pair_tilesum_kernel<<<ptiles, PS_THREADS, 0, stream>>>(sp, npairs, trec, tnz);
         colscan_scan_launch(stream, trec, tnz, (i64)ptiles, totals, nzstart);
-        pair_emit_kernel<<<ptiles, PS_THREADS, 0, stream>>>(sp, npairs, chunkbits, trec, tnz, offs, nzcol, nzstart);
+        pair_emit_kernel<<<ptiles, PS_THREADS, 0, stream>>>(sp, npairs, trec, tnz, offs, nzcol, nzstart);
         lc.add(3);
         XSB_CUDA(cudaGetLastError());
     }
-    (void)d_scal;
     // ---- pass 2
     const unsigned sblocks = (nchunks + GP_WARPS - 1) / GP_WARPS;
     group_scatter_kernel<<<sblocks, GP_WARPS * 32, sizeof(ScatterSpace) * GP_WARPS, stream>>>(

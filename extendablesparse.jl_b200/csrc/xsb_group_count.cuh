@@ -1,7 +1,5 @@
-// xsb_group_count.cuh -- the counting half of the two-pass grouping (xsb_group.cu) as device
-// functions, so that the kernels that PRODUCE staged records (pack / emit kernels, xsb_insert.cu)
-// can count a chunk while its records are still in registers or shared memory instead of having
-// group_count_kernel read them back from HBM at flush time.
+// xsb_group_count.cuh -- the counting half of the two-pass grouping (xsb_group.cu): per-chunk
+// distinct columns and their record counts, as device functions of group_count_kernel.
 #pragma once
 #include "xsb_internal.h"
 
@@ -19,6 +17,20 @@ constexpr int GP_WARPS = 8;
 constexpr u32 GP_EMPTY = 0xffffffffu;
 
 __device__ __forceinline__ u32 gp_hash(u32 col) { return (col * 0x9E3779B1u) >> (32 - GP_HBITS); }
+
+// where a chunk's (column, count) pairs go: fields of the grouping workspace (xsb_group.cu)
+struct CountTarget
+{
+    u32 *pair_total;  // ticket: pairs appended so far
+    u32 *flags;       // != 0: a chunk had too many distinct columns / the pair list is full
+    Rec *pairs;       // (column, ticket position << 16 | count)
+    u32 *chunkcols;   // column of pair p
+    uint2 *chunkinfo; // per chunk: (first pair, pairs)
+    u32 cap;          // room of the pair list
+    int colshift;
+    u32 colmask;
+    unsigned short *chunkcnt; // records of pair p (1..chunk size)
+};
 
 struct CountSpace
 {

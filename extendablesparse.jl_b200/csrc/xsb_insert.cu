@@ -1002,6 +1002,7 @@ emit_p1fem_kernel(i64 nxn, i64 nyn, i64 nzn, KeyLayout L, u32 tid, u32 flavour, 
     const i64 nrec = (t_last - t_first) * FEM_REC;
     const i64 pos0 = (t_first - tet_begin) * FEM_REC;
     Rec *dst = out + pos0;
+#pragma unroll 2 // unrolled further, the loop needs more registers than the tetrahedron kernel above it
     for (i64 q = threadIdx.x; q < nrec; q += FEM_THREADS)
     {
         const int tt = (int)q / FEM_REC;

@@ -104,10 +104,6 @@ Rec *radix_sort_records(cudaStream_t stream, Rec *a, Rec *b, u64 n, const SortPl
 
 void partition_records(cudaStream_t stream, const Rec *in, Rec *out, u64 n, int shift, int bits, void *workspace,
                        LaunchCounter &lc, u64 *counts_host);
-void set_sort_variant(int v);
-int get_sort_variant();
-void sort_selftest(cudaStream_t stream, u64 n, int nbits, int variant, int reps, float *ms_hist, float *ms_pass,
-                   u64 *violations_out, int *npasses_out);
 
 // ---- xsb_flush.cu
 struct CscView
@@ -125,15 +121,6 @@ size_t reduce_workspace_bytes(u64 nrec, i64 ncols);
 void reduce_emit_csc(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout L, int combine, int mode,
                      bool plain_adds, i64 ncols, int idx64, int base, void *rowval_out, double *nzval_out,
                      void *colptr_out, void *workspace, u64 *d_nnz, LaunchCounter &lc, StageTimer *timer);
-
-// ---- xsb_column.cu
-size_t column_workspace_bytes(u64 nrec, i64 ncols);
-bool column_path_supported(const KeyLayout &L);
-// records sorted by column only -> CSC (rows ordered per column in shared memory)
-void column_reduce_emit_csc(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout L, int combine,
-                            bool plain_adds, i64 ncols, int idx64, int base, void *rowval_out, double *nzval_out,
-                            void *colptr_out, void *workspace, u64 *d_nnz, u32 *d_overflow, LaunchCounter &lc,
-                            StageTimer *timer);
 
 // ---- xsb_colfold.cu
 size_t colfold_workspace_bytes(u64 nrec, i64 ncols);
@@ -160,46 +147,16 @@ struct ChunkOrder
 {
     u32 c_old, c_own, c_low;
 };
-// where a chunk's (column, count) pairs go: fields of the grouping workspace (xsb_group.cu)
-struct CountTarget
-{
-    u32 *pair_total;  // ticket: pairs appended so far
-    u32 *flags;       // != 0: a chunk had too many distinct columns / the pair list is full
-    Rec *pairs;       // (column, ticket position << 16 | count)
-    u32 *chunkcols;   // column of pair p
-    uint2 *chunkinfo; // per chunk: (first pair, pairs)
-    u32 cap;          // room of the pair list
-    int colshift;
-    u32 colmask;
-    unsigned short *chunkcnt; // records of pair p (1..chunk size)
-};
 constexpr u32 kMaxColPairs = 128; // a column met by more chunks than this sends the flush to the pair SORT
 
-// Counting done ahead of the flush by the kernels that staged the records ("count rides along
-// with insertion"): the first counted_chunks chunks of the flush's input already have their pairs in
-// `pairs` and their chunkinfo / chunkcols in `ws` (laid out for cap_records records).
-struct PreCounted
-{
-    void *ws;
-    Rec *pairs;
-    u64 cap_records;
-    u32 counted_chunks;
-    // chunks [counted_chunks, cols_chunks) are not counted yet, but their producers left the column id
-    // of every record in cols[record position]: the counting pass reads 4 instead of 16 bytes per record
-    const u32 *cols;
-    u32 cols_chunks;
-};
-size_t group_pair_capacity(u64 nrec);
-CountTarget group_count_target(void *ws, Rec *pairs, u64 cap_records, i64 ncols, const KeyLayout &L);
-void group_precount_reset(cudaStream_t stream, void *ws, u64 cap_records, i64 ncols);
 int group_chunk_records();
 size_t group_workspace_bytes(u64 nrec, i64 ncols);
 bool group_supported(const KeyLayout &L, u64 nrec, i64 ncols);
 // stable grouping by column in two passes (sparse per-chunk histograms); false: no column locality
 bool group_by_column(cudaStream_t stream, const Rec *in, Rec *out, u64 nrec, i64 ncols, const KeyLayout &L, void *workspace,
-                     void *sort_workspace, u32 *nzcol, u32 *nzstart, u64 *totals, u64 *h_scal_pinned, u64 *d_scal,
-                     LaunchCounter &lc, StageTimer *timer, int *pair_passes, u64 *npairs_out, int ownershift = -1,
-                     u32 me = 0, const ChunkOrder *order = nullptr, const PreCounted *pre = nullptr);
+                     void *sort_workspace, u32 *nzcol, u32 *nzstart, u64 *totals, u64 *h_scal_pinned, LaunchCounter &lc,
+                     StageTimer *timer, int *pair_passes, u64 *npairs_out, int ownershift = -1, u32 me = 0,
+                     const ChunkOrder *order = nullptr);
 // ownershift >= 0: records whose key >> ownershift != me belong to other ranks and are skipped
 // parked entries -> rowval / nzval
 void colfold_compact(cudaStream_t stream, const Rec *tmp, u64 nrec, i64 ncols, int idx64, int base,

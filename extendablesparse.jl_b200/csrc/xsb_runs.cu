@@ -23,7 +23,6 @@
 // written once + 20 B per (chunk, column) pair -- SURVEY.md 8(d)'s algorithmic bytes plus the pairs.
 #include "xsb_chunk.cuh"
 #include "xsb_internal.h"
-#include <cstdlib>
 
 namespace xsb {
 
@@ -694,13 +693,6 @@ runfold_kernel(const Rec *__restrict__ buf, int low, int rowbits, u32 maxlen, co
 // host side
 // ------------------------------------------------------------------------
 namespace {
-int env_int(const char *name, int dflt)
-{
-    const char *e = getenv(name);
-    return e && *e ? atoi(e) : dflt;
-}
-const int g_runs_hbits = env_int("XSB_RUNS_HBITS", 0); // 4|5|6|15: fixes the fold's table shape (tuning)
-
 struct RwLayout
 {
     size_t off_colpairs, off_status, off_fstatus, off_pstart, off_bucket, clear_bytes, bytes;
@@ -829,8 +821,6 @@ void launch_runfold_t(cudaStream_t stream, unsigned blocks, const Rec *buf, int 
 }
 } // namespace
 
-int runs_fold_levels() { return 4; }
-
 // level 0..3 = table shapes 4, 15, 5, 6.  *d_redo afterwards: bit 0: a column did not fit the table (bit 2 as well:
 // not even the largest one); bit 1: a column is too long / met by too many chunks for one thread.
 void runs_fold(cudaStream_t stream, const Rec *buf, const KeyLayout &L, i64 ncols, int idx64, int base, const CscView &old,
@@ -842,14 +832,6 @@ void runs_fold(cudaStream_t stream, const Rec *buf, const KeyLayout &L, i64 ncol
     u32 *pstart = reinterpret_cast<u32 *>(ws + l.off_pstart);
     u64 *bucket = reinterpret_cast<u64 *>(ws + l.off_bucket);
     u64 *status = reinterpret_cast<u64 *>(ws + l.off_fstatus);
-    if (g_runs_hbits == 4)
-        level = 0;
-    else if (g_runs_hbits == 15)
-        level = 1;
-    else if (g_runs_hbits == 5)
-        level = 2;
-    else if (g_runs_hbits == 6)
-        level = 3;
     const unsigned tpb = 32u * (unsigned)(level == 3 ? RfShape<6>::kWarps
                                                       : (level == 2 ? RfShape<5>::kWarps
                                                                     : (level == 1 ? RfShape<15>::kWarps : RfShape<4>::kWarps)));

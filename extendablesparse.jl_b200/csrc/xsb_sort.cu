@@ -288,35 +288,10 @@ onesweep_kernel(const Rec *__restrict__ in, Rec *__restrict__ out, u32 n, u32 nt
 // ------------------------------------------------------------------------
 // host driver
 // ------------------------------------------------------------------------
-typedef void (*OnesweepFn)(const Rec *, Rec *, u32, u32, int, int, const u64 *, u64 *, u32 *, u32 *);
-struct OnesweepVariant
-{
-    OnesweepFn fn;
-    int threads, tile;
-};
-template <int THREADS, int IPT, int MINBLK> static OnesweepVariant make_variant()
-{
-    return OnesweepVariant{onesweep_kernel<THREADS, IPT, MINBLK>, THREADS, THREADS * IPT};
-}
-static const OnesweepVariant kVariants[] = {
-    make_variant<256, 16, 2>(), // 0: 4096-record tiles, 2 CTAs/SM
-    make_variant<256, 8, 4>(),  // 1: 2048-record tiles, 4 CTAs/SM
-    make_variant<512, 8, 2>(),  // 2: 4096-record tiles, 2 x 16 warps
-    make_variant<256, 12, 3>(), // 3: 3072-record tiles, 3 CTAs/SM
-    make_variant<512, 6, 3>(),  // 4: 3072-record tiles, 3 x 16 warps
-    make_variant<256, 8, 3>(),  // 5
-    make_variant<512, 4, 4>(),  // 6: 2048-record tiles, 4 x 16 warps
-};
-constexpr int kNumVariants = (int)(sizeof(kVariants) / sizeof(kVariants[0]));
-static int g_variant = 2; // 512 threads x 8 records: best of the measured tile shapes (tools/tune_sort.py)
-constexpr int kMinTile = 2048;
-
-void set_sort_variant(int v)
-{
-    if (v >= 0 && v < kNumVariants)
-        g_variant = v;
-}
-int get_sort_variant() { return g_variant; }
+// Onesweep tile: 512 threads x 8 records, 2 CTAs per SM -- the fastest of the tile shapes measured on B200.
+constexpr int OS_THREADS = 512, OS_IPT = 8, OS_MINBLK = 2;
+constexpr int OS_TILE = OS_THREADS * OS_IPT;
+constexpr int kMinTile = 2048; // the workspace is sized for tiles this small (room to spare for OS_TILE)
 
 static u64 sort_portion(int tile) { return ((1ull << 30) - 1ull) / (u64)tile * (u64)tile; }
 
@@ -359,10 +334,9 @@ Rec *radix_sort_records(cudaStream_t stream, Rec *a, Rec *b, u64 n, const SortPl
     const bool nosort = n <= 1 || plan.npasses == 0;
     if (nosort && (colcnt == nullptr || n == 0))
         return a;
-    const OnesweepVariant &var = kVariants[g_variant];
-    static FuncAttrOnce once[kNumVariants];
-    once[g_variant].set(reinterpret_cast<const void *>(var.fn), (int)(var.tile * sizeof(Rec)));
-    const u64 portion = sort_portion(var.tile);
+    static FuncAttrOnce once;
+    once.set(onesweep_kernel<OS_THREADS, OS_IPT, OS_MINBLK>, (int)(OS_TILE * sizeof(Rec)));
+    const u64 portion = sort_portion(OS_TILE);
     unsigned char *ws = static_cast<unsigned char *>(workspace);
     u64 *ghist = reinterpret_cast<u64 *>(ws);
     u64 *gnext0 = ghist + kMaxPasses * kRadix;
@@ -402,10 +376,10 @@ Rec *radix_sort_records(cudaStream_t stream, Rec *a, Rec *b, u64 n, const SortPl
         for (u64 off = 0; off < n; off += portion)
         {
             const u32 cnt = (u32)std::min<u64>(portion, n - off);
-            const u32 ntiles = (cnt + var.tile - 1) / var.tile;
+            const u32 ntiles = (cnt + OS_TILE - 1) / OS_TILE;
             const bool more = off + portion < n;
             XSB_CUDA(cudaMemsetAsync(counter, 0, 256 + sizeof(u32) * (size_t)ntiles * nbins, stream));
-            var.fn<<<ntiles, var.threads, var.tile * sizeof(Rec), stream>>>(
+            onesweep_kernel<OS_THREADS, OS_IPT, OS_MINBLK><<<ntiles, OS_THREADS, OS_TILE * sizeof(Rec), stream>>>(
                 src + off, dst, cnt, ntiles, plan.shift[p], plan.bits[p], gbase, more ? gn[flip] : nullptr,
                 status, counter);
             lc.add();
@@ -453,10 +427,9 @@ void partition_records(cudaStream_t stream, const Rec *in, Rec *out, u64 n, int 
         counts_host[d] = h[d];
     histogram_scan_kernel<<<1, kRadix, 0, stream>>>(ghist, 1);
     lc.add();
-    const OnesweepVariant &var = kVariants[g_variant];
-    static FuncAttrOnce once[kNumVariants];
-    once[g_variant].set(reinterpret_cast<const void *>(var.fn), (int)(var.tile * sizeof(Rec)));
-    const u64 portion = sort_portion(var.tile);
+    static FuncAttrOnce once;
+    once.set(onesweep_kernel<OS_THREADS, OS_IPT, OS_MINBLK>, (int)(OS_TILE * sizeof(Rec)));
+    const u64 portion = sort_portion(OS_TILE);
     u64 *gnext0 = ghist + kMaxPasses * kRadix;
     u64 *gnext1 = gnext0 + kRadix;
     u32 *counter = reinterpret_cast<u32 *>(gnext1 + kRadix);
@@ -467,11 +440,11 @@ void partition_records(cudaStream_t stream, const Rec *in, Rec *out, u64 n, int 
     for (u64 off = 0; off < n; off += portion)
     {
         const u32 cnt = (u32)std::min<u64>(portion, n - off);
-        const u32 ntiles = (cnt + var.tile - 1) / var.tile;
+        const u32 ntiles = (cnt + OS_TILE - 1) / OS_TILE;
         const bool more = off + portion < n;
         XSB_CUDA(cudaMemsetAsync(counter, 0, 256 + sizeof(u32) * (size_t)ntiles * nb, stream));
-        var.fn<<<ntiles, var.threads, var.tile * sizeof(Rec), stream>>>(in + off, out, cnt, ntiles, shift, bits, gbase,
-                                                                        more ? gn[flip] : nullptr, status, counter);
+        onesweep_kernel<OS_THREADS, OS_IPT, OS_MINBLK><<<ntiles, OS_THREADS, OS_TILE * sizeof(Rec), stream>>>(
+            in + off, out, cnt, ntiles, shift, bits, gbase, more ? gn[flip] : nullptr, status, counter);
         lc.add();
         if (more)
         {
@@ -480,86 +453,6 @@ void partition_records(cudaStream_t stream, const Rec *in, Rec *out, u64 n, int 
         }
     }
     XSB_CUDA(cudaGetLastError());
-}
-
-// ------------------------------------------------------------------------
-// self test / micro benchmark of the sort (random keys, stability checked)
-// ------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) selftest_fill_kernel(Rec *__restrict__ out, u64 n, int nbits, u64 seed)
-{
-    const u64 stride = (u64)gridDim.x * blockDim.x;
-    const u64 mask = nbits >= 64 ? ~0ull : ((1ull << nbits) - 1ull);
-    for (u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += stride)
-    {
-        u64 x = k + seed * 0x9e3779b97f4a7c15ull;
-        x ^= x >> 30;
-        x *= 0xbf58476d1ce4e5b9ull;
-        x ^= x >> 27;
-        x *= 0x94d049bb133111ebull;
-        x ^= x >> 31;
-        Rec r;
-        r.key = x & mask;
-        r.val = (double)k;
-        st_rec(out + k, r);
-    }
-}
-
-__global__ void __launch_bounds__(256)
-selftest_check_kernel(const Rec *__restrict__ in, u64 n, u64 *__restrict__ violations)
-{
-    const u64 stride = (u64)gridDim.x * blockDim.x;
-    for (u64 k = (u64)blockIdx.x * blockDim.x + threadIdx.x + 1; k < n; k += stride)
-    {
-        const Rec a = in[k - 1], b = in[k];
-        if (a.key > b.key || (a.key == b.key && !(a.val < b.val)))
-            atomicAdd(violations, 1ull);
-    }
-}
-
-void sort_selftest(cudaStream_t stream, u64 n, int nbits, int variant, int reps, float *ms_hist, float *ms_pass,
-                   u64 *violations_out, int *npasses_out)
-{
-    const int saved = g_variant;
-    set_sort_variant(variant);
-    Rec *a = nullptr, *b = nullptr;
-    void *ws = nullptr;
-    u64 *d_viol = nullptr;
-    XSB_CUDA(cudaMallocAsync(&a, sizeof(Rec) * n, stream));
-    XSB_CUDA(cudaMallocAsync(&b, sizeof(Rec) * n, stream));
-    XSB_CUDA(cudaMallocAsync(&ws, sort_workspace_bytes(n), stream));
-    XSB_CUDA(cudaMallocAsync(&d_viol, sizeof(u64), stream));
-    XSB_CUDA(cudaMemsetAsync(d_viol, 0, sizeof(u64), stream));
-    const SortPlan plan = make_sort_plan(0, nbits);
-    LaunchCounter lc;
-    StageTimes acc;
-    Rec *res = nullptr;
-    for (int r = 0; r < reps + 1; ++r)
-    {
-        selftest_fill_kernel<<<kNumSM * 8, 256, 0, stream>>>(a, n, nbits, 12345);
-        StageTimer t;
-        res = radix_sort_records(stream, a, b, n, plan, ws, lc, &t);
-        XSB_CUDA(cudaStreamSynchronize(stream));
-        StageTimes st;
-        t.collect(st);
-        if (r > 0)
-        {
-            acc.histogram += st.histogram;
-            acc.sort += st.sort;
-        }
-    }
-    selftest_check_kernel<<<kNumSM * 8, 256, 0, stream>>>(res, n, d_viol);
-    u64 viol = 0;
-    XSB_CUDA(cudaMemcpyAsync(&viol, d_viol, sizeof(u64), cudaMemcpyDeviceToHost, stream));
-    XSB_CUDA(cudaStreamSynchronize(stream));
-    cudaFreeAsync(a, stream);
-    cudaFreeAsync(b, stream);
-    cudaFreeAsync(ws, stream);
-    cudaFreeAsync(d_viol, stream);
-    set_sort_variant(saved);
-    *ms_hist = acc.histogram / reps;
-    *ms_pass = acc.sort / reps / std::max(plan.npasses, 1);
-    *violations_out = viol;
-    *npasses_out = plan.npasses;
 }
 
 } // namespace xsb

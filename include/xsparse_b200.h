@@ -94,8 +94,7 @@ typedef struct xsb_flush_stats
     int32_t sort_passes;      /* onesweep passes executed              */
     int32_t sort_bits;        /* key bits sorted                       */
     int32_t kernel_launches;  /* kernels launched by the flush         */
-    int32_t column_path;      /* 0: (col,row) sort + flat reduction; 1: column sort + in-tile row ordering;
-                                 2: column sort + hash fold; 3: two-pass grouping by column + hash fold;
+    int32_t column_path;      /* 0: (col,row) sort + flat reduction; 2: column sort + hash fold; 3: two-pass grouping by column + hash fold;
                                  4: grouped chunks (records grouped by column while they were staged) +
                                     thread-per-column merge with the resident CSC -- the product path */
     float ms_total;           /* device time of the whole flush (CUDA events; 0 unless profiling on) */
@@ -355,13 +354,6 @@ int32_t xsb_stream_count_blockrd(int64_t nx, int64_t ny, int64_t nz, int32_t ns,
 int32_t xsb_debug_fetch_staged(xsb_matrix *h, int32_t tid, void *I, void *J, void *V,
                                int32_t *flavour, int64_t capacity, int64_t *count);
 
-/* Tuning/self-test aids: choose the onesweep tile shape; sort n random nbits-wide keys,
- * report per-pass time and the number of order/stability violations (must be 0). */
-int32_t xsb_debug_set_sort_variant(int32_t variant);
-int32_t xsb_debug_sort_selftest(xsb_matrix *h, int64_t n, int32_t nbits, int32_t variant, int32_t reps,
-                                float *ms_histogram, float *ms_per_pass, int64_t *violations,
-                                int32_t *npasses);
-
 /* ------------------------------------------------------------------ */
 /* streams, timing                                                     */
 /* ------------------------------------------------------------------ */
@@ -373,13 +365,13 @@ int32_t xsb_timer_start(xsb_matrix *h);
 int32_t xsb_timer_stop(xsb_matrix *h, float *ms_out);
 /* Per-stage CUDA-event timing inside xsb_flush (off by default). */
 int32_t xsb_set_profiling(xsb_matrix *h, int32_t enable);
-/* Flush algorithm.  AUTO: stable radix sort on the column bits only; a warp per group of columns
- * folds duplicates through a shared-memory hash table in stream order and sorts only the distinct
- * entries by row (falls back by itself when a group exceeds the table).  All strategies give the
- * same bits. */
+/* Flush algorithm.  AUTO: records brought together by column (grouped chunks, two-pass grouping or
+ * a stable radix sort on the column bits); per column, duplicates are folded through a hash table in
+ * stream order and only the distinct entries are sorted by row (falls back to the FULLSORT path by
+ * itself when a column does not fit).  FULLSORT: (col,row) radix sort + flat segmented reduction.
+ * Both give the same bits; any other value returns XSB_EINVAL. */
 #define XSB_STRATEGY_AUTO 0
-#define XSB_STRATEGY_FULLSORT 1 /* (col,row) radix sort + flat segmented reduction */
-#define XSB_STRATEGY_COLSORT 2  /* column-only sort + per-column bitonic row ordering  */
+#define XSB_STRATEGY_FULLSORT 1
 int32_t xsb_set_strategy(xsb_matrix *h, int32_t strategy);
 /* How STRATEGY_AUTO brings the records of a column together.  AUTO: try the two-pass grouping
  * (sparse per-chunk column histograms; pays off when consecutive insertions touch few distinct

@@ -731,9 +731,8 @@ def test_full_size_fd_properties(xsb):
 
 # ---------------------------------------------------------------- flush strategies
 def test_strategies_agree_and_long_columns_fall_back(xsb, oracle):
-    """Column sort + hash fold (AUTO), column sort + in-tile row ordering (COLSORT) and the (col,row)
-    sort (FULLSORT) give the same bits; a column too rich for the in-warp paths makes AUTO and
-    COLSORT finish with the general path."""
+    """Column sort + hash fold (AUTO) and the (col,row) sort (FULLSORT) give the same bits; a column too
+    rich for the in-warp path makes AUTO finish with the general path.  No other strategy is accepted."""
     rng = np.random.default_rng(77)
     m, n, cnt = 3000, 500, 60000
     I = rng.integers(1, m + 1, cnt)
@@ -742,8 +741,7 @@ def test_strategies_agree_and_long_columns_fall_back(xsb, oracle):
     A = oracle.OracleExt(m, n)
     A.insert_batch(I, J, V, oracle.UPDATE)
     ref = A.csc()
-    for strat, expect_col in ((xsb.capi.STRATEGY_AUTO, 2), (xsb.capi.STRATEGY_COLSORT, 1),
-                              (xsb.capi.STRATEGY_FULLSORT, 0)):
+    for strat, expect_col in ((xsb.capi.STRATEGY_AUTO, 2), (xsb.capi.STRATEGY_FULLSORT, 0)):
         h = xsb.Handle(m, n)
         h.set_strategy(strat)
         h.insert_batch(I, J, V, xsb.UPDATE)
@@ -755,14 +753,13 @@ def test_strategies_agree_and_long_columns_fall_back(xsb, oracle):
     J2[:3000] = 7
     A = oracle.OracleExt(m, n)
     A.insert_batch(I, J2, V, oracle.UPDATE)
-    for strat in (xsb.capi.STRATEGY_AUTO, xsb.capi.STRATEGY_COLSORT):
-        h = xsb.Handle(m, n)
-        h.set_strategy(strat)
-        h.insert_batch(I, J2, V, xsb.UPDATE)
-        h.flush()
-        st = h.flush_stats()
-        assert st["column_path"] == 0 and st["sort_passes"] > 3
-        assert_csc_equal(h.fetch_csc_numpy(), A.csc())
+    h = xsb.Handle(m, n)
+    h.set_strategy(xsb.capi.STRATEGY_AUTO)
+    h.insert_batch(I, J2, V, xsb.UPDATE)
+    h.flush()
+    st = h.flush_stats()
+    assert st["column_path"] == 0 and st["sort_passes"] > 3
+    assert_csc_equal(h.fetch_csc_numpy(), A.csc())
     # columns of every length around the warp-sort sizes (31..257 records), duplicates included
     lens = [1, 2, 31, 32, 33, 63, 64, 65, 127, 128, 129, 255, 256]
     Jl = np.concatenate([np.full(L, k + 1) for k, L in enumerate(lens)])
@@ -771,13 +768,17 @@ def test_strategies_agree_and_long_columns_fall_back(xsb, oracle):
     perm = rng.permutation(len(Jl))
     A = oracle.OracleExt(50, len(lens))
     A.insert_batch(Il[perm], Jl[perm], Vl[perm], oracle.RAW)
-    for strat, expect_col in ((xsb.capi.STRATEGY_AUTO, 2), (xsb.capi.STRATEGY_COLSORT, 1)):
-        h = xsb.Handle(50, len(lens))
-        h.set_strategy(strat)
-        h.insert_batch(Il[perm], Jl[perm], Vl[perm], xsb.RAW)
-        h.flush()
-        assert h.flush_stats()["column_path"] == expect_col
-        assert_csc_equal(h.fetch_csc_numpy(), A.csc())
+    h = xsb.Handle(50, len(lens))
+    h.set_strategy(xsb.capi.STRATEGY_AUTO)
+    h.insert_batch(Il[perm], Jl[perm], Vl[perm], xsb.RAW)
+    h.flush()
+    assert h.flush_stats()["column_path"] == 2
+    assert_csc_equal(h.fetch_csc_numpy(), A.csc())
+    # any value but AUTO (0) and FULLSORT (1) is rejected
+    h = xsb.Handle(m, n)
+    with pytest.raises(xsb.capi.XsbError) as e:
+        h.set_strategy(2)
+    assert e.value.code == xsb.capi.EINVAL
 
 
 def test_hash_fold_groups_of_columns(xsb, oracle):

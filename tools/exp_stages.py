@@ -2,7 +2,6 @@
 """Stage timings of one flush! per workload (development tool, not a bench line).
 
   python tools/exp_stages.py [fem128] [fd200] [rd96] [fem64] ...   (default: fem128 fd200 rd96)
-Environment knobs of the library (XSB_THREAD_FOLD, XSB_THREAD_HBITS, ...) are honoured.
 """
 import os
 import sys
