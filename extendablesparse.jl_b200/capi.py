@@ -108,6 +108,7 @@ SIGNATURES = {
     "xsb_reserve": (_i32, [_p, _i32, _i64]),
     "xsb_insert_batch": (_i32, [_p, _i32, _p, _p, _p, _i64, _i32]),
     "xsb_insert_triplets": (_i32, [_p, _i32, _p, _i64, _i32]),
+    "xsb_insert_elements": (_i32, [_p, _i32, _i32, _i64, _p, _p, _i32]),
     "xsb_pending": (_i32, [_p, C.POINTER(_i64)]),
     "xsb_flush": (_i32, [_p, _i32, C.POINTER(_i64), C.POINTER(_i32)]),
     "xsb_flush_ex": (_i32, [_p, _i32, _i32, C.POINTER(_i64), C.POINTER(_i32)]),
@@ -115,6 +116,7 @@ SIGNATURES = {
     "xsb_get_values": (_i32, [_p, _p, _p, _p, _i64]),
     "xsb_zero_values": (_i32, [_p]),
     "xsb_freeze_pattern": (_i32, [_p, _p, _p, _i64]),
+    "xsb_freeze_elements": (_i32, [_p, _i32, _i64, _p]),
     "xsb_reassemble_values": (_i32, [_p, _p, _i64, _i32]),
     "xsb_reassemble_values_zeroed": (_i32, [_p, _p, _i64, _i32]),
     "xsb_unfreeze": (_i32, [_p]),
@@ -352,6 +354,40 @@ class Handle:
         if count is None:
             count = len(T)
         self._c(lib().xsb_insert_triplets(self._h, tid, ptr(T), count, flavour))
+
+    def _element_arrays(self, dofs, Aloc=None):
+        """(ncells, k) connectivity in the handle's index type and (ncells, k, k) Float64 element matrices, both
+        C-contiguous: the column-major k x ncells / k x k x ncells arrays of the C ABI (Aloc[c, jl, il] is entry
+        (il, jl) of element c).  numpy arrays are converted, torch tensors (host or device) must already match."""
+        if hasattr(dofs, "data_ptr"):
+            want = "torch.int64" if self.idx_type == I64 else "torch.int32"
+            if str(dofs.dtype) != want:
+                raise TypeError(f"dofs must be {want}")
+        else:
+            dofs = np.ascontiguousarray(dofs, self.idx_dtype)
+        if dofs.ndim != 2:
+            raise ValueError("dofs must have shape (ncells, k)")
+        ncells, k = (int(x) for x in dofs.shape)
+        if Aloc is not None:
+            if hasattr(Aloc, "data_ptr"):
+                if str(Aloc.dtype) != "torch.float64":
+                    raise TypeError("Aloc must be torch.float64")
+            else:
+                Aloc = np.ascontiguousarray(Aloc, np.float64)
+            if tuple(Aloc.shape) != (ncells, k, k):
+                raise ValueError(f"Aloc must have shape (ncells, k, k) = {(ncells, k, k)}, not {tuple(Aloc.shape)}")
+        return dofs, Aloc, ncells, k
+
+    def insert_elements(self, dofs, Aloc, flavour=RAW, tid=0):
+        """k*k*ncells calls of an element loop: call k*k*c + k*jl + il is (dofs[c, il], dofs[c, jl], Aloc[c, jl, il])."""
+        dofs, Aloc, ncells, k = self._element_arrays(dofs, Aloc)
+        self._c(lib().xsb_insert_elements(self._h, tid, k, ncells, ptr(dofs), ptr(Aloc), flavour))
+
+    def freeze_elements(self, dofs):
+        """freeze_pattern for the stream insert_elements(dofs, .) stages; reassemble_values(Aloc) then takes the
+        element matrices as they are."""
+        dofs, _, ncells, k = self._element_arrays(dofs)
+        self._c(lib().xsb_freeze_elements(self._h, k, ncells, ptr(dofs)))
 
     def flush(self, mode=DETERMINISTIC, combine=COMBINE_SEED):
         nnz, changed = _i64(0), _i32(0)

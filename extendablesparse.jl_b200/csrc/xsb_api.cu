@@ -1209,6 +1209,59 @@ void end_emit(xsb_matrix *h, int32_t tid, int32_t flavour, i64 count)
         h->has_assign = true;
 }
 
+// the limits of an element batch: k in [1, 64]; its k^2 ncells calls stay below 2^63
+i64 element_calls(int32_t k, int64_t ncells)
+{
+    REQUIRE(k >= 1 && k <= 64, XSB_EINVAL, "element size k must be in [1, 64]");
+    REQUIRE(ncells >= 0, XSB_EINVAL, "negative element count");
+    REQUIRE(ncells <= INT64_MAX / ((i64)k * k), XSB_EINVAL, "k^2 * ncells overflows");
+    return (i64)k * k * ncells;
+}
+
+// xsb_freeze_pattern / xsb_freeze_elements
+void freeze_check(xsb_matrix *h, i64 count)
+{
+    REQUIRE(count >= 0 && (u64)count < (1ull << 32), XSB_EINVAL, "count must be below 2^32");
+    REQUIRE(h->pending() == 0, XSB_ESTATE, "flush! before freezing the pattern");
+}
+
+// `lookup(slot)` finds the nzval slot of every call of the stream; the entry -> nzval map is built from them
+template <class Lookup> int32_t freeze_impl(xsb_matrix *h, i64 count, Lookup &&lookup)
+{
+    cudaStream_t s = h->stream;
+    i64 *slot = static_cast<i64 *>(h->dalloc(8 * (size_t)count));
+    write_scalar(h, 2, 0);
+    write_scalar(h, 3, ~0ull);
+    lookup(slot);
+    const u64 oob = read_scalar(h, 3);
+    const u64 missing = read_scalar(h, 2);
+    if (oob != ~0ull || missing != 0)
+    {
+        h->dfree(slot);
+        if (oob != ~0ull)
+            throw ApiError(XSB_EBOUNDS, "BoundsError: position " + std::to_string(oob) + " is outside the matrix");
+        throw ApiError(XSB_EILLEGAL, std::to_string(missing) + " positions are not in the frozen pattern");
+    }
+    Rec *A = static_cast<Rec *>(h->dalloc(sizeof(Rec) * (size_t)count));
+    Rec *B = static_cast<Rec *>(h->dalloc(sizeof(Rec) * (size_t)count));
+    void *ws = h->dalloc(sort_workspace_bytes((u64)count));
+    slots_to_records(s, slot, count, A, h->lc);
+    const SortPlan plan = make_sort_plan(0, ceil_log2(std::max<i64>(h->nnz, 2)));
+    Rec *sorted = radix_sort_records(s, A, B, (u64)count, plan, ws, h->lc, nullptr);
+    h->f_perm = static_cast<u32 *>(h->dalloc(4 * (size_t)std::max<i64>(count, 1)));
+    h->f_segstart = static_cast<u32 *>(h->dalloc(4 * (size_t)(h->nnz + 1)));
+    h->f_slot = static_cast<u32 *>(h->dalloc(4 * (size_t)std::max<i64>(count, 1)));
+    build_frozen_map(s, sorted, count, h->nnz, h->f_perm, h->f_segstart, h->f_slot, h->lc);
+    h->dfree(A);
+    h->dfree(B);
+    h->dfree(ws);
+    h->dfree(slot);
+    h->f_count = count;
+    h->frozen = true;
+    h->sync();
+    return XSB_OK;
+}
+
 } // namespace
 
 extern "C" {
@@ -2165,6 +2218,47 @@ int32_t xsb_insert_triplets(xsb_matrix *h, int32_t tid, const xsb_triplet *T, in
     });
 }
 
+int32_t xsb_insert_elements(xsb_matrix *h, int32_t tid, int32_t k, int64_t ncells, const void *dofs, const double *Aloc,
+                            int32_t flavour)
+{
+    return guard(h, [&]() -> int32_t {
+        REQUIRE(h, XSB_EINVAL, "NULL handle");
+        check_tid_flavour(h, tid, flavour);
+        const i64 count = element_calls(k, ncells);
+        if (count == 0)
+            return XSB_OK;
+        REQUIRE(dofs && Aloc, XSB_EINVAL, "NULL array");
+        Rec *dst = begin_emit(h, tid, flavour, count);
+        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells), dA(h, Aloc, 8 * (size_t)count);
+        write_scalar(h, 1, ~0ull);
+        RunTarget rt;
+        u32 chunk0 = 0, pos0 = 0, chunks = 0;
+        const bool grouped = runs_begin(h, tid, count, insert_elements_chunks(k, ncells), &rt, &chunk0, &pos0);
+        const i64 nmax = std::min<i64>(h->m, h->n_global); // a dof is the row and the column of its element's calls
+        if (grouped)
+            chunks = insert_elements_grouped(h->stream, dD.ptr, static_cast<const double *>(dA.ptr), k, ncells, h->idx64,
+                                             h->base, nmax, h->Ls, (u32)tid, (u32)flavour, dst, h->d_scal + 1, h->lc,
+                                             h->stage_flags(tid), rt, chunk0, pos0);
+        else
+            insert_elements(h->stream, dD.ptr, static_cast<const double *>(dA.ptr), k, ncells, h->idx64, h->base, nmax, h->Ls,
+                            (u32)tid, (u32)flavour, dst, h->d_scal + 1, h->lc, h->stage_flags(tid));
+        const u64 bad = read_scalar(h, 1);
+        if (bad != ~0ull)
+        {
+            if (grouped)
+                h->runs.dead = true; // the rejected batch left runs behind: the index is rebuilt at flush time
+            throw ApiError(XSB_EBOUNDS, "BoundsError: element " + std::to_string(bad) +
+                                            " of the batch has a dof outside the matrix; batch rejected");
+        }
+        if (h->n_tid > 1 && flavour == XSB_ASSIGN)
+            check_mt_assign(h, dst, count);
+        end_emit(h, tid, flavour, count);
+        if (grouped)
+            runs_end(h, count, chunks);
+        return XSB_OK;
+    });
+}
+
 int32_t xsb_pending(const xsb_matrix *h, int64_t *count)
 {
     if (!h || !count)
@@ -2240,44 +2334,30 @@ int32_t xsb_freeze_pattern(xsb_matrix *h, const void *I, const void *J, int64_t 
 {
     return guard(h, [&]() -> int32_t {
         REQUIRE(h, XSB_EINVAL, "NULL handle");
-        REQUIRE(count >= 0 && (u64)count < (1ull << 32), XSB_EINVAL, "count must be below 2^32");
-        REQUIRE(h->pending() == 0, XSB_ESTATE, "flush! before freezing the pattern");
+        freeze_check(h, count);
         REQUIRE(count == 0 || (I && J), XSB_EINVAL, "NULL array");
         h->drop_frozen();
-        cudaStream_t s = h->stream;
         DevIn dI(h, I, h->isz() * (size_t)count), dJ(h, J, h->isz() * (size_t)count);
-        i64 *slot = static_cast<i64 *>(h->dalloc(8 * (size_t)count));
-        write_scalar(h, 2, 0);
-        write_scalar(h, 3, ~0ull);
-        lookup_slots(s, h->view(), h->m, h->n, h->idx64, h->base, dI.ptr, dJ.ptr, count, slot, h->d_scal + 2,
-                     h->d_scal + 3, h->lc);
-        const u64 oob = read_scalar(h, 3);
-        const u64 missing = read_scalar(h, 2);
-        if (oob != ~0ull || missing != 0)
-        {
-            h->dfree(slot);
-            if (oob != ~0ull)
-                throw ApiError(XSB_EBOUNDS, "BoundsError: position " + std::to_string(oob) + " is outside the matrix");
-            throw ApiError(XSB_EILLEGAL, std::to_string(missing) + " positions are not in the frozen pattern");
-        }
-        Rec *A = static_cast<Rec *>(h->dalloc(sizeof(Rec) * (size_t)count));
-        Rec *B = static_cast<Rec *>(h->dalloc(sizeof(Rec) * (size_t)count));
-        void *ws = h->dalloc(sort_workspace_bytes((u64)count));
-        slots_to_records(s, slot, count, A, h->lc);
-        const SortPlan plan = make_sort_plan(0, ceil_log2(std::max<i64>(h->nnz, 2)));
-        Rec *sorted = radix_sort_records(s, A, B, (u64)count, plan, ws, h->lc, nullptr);
-        h->f_perm = static_cast<u32 *>(h->dalloc(4 * (size_t)std::max<i64>(count, 1)));
-        h->f_segstart = static_cast<u32 *>(h->dalloc(4 * (size_t)(h->nnz + 1)));
-        h->f_slot = static_cast<u32 *>(h->dalloc(4 * (size_t)std::max<i64>(count, 1)));
-        build_frozen_map(s, sorted, count, h->nnz, h->f_perm, h->f_segstart, h->f_slot, h->lc);
-        h->dfree(A);
-        h->dfree(B);
-        h->dfree(ws);
-        h->dfree(slot);
-        h->f_count = count;
-        h->frozen = true;
-        h->sync();
-        return XSB_OK;
+        return freeze_impl(h, count, [&](i64 *slot) {
+            lookup_slots(h->stream, h->view(), h->m, h->n, h->idx64, h->base, dI.ptr, dJ.ptr, count, slot, h->d_scal + 2,
+                         h->d_scal + 3, h->lc);
+        });
+    });
+}
+
+int32_t xsb_freeze_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs)
+{
+    return guard(h, [&]() -> int32_t {
+        REQUIRE(h, XSB_EINVAL, "NULL handle");
+        const i64 count = element_calls(k, ncells);
+        freeze_check(h, count);
+        REQUIRE(count == 0 || dofs, XSB_EINVAL, "NULL array");
+        h->drop_frozen();
+        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells);
+        return freeze_impl(h, count, [&](i64 *slot) {
+            lookup_slots_elements(h->stream, h->view(), h->m, h->n, h->idx64, h->base, dD.ptr, k, count, slot, h->d_scal + 2,
+                                  h->d_scal + 3, h->lc);
+        });
     });
 }
 

@@ -23,6 +23,7 @@ namespace xsb {
 
 constexpr u32 CH_EMPTY = 0xffffffffu;
 constexpr int CH_RECORDS = 512; // records per chunk of the packing kernels and of the flush-time kernel
+constexpr u32 CH_RUN_MAX = 2047; // records of one run: the count field of the flush's run descriptor (xsb_runs.cu)
 
 template <int HB> struct ChunkSpaceT
 {
@@ -153,16 +154,16 @@ __device__ __forceinline__ u32 chunk_visit_batch(ChunkSpaceT<HB> &ws, u32 g, boo
 }
 
 // offsets of the runs: exclusive sum of the columns' record counts in order of first appearance.
-// MUL: every counted request stands for MUL records (a producer that knows that its records come in groups of
-// MUL per column counts the groups: emit_p1fem_grouped_kernel)
-template <int HB, u32 MUL = 1> __device__ __forceinline__ void chunk_scan(ChunkSpaceT<HB> &ws, u32 d, int lane)
+// mul: every counted request stands for mul records (a producer that knows that its records come in groups of
+// mul per column counts the groups: emit_p1fem_grouped_kernel, 5; insert_elements_kernel, k at run time)
+template <int HB> __device__ __forceinline__ void chunk_scan(ChunkSpaceT<HB> &ws, u32 d, int lane, u32 mul = 1)
 {
     constexpr u32 full = 0xffffffffu;
     const u32 per = (d + 31u) >> 5;
     const u32 j0 = min((u32)lane * per, d), j1 = min(j0 + per, d);
     u32 sum = 0;
     for (u32 j = j0; j < j1; ++j)
-        sum += MUL * ws.cnt[ws.cand[j]];
+        sum += mul * ws.cnt[ws.cand[j]];
     u32 incl = sum;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1)
@@ -176,7 +177,7 @@ template <int HB, u32 MUL = 1> __device__ __forceinline__ void chunk_scan(ChunkS
     {
         const u32 s = ws.cand[j];
         ws.start[s] = (unsigned short)run;
-        run += MUL * ws.cnt[s];
+        run += mul * ws.cnt[s];
     }
     __syncwarp();
 }
@@ -190,9 +191,9 @@ __device__ __forceinline__ u32 chunk_dest(const unsigned short *start, u32 packe
 // completion order, the flush orders the runs of a column by their position in the staging buffer.
 // grouped == false: the chunk gave up (too many distinct columns: no column locality) and was stored
 // in stream order; the flag sends the flush to the radix-sort path.
-template <int HB, u32 MUL = 1>
+template <int HB>
 __device__ __forceinline__ void chunk_publish(ChunkSpaceT<HB> &ws, const RunTarget &rt, u32 chunk, u32 abs_start, u32 d,
-                                              bool grouped, int lane)
+                                              bool grouped, int lane, u32 mul = 1)
 {
     constexpr u32 full = 0xffffffffu;
     u32 base = 0;
@@ -213,7 +214,7 @@ __device__ __forceinline__ void chunk_publish(ChunkSpaceT<HB> &ws, const RunTarg
     {
         const u32 s = ws.cand[j];
         rt.pcol[base + j] = ws.key[s];
-        rt.pinfo[base + j] = ((u32)ws.start[s] << 16) | (MUL * (u32)ws.cnt[s]);
+        rt.pinfo[base + j] = ((u32)ws.start[s] << 16) | (mul * (u32)ws.cnt[s]);
     }
 }
 
@@ -248,6 +249,60 @@ __device__ __forceinline__ void chunk_publish_singletons(const RunTarget &rt, u3
         {
             rt.pcol[base + p] = g[b];
             rt.pinfo[base + p] = (p << 16) | 1u;
+        }
+    }
+}
+
+// chunk_publish for a chunk in which a column holds more than CH_RUN_MAX records (more than a run descriptor
+// counts; insert_elements_kernel with elements that repeat a dof): the column's records, neighbours in the grouped
+// chunk, are published as several runs of at most CH_RUN_MAX records.  The flush orders a column's runs by position,
+// so the pieces keep the records' order.
+template <int HB>
+__device__ __forceinline__ void chunk_publish_split(ChunkSpaceT<HB> &ws, const RunTarget &rt, u32 chunk, u32 abs_start, u32 d,
+                                                    int lane, u32 mul)
+{
+    constexpr u32 full = 0xffffffffu;
+    const u32 per = (d + 31u) >> 5;
+    const u32 j0 = min((u32)lane * per, d), j1 = min(j0 + per, d);
+    u32 sum = 0; // runs of this lane's columns
+    for (u32 j = j0; j < j1; ++j)
+        sum += (mul * ws.cnt[ws.cand[j]] + CH_RUN_MAX - 1u) / CH_RUN_MAX;
+    u32 incl = sum;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1)
+    {
+        const u32 t = __shfl_up_sync(full, incl, o);
+        if (lane >= o)
+            incl += t;
+    }
+    const u32 total = __shfl_sync(full, incl, 31);
+    u32 base = 0;
+    if (lane == 0)
+        base = atomicAdd(rt.counters, total);
+    base = __shfl_sync(full, base, 0);
+    const bool room = (u64)base + total <= (u64)rt.cap;
+    if (lane == 0)
+    {
+        rt.chunkinfo[chunk] = make_uint2(base, room ? total : 0u);
+        rt.chunkstart[chunk] = abs_start;
+        if (!room)
+            atomicOr(rt.counters + 1, 1u);
+    }
+    if (!room)
+        return;
+    u32 q = base + incl - sum;
+    for (u32 j = j0; j < j1; ++j)
+    {
+        const u32 s = ws.cand[j];
+        u32 off = ws.start[s], len = mul * (u32)ws.cnt[s];
+        while (len > 0u)
+        {
+            const u32 piece = min(len, CH_RUN_MAX);
+            rt.pcol[q] = ws.key[s];
+            rt.pinfo[q] = (off << 16) | piece;
+            ++q;
+            off += piece;
+            len -= piece;
         }
     }
 }

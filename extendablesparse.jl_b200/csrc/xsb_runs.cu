@@ -176,6 +176,7 @@ runpair_scan_kernel(const u32 *__restrict__ colpairs, i64 n, u32 *__restrict__ p
 }
 
 // run descriptor: [region rank : 2][position of the run's first record : 32][records : 11]
+static_assert(CH_RUN_MAX < (1u << 11) && CH_RECORDS <= CH_RUN_MAX, "a run's records must fit the descriptor's count");
 __device__ __forceinline__ u64 run_entry(u32 rank, u32 pos, u32 cnt) { return ((u64)rank << 43) | ((u64)pos << 11) | (u64)cnt; }
 
 // A warp drops the pairs of RB_CHUNKS chunks into their columns' buckets; colpairs counts DOWN: afterwards it is zero

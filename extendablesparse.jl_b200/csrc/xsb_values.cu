@@ -68,16 +68,41 @@ __device__ __forceinline__ i64 find_slot(const Ti *__restrict__ colptr, const Ti
     return (lo < end && rowval[lo] == want) ? lo : -1;
 }
 
-template <typename Ti>
+// where the positions of a lookup come from: (I[p], J[p]) arrays, or call p of an element loop
+template <typename Ti> struct PosIJ
+{
+    const Ti *I, *J;
+    __device__ __forceinline__ void at(i64 p, i64 &i, i64 &j) const
+    {
+        i = (i64)I[p];
+        j = (i64)J[p];
+    }
+};
+template <typename Ti> struct PosElements
+{
+    const Ti *dofs; // k x ncells, column-major
+    i64 k;
+    // call p = k^2 c + k jl + il is (dofs[il, c], dofs[jl, c])
+    __device__ __forceinline__ void at(i64 p, i64 &i, i64 &j) const
+    {
+        const i64 kk = k * k, c = p / kk, r = p - c * kk, jl = r / k;
+        i = (i64)dofs[c * k + (r - jl * k)];
+        j = (i64)dofs[c * k + jl];
+    }
+};
+
+template <typename Ti, class Pos>
 __global__ void __launch_bounds__(256)
-lookup_kernel(const Ti *__restrict__ colptr, const Ti *__restrict__ rowval, Ti base, i64 m, i64 n,
-              const Ti *__restrict__ I, const Ti *__restrict__ J, i64 count, i64 *__restrict__ slot,
-              u64 *__restrict__ d_missing, u64 *__restrict__ d_oob)
+lookup_kernel(const Ti *__restrict__ colptr, const Ti *__restrict__ rowval, Ti base, i64 m, i64 n, Pos pos, i64 count,
+              i64 *__restrict__ slot, u64 *__restrict__ d_missing, u64 *__restrict__ d_oob)
 {
     const i64 stride = (i64)gridDim.x * blockDim.x;
     for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < count; k += stride)
     {
-        const i64 i = (i64)I[k] - base, j = (i64)J[k] - base;
+        i64 i, j;
+        pos.at(k, i, j);
+        i -= base;
+        j -= base;
         i64 s = -1;
         if (i < 0 || i >= m || j < 0 || j >= n)
             atomicMin(d_oob, (u64)k);
@@ -91,22 +116,38 @@ lookup_kernel(const Ti *__restrict__ colptr, const Ti *__restrict__ rowval, Ti b
     }
 }
 
-void lookup_slots(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *I,
-                  const void *J, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+template <typename Ti, class Pos>
+static void launch_lookup(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int base, Pos pos, i64 count, i64 *slot,
+                          u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
 {
     if (count <= 0)
         return;
-    const int blocks = grid_for(count, 256);
-    if (idx64)
-        lookup_kernel<int64_t><<<blocks, 256, 0, stream>>>((const int64_t *)csc.colptr, (const int64_t *)csc.rowval,
-                                                           (int64_t)base, m, n, (const int64_t *)I,
-                                                           (const int64_t *)J, count, slot, d_missing, d_oob);
-    else
-        lookup_kernel<int32_t><<<blocks, 256, 0, stream>>>((const int32_t *)csc.colptr, (const int32_t *)csc.rowval,
-                                                           (int32_t)base, m, n, (const int32_t *)I,
-                                                           (const int32_t *)J, count, slot, d_missing, d_oob);
+    lookup_kernel<Ti, Pos><<<grid_for(count, 256), 256, 0, stream>>>((const Ti *)csc.colptr, (const Ti *)csc.rowval, (Ti)base,
+                                                                      m, n, pos, count, slot, d_missing, d_oob);
     lc.add();
     XSB_CUDA(cudaGetLastError());
+}
+
+void lookup_slots(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *I,
+                  const void *J, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+{
+    if (idx64)
+        launch_lookup<int64_t>(stream, csc, m, n, base, PosIJ<int64_t>{(const int64_t *)I, (const int64_t *)J}, count, slot,
+                               d_missing, d_oob, lc);
+    else
+        launch_lookup<int32_t>(stream, csc, m, n, base, PosIJ<int32_t>{(const int32_t *)I, (const int32_t *)J}, count, slot,
+                               d_missing, d_oob, lc);
+}
+
+void lookup_slots_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *dofs,
+                           int k, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+{
+    if (idx64)
+        launch_lookup<int64_t>(stream, csc, m, n, base, PosElements<int64_t>{(const int64_t *)dofs, (i64)k}, count, slot,
+                               d_missing, d_oob, lc);
+    else
+        launch_lookup<int32_t>(stream, csc, m, n, base, PosElements<int32_t>{(const int32_t *)dofs, (i64)k}, count, slot,
+                               d_missing, d_oob, lc);
 }
 
 __global__ void __launch_bounds__(256)

@@ -125,6 +125,9 @@ class DistExtendableSparseMatrix:
     def insert_batch(self, I, J, V, flavour=0):
         self.h.insert_batch(I, J, V, flavour)
 
+    def insert_elements(self, dofs, Aloc, flavour=1):  # XSB_RAW: the element loop's rawupdateindex!
+        self.h.insert_elements(dofs, Aloc, flavour)
+
     def _send_buffer(self, records: int) -> torch.Tensor:
         words = 2 * max(records, 1)
         if self._send is None or self._send.numel() < words:

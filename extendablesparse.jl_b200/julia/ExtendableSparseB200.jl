@@ -218,6 +218,22 @@ function insert!(a::B200Assembler{Tv, Ti}, I::Vector{Ti}, J::Vector{Ti}, V::Vect
                           a.handle, tid, I, J, V, length(V), flavour))
 end
 
+"""
+    insert_elements!(a, dofs, Aloc; flavour = XSB_RAW, tid = 0)
+
+Element loop of test/femtools.jl:45-72 in one call: for every cell `c`, `for jl, for il`,
+`rawupdateindex!(A, +, Aloc[il, jl, c], dofs[il, c], dofs[jl, c])` (or the `flavour`'s call), in that order.
+`dofs` is `cellnodes` (k x ncells), `Aloc` the k x k x ncells element matrices.
+"""
+function insert_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}, Aloc::Array{Tv, 3};
+                          flavour = XSB_RAW, tid = 0) where {Tv, Ti}
+    k = size(dofs, 1)
+    size(Aloc) == (k, k, size(dofs, 2)) || throw(DimensionMismatch("size(Aloc) must be (k, k, size(dofs, 2))"))
+    check(a.handle, ccall((:xsb_insert_elements, libxsb), Int32,
+                          (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Cvoid}, Ptr{Cvoid}, Int32),
+                          a.handle, tid, k, size(dofs, 2), dofs, Aloc, flavour))
+end
+
 "flush! + sparse(A): two-phase -- query nnz, allocate Julia arrays, fetch (ownership stays with Julia)"
 function fetch!(a::B200Assembler{Tv, Ti}, mode = XSB_DETERMINISTIC) where {Tv, Ti}
     nnz = Ref{Int64}(0); changed = Ref{Int32}(0)
@@ -235,6 +251,11 @@ end
 function freeze!(a::B200Assembler{Tv, Ti}, I::Vector{Ti}, J::Vector{Ti}) where {Tv, Ti}
     check(a.handle, ccall((:xsb_freeze_pattern, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int64),
                           a.handle, I, J, length(I)))
+end
+"freeze! for the element loop of insert_elements!: then `reassemble!(a, vec(Aloc))` each step"
+function freeze_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}) where {Tv, Ti}
+    check(a.handle, ccall((:xsb_freeze_elements, libxsb), Int32, (Ptr{Cvoid}, Int32, Int64, Ptr{Cvoid}),
+                          a.handle, size(dofs, 1), size(dofs, 2), dofs))
 end
 function reassemble!(a::B200Assembler{Tv}, V::Vector{Tv}; mode = XSB_DETERMINISTIC, zero = true) where {Tv}
     # zero = true: nonzeros(A) .= 0 and the re-assembly as ONE pass over nzval (xsb_reassemble_values_zeroed)
@@ -319,6 +340,6 @@ end
 
 export peer_exchange!, route_step!, peer_exchange_close!
 export SparseMatrixB200, B200Assembler, pattern_equal, B200ExtendableSparseMatrixCSC, STB200ExtendableSparseMatrixCSC,
-       set_csc!, insert!, fetch!, freeze!, reassemble!, pointblock, XsbTriplet
+       set_csc!, insert!, insert_elements!, fetch!, freeze!, freeze_elements!, reassemble!, pointblock, XsbTriplet
 
 end # module

@@ -115,6 +115,13 @@ class ExtendableSparseMatrix:
         self._ship(tid)
         self._h.insert_batch(I, J, V, flavour, tid)
 
+    def insert_elements(self, dofs, Aloc, flavour=capi.RAW, tid=0):
+        """Element loop (test/femtools.jl:45-72): for every element c, for jl, for il,
+        rawupdateindex!(A, +, Aloc[c, jl, il], dofs[c, il], dofs[c, jl]) (or the `flavour`'s call).
+        dofs (ncells, k), 1-based; Aloc (ncells, k, k)."""
+        self._ship(tid)
+        self._h.insert_elements(dofs, Aloc, flavour, tid)
+
     # -- flush!/sparse/nnz/reset!
     def flush(self):
         for t in range(self._n_tid):

@@ -176,6 +176,20 @@ typedef struct xsb_triplet
 } xsb_triplet;
 int32_t xsb_insert_triplets(xsb_matrix *h, int32_t tid, const xsb_triplet *T, int64_t count, int32_t flavour);
 
+/* k*k*ncells calls of updateindex!/rawupdateindex!/setindex!(A,[+,]v,i,j[,tid]) of an element loop
+ * (test/femtools.jl:45-72), given as connectivity and dense element matrices, Julia's column-major arrays:
+ *   dofs  k x ncells, the handle's idx_type and index_base: dofs[l + k*c] = cellnodes[l+1, c+1];
+ *   Aloc  k x k x ncells Float64:                         Aloc[il + k*jl + k*k*c] = Aloc[il+1, jl+1, c+1].
+ * Value p of Aloc in memory order is call p: (row = dofs[il,c], col = dofs[jl,c], v = Aloc[il,jl,c]) -- elements
+ * in order, inside an element column by column, inside a column row by row.  The result equals xsb_insert_batch of
+ * that expanded stream bit for bit (any flavour, tid, slab handle -- global dofs --, host or device pointers), and
+ * xsb_reassemble_values[_zeroed](h, Aloc, k*k*ncells, mode) after xsb_freeze_elements takes Aloc unchanged.
+ * 1 <= k <= 64, else XSB_EINVAL.  A dof outside the matrix rejects the whole batch with XSB_EBOUNDS; the message
+ * names the first offending element by its position in the batch.  The staging follows the handle's precount and
+ * grouping settings like the emitters: whole elements are grouped by column while they are staged. */
+int32_t xsb_insert_elements(xsb_matrix *h, int32_t tid, int32_t k, int64_t ncells, const void *dofs, const double *Aloc,
+                            int32_t flavour);
+
 /* Number of staged insertions (an upper bound of nnznew(A), genericextendable...:21). */
 int32_t xsb_pending(const xsb_matrix *h, int64_t *count);
 
@@ -279,6 +293,9 @@ int32_t xsb_route_unpack_peer(xsb_matrix *h);
  * (the CSC-hit branch extendable.jl:164-166 resolved once instead of per insert).
  * Every (i,j) must already be in the pattern, else XSB_EILLEGAL. */
 int32_t xsb_freeze_pattern(xsb_matrix *h, const void *I, const void *J, int64_t count);
+/* xsb_freeze_pattern for the stream xsb_insert_elements(h, ., k, ncells, dofs, ., .) would stage: the element
+ * loop's positions from its connectivity alone; errors as xsb_freeze_pattern (XSB_EBOUNDS names the call). */
+int32_t xsb_freeze_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs);
 /* nzval[slot(k)] += V[k] for the frozen stream; deterministic mode folds every entry's values in stream order,
  * starting from the resident value (bit-exact with the in-place CSC-hit updates); fast mode is one atomic add
  * per insertion through the 4-byte entry -> nzval map. */
