@@ -828,15 +828,15 @@ void ora_mt_destroy(ora_mt *e)
     free(e);
 }
 
-/* rawupdateindex!/updateindex!(ext,+,v,i,j,tid): genericmt...:87-114; tid is 1-based */
+/* rawupdateindex!/updateindex!(ext,+,v,i,j,tid): genericmt...:87-114, setindex!: :63-68; tid is 1-based */
 int ora_mt_update(ora_mt *e, double v, i64 i, i64 j, i64 tid, int flavour)
 {
     i64 k = csc_findindex(e->csc, i, j);
     if (k < 0 || tid < 1 || tid > e->np)
         return ORA_EBOUNDS;
     if (k > 0)
-    {
-        e->csc->nzval[k - 1] = e->csc->nzval[k - 1] + v;
+    { /* setindex! of a stored entry overwrites it */
+        e->csc->nzval[k - 1] = flavour == ORA_ASSIGN ? v : e->csc->nzval[k - 1] + v;
         return ORA_OK;
     }
     if (flavour == ORA_ASSIGN)

@@ -285,6 +285,19 @@ def test_mt_matches_ext(oracle):
     assert np.array_equal(A3.csc()[2], A0.csc()[2])
 
 
+def test_mt_setindex_of_stored_entry_overwrites(oracle):
+    """setindex! of an entry the CSC already holds overwrites it (genericmt...:63-68); a new one is an error.
+    The oracle used to add the value, which the GPU key-layout tests caught."""
+    A = oracle.OracleMT(3, 3, 2)
+    A.update(1.5, 2, 2, 1, oracle.RAW)
+    A.flush()
+    A.update(4.0, 2, 2, 2, oracle.ASSIGN)
+    A.update(0.5, 2, 2, 1, oracle.UPDATE)
+    assert A.csc()[2].tolist() == [4.5]
+    with pytest.raises(RuntimeError):
+        A.update(1.0, 1, 1, 1, oracle.ASSIGN)
+
+
 def test_mt_threaded_matches_serial(oracle):
     """testassemble_parallel! (test/femtools.jl:75-110): partitions of a colour inserted by concurrent
     threads give the bits of the serial tid-wise insertion; second assembly = CSC hits only."""
