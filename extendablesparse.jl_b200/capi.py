@@ -120,6 +120,13 @@ SIGNATURES = {
     "xsb_reassemble_values": (_i32, [_p, _p, _i64, _i32]),
     "xsb_reassemble_values_zeroed": (_i32, [_p, _p, _i64, _i32]),
     "xsb_unfreeze": (_i32, [_p]),
+    "xsb_freeze_slab": (_i32, [_p, _p, _p, _i64, C.POINTER(_i64)]),
+    "xsb_freeze_slab_elements": (_i32, [_p, _i32, _i64, _p, C.POINTER(_i64)]),
+    "xsb_freeze_slab_prepare": (_i32, [_p, _p, _i64]),
+    "xsb_freeze_slab_finish": (_i32, [_p, _p, C.POINTER(_i64)]),
+    "xsb_frozen_slab_counts": (_i32, [_p, C.POINTER(_i64), C.POINTER(_i64)]),
+    "xsb_reassemble_slab_pack": (_i32, [_p, _p, _i64, _p]),
+    "xsb_reassemble_slab_values": (_i32, [_p, _p, _i64, _p, _i32, _i32]),
     "xsb_mark_dirichlet": (_i32, [_p, _f64, _p]),
     "xsb_eliminate_dirichlet": (_i32, [_p, _p]),
     "xsb_pattern_hash": (_i32, [_p, C.POINTER(_u64)]),
@@ -431,6 +438,64 @@ class Handle:
 
     def unfreeze(self):
         self._c(lib().xsb_unfreeze(self._h))
+
+    # a stream of GLOBAL positions frozen across column slabs (see include/xsparse_b200.h, xsb_freeze_slab)
+    def _rank_counts(self):
+        return (_i64 * max(getattr(self, "n_ranks", 1), 1))()
+
+    def freeze_slab(self, I, J, count=None):
+        """First step of the slab freeze: returns the positions per owning rank (own rank: the ones kept)."""
+        I = np.ascontiguousarray(I, self.idx_dtype) if not hasattr(I, "data_ptr") else I
+        J = np.ascontiguousarray(J, self.idx_dtype) if not hasattr(J, "data_ptr") else J
+        if count is None:
+            count = len(I)
+        counts = self._rank_counts()
+        self._c(lib().xsb_freeze_slab(self._h, ptr(I), ptr(J), count, counts))
+        return [int(c) for c in counts]
+
+    def freeze_slab_elements(self, dofs):
+        """freeze_slab for the stream insert_elements(dofs, .) stages ((ncells, k) connectivity)."""
+        dofs, _, ncells, k = self._element_arrays(dofs)
+        counts = self._rank_counts()
+        self._c(lib().xsb_freeze_slab_elements(self._h, k, ncells, ptr(dofs), counts))
+        return [int(c) for c in counts]
+
+    def freeze_slab_prepare(self, send_positions, capacity):
+        """The foreign positions (8 bytes each: u32 row, u32 owner-relative column), destination after destination,
+        into device memory."""
+        self._c(lib().xsb_freeze_slab_prepare(self._h, ptr(send_positions), int(capacity)))
+
+    def freeze_slab_finish(self, recv_positions, recv_counts):
+        """The received positions, sources ascending (own rank left out); completes the freeze."""
+        arr = self._rank_counts()
+        for r, c in enumerate(recv_counts):
+            arr[r] = int(c)
+        self._c(lib().xsb_freeze_slab_finish(self._h, ptr(recv_positions), arr))
+
+    def frozen_slab_counts(self):
+        """(send_counts, recv_counts) of the per-step exchange of a frozen slab stream."""
+        s, r = self._rank_counts(), self._rank_counts()
+        self._c(lib().xsb_frozen_slab_counts(self._h, s, r))
+        return [int(c) for c in s], [int(c) for c in r]
+
+    def reassemble_slab_pack(self, V, send_values, count=None):
+        """The values of the foreign positions into send_values (device float64), laid out as at prepare."""
+        if isinstance(V, np.ndarray):
+            V = np.ascontiguousarray(V, np.float64)
+        if count is None:
+            count = len(V)
+        self._c(lib().xsb_reassemble_slab_pack(self._h, ptr(V), count, ptr(send_values)))
+
+    def reassemble_slab_values(self, V, recv_values, mode=DETERMINISTIC, zero_first=False, count=None):
+        """Own values V (one per position of the frozen stream) and the received ones folded into the slab."""
+        if isinstance(V, np.ndarray):
+            V = np.ascontiguousarray(V, np.float64)
+        if isinstance(recv_values, np.ndarray):
+            recv_values = np.ascontiguousarray(recv_values, np.float64)
+        if count is None:
+            count = len(V)
+        self._c(lib().xsb_reassemble_slab_values(self._h, ptr(V), count, ptr(recv_values), int(mode),
+                                                 int(bool(zero_first))))
 
     def mark_dirichlet(self, penalty=1.0e20):
         mk = np.zeros(self.n, np.uint8)

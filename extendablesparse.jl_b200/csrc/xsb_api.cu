@@ -97,6 +97,15 @@ struct xsb_matrix
     u32 *f_slot = nullptr;     // 4-byte entry -> nzval map of the frozen stream (fast mode)
     u32 *f_perm = nullptr;     // stream positions in nzval order (deterministic mode)
     u32 *f_segstart = nullptr; // first of them per nzval entry
+    // stream frozen across column slabs (xsb_freeze_slab*): global positions, those in other ranks' columns travel
+    // to their owner.  The map above then indexes [received from lower ranks | own stream | from higher ranks].
+    int fs_state = 0;                  // 0: none, 1: half frozen (until xsb_freeze_slab_finish), 2: frozen
+    i64 fs_send[kMaxRanks] = {0};      // positions per owner (own rank: the ones kept)
+    i64 fs_recv[kMaxRanks] = {0};      // positions received per source (own rank: 0)
+    i64 fs_foreign = 0, fs_low = 0, fs_total = 0; // sent; received from lower ranks; size of the combined space
+    u32 *fs_send_idx = nullptr;        // stream indices of the sent positions, destination after destination
+    u64 *fs_send_pos = nullptr;        // their {row, owner-relative column} (until the freeze is complete)
+    i64 *fs_slot = nullptr;            // nzval slot per own stream position, -1: foreign (until complete)
 
     double *blocks = nullptr; // result handle of xsb_pointblock: nnz dense bs x bs blocks, column-major, CSC order
     int block_size = 0;
@@ -250,6 +259,22 @@ struct xsb_matrix
         f_segstart = nullptr;
         frozen = false;
         f_count = 0;
+        dfree(fs_send_idx);
+        dfree(fs_send_pos);
+        dfree(fs_slot);
+        fs_send_idx = nullptr;
+        fs_send_pos = nullptr;
+        fs_slot = nullptr;
+        fs_state = 0;
+        fs_foreign = fs_low = fs_total = 0;
+        for (int r = 0; r < kMaxRanks; ++r)
+            fs_send[r] = fs_recv[r] = 0;
+    }
+    // insertions and flushes abandon a slab freeze that is still waiting for xsb_freeze_slab_finish
+    void drop_half_freeze()
+    {
+        if (fs_state == 1)
+            drop_frozen();
     }
     void clear_staging(bool release)
     {
@@ -737,6 +762,7 @@ int32_t do_flush(xsb_matrix *h, int32_t mode, int32_t combine, int64_t *nnz_out,
     REQUIRE(mode == XSB_DETERMINISTIC || mode == XSB_FAST, XSB_EINVAL, "unknown summation mode");
     REQUIRE(combine == XSB_COMBINE_SEED || combine == XSB_COMBINE_ADD, XSB_EINVAL, "unknown combine mode");
     const i64 n_ins = h->pending();
+    h->drop_half_freeze();
     h->lc.in_flush = 0;
     h->alloc_ms = 0.f;
     std::memset(&h->stats, 0, sizeof(h->stats));
@@ -1163,6 +1189,7 @@ Rec *begin_emit(xsb_matrix *h, int32_t tid, int32_t flavour, i64 count)
     check_tid_flavour(h, tid, flavour);
     REQUIRE(count >= 0, XSB_EINVAL, "negative count");
     REQUIRE(!h->routed, XSB_ESTATE, "routed records are pending: flush before inserting again");
+    h->drop_half_freeze();
     h->ensure_stage(tid, count);
     Stage &st = h->stage[tid];
     return st.buf + st.front + st.count;
@@ -1258,6 +1285,70 @@ template <class Lookup> int32_t freeze_impl(xsb_matrix *h, i64 count, Lookup &&l
     h->dfree(slot);
     h->f_count = count;
     h->frozen = true;
+    h->sync();
+    return XSB_OK;
+}
+
+// the calls of a stream frozen across column slabs
+void slab_freeze_check(xsb_matrix *h)
+{
+    REQUIRE(h, XSB_EINVAL, "NULL handle");
+    REQUIRE(h->nranks > 0, XSB_ESTATE, "not a slab handle");
+    REQUIRE(h->pending() == 0, XSB_ESTATE, "insertions are pending: flush! first");
+}
+
+// xsb_freeze_slab / xsb_freeze_slab_elements: `classify(slot, tags)` resolves the own positions and tags every
+// position with its owner; the stable copy-out of the routing (xsb_route.cu, on a layout whose owner field starts at
+// bit 32 above the stream index) gathers the foreign ones destination after destination.  Leaves the handle half
+// frozen.
+template <class Classify> int32_t freeze_slab_impl(xsb_matrix *h, i64 count, int64_t *send_counts, Classify &&classify)
+{
+    cudaStream_t s = h->stream;
+    const size_t room = (size_t)std::max<i64>(count, 1);
+    i64 *slot = static_cast<i64 *>(h->dalloc(8 * room));
+    Rec *tags = static_cast<Rec *>(h->dalloc(sizeof(Rec) * room));
+    write_scalar(h, 2, 0);
+    write_scalar(h, 3, ~0ull);
+    classify(slot, tags);
+    const u64 oob = read_scalar(h, 3);
+    const u64 missing = read_scalar(h, 2);
+    if (oob != ~0ull || missing != 0)
+    {
+        h->dfree(slot);
+        h->dfree(tags);
+        if (oob != ~0ull)
+            throw ApiError(XSB_EBOUNDS, "BoundsError: position " + std::to_string(oob) + " of the stream is outside the matrix");
+        throw ApiError(XSB_EILLEGAL, std::to_string(missing) + " positions in this rank's columns are not in the frozen pattern");
+    }
+    KeyLayout Lr = h->L; // owner field at bit 32, the stream index below it
+    Lr.low = 32;
+    Lr.tidbits = Lr.rowbits = Lr.colbits = 0;
+    void *ws = h->dalloc(route_workspace_bytes((u64)room, h->nranks));
+    u64 counts[kMaxRanks] = {0};
+    route_count(s, tags, (u64)count, Lr, ws, counts, h->lc);
+    i64 foreign = 0;
+    for (int r = 0; r < h->nranks; ++r)
+        if (r != h->rank)
+            foreign += (i64)counts[r];
+    const size_t froom = (size_t)std::max<i64>(foreign, 1);
+    Rec *gathered = static_cast<Rec *>(h->dalloc(sizeof(Rec) * froom));
+    route_extract(s, tags, (u64)count, Lr, ws, counts, gathered, h->lc);
+    h->fs_send_idx = static_cast<u32 *>(h->dalloc(4 * froom));
+    h->fs_send_pos = static_cast<u64 *>(h->dalloc(8 * froom));
+    slab_split(s, gathered, foreign, h->fs_send_idx, h->fs_send_pos, h->lc);
+    h->dfree(gathered);
+    h->dfree(ws);
+    h->dfree(tags);
+    h->fs_slot = slot;
+    for (int r = 0; r < h->nranks; ++r)
+    {
+        h->fs_send[r] = (i64)counts[r];
+        if (send_counts)
+            send_counts[r] = (int64_t)counts[r];
+    }
+    h->fs_foreign = foreign;
+    h->f_count = count;
+    h->fs_state = 1;
     h->sync();
     return XSB_OK;
 }
@@ -2366,6 +2457,8 @@ static int32_t reassemble_impl(xsb_matrix *h, const void *V, int64_t count, int3
     return guard(h, [&]() -> int32_t {
         REQUIRE(h, XSB_EINVAL, "NULL handle");
         REQUIRE(h->frozen, XSB_ESTATE, "no frozen pattern");
+        REQUIRE(h->fs_state == 0, XSB_ESTATE,
+                "the frozen stream spans column slabs: re-assemble with xsb_reassemble_slab_pack / _values");
         REQUIRE(count == h->f_count, XSB_ESIZE, "value count differs from the frozen stream");
         REQUIRE(mode == XSB_DETERMINISTIC || mode == XSB_FAST, XSB_EINVAL, "unknown summation mode");
         if (count == 0)
@@ -2404,6 +2497,194 @@ int32_t xsb_unfreeze(xsb_matrix *h)
     return guard(h, [&]() -> int32_t {
         REQUIRE(h, XSB_EINVAL, "NULL handle");
         h->drop_frozen();
+        return XSB_OK;
+    });
+}
+
+int32_t xsb_freeze_slab(xsb_matrix *h, const void *I, const void *J, int64_t count, int64_t *send_counts)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_freeze_check(h);
+        freeze_check(h, count);
+        REQUIRE(count == 0 || (I && J), XSB_EINVAL, "NULL array");
+        h->drop_frozen();
+        DevIn dI(h, I, h->isz() * (size_t)count), dJ(h, J, h->isz() * (size_t)count);
+        return freeze_slab_impl(h, count, send_counts, [&](i64 *slot, Rec *tags) {
+            slab_classify(h->stream, h->view(), h->m, h->n_global, h->Ls, h->idx64, h->base, dI.ptr, dJ.ptr, count, slot,
+                          tags, h->d_scal + 2, h->d_scal + 3, h->lc);
+        });
+    });
+}
+
+int32_t xsb_freeze_slab_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs, int64_t *send_counts)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_freeze_check(h);
+        const i64 count = element_calls(k, ncells);
+        freeze_check(h, count);
+        REQUIRE(count == 0 || dofs, XSB_EINVAL, "NULL array");
+        h->drop_frozen();
+        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells);
+        return freeze_slab_impl(h, count, send_counts, [&](i64 *slot, Rec *tags) {
+            slab_classify_elements(h->stream, h->view(), h->m, h->n_global, h->Ls, h->idx64, h->base, dD.ptr, k, count,
+                                   slot, tags, h->d_scal + 2, h->d_scal + 3, h->lc);
+        });
+    });
+}
+
+int32_t xsb_freeze_slab_prepare(xsb_matrix *h, void *send_positions, int64_t capacity)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_freeze_check(h);
+        REQUIRE(h->fs_state == 1, XSB_ESTATE, "no slab freeze in progress: xsb_freeze_slab first");
+        REQUIRE(capacity >= h->fs_foreign, XSB_EINVAL,
+                "send buffer too small: " + std::to_string(h->fs_foreign) + " positions leave this rank");
+        REQUIRE(h->fs_foreign == 0 || (send_positions && is_device_ptr(send_positions)), XSB_EINVAL,
+                "send buffer must be device memory");
+        if (h->fs_foreign > 0)
+            XSB_CUDA(cudaMemcpyAsync(send_positions, h->fs_send_pos, 8 * (size_t)h->fs_foreign, cudaMemcpyDeviceToDevice,
+                                     h->stream));
+        h->sync();
+        return XSB_OK;
+    });
+}
+
+int32_t xsb_freeze_slab_finish(xsb_matrix *h, const void *recv_positions, const int64_t *recv_counts)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_freeze_check(h);
+        REQUIRE(h->fs_state == 1, XSB_ESTATE, "no slab freeze in progress: xsb_freeze_slab first");
+        try
+        {
+            REQUIRE(recv_counts, XSB_EINVAL, "NULL recv_counts");
+            i64 low = 0, high = 0;
+            for (int r = 0; r < h->nranks; ++r)
+            {
+                if (r == h->rank)
+                    continue;
+                REQUIRE(recv_counts[r] >= 0 && recv_counts[r] < ((i64)1 << 32), XSB_EINVAL, "bad receive count");
+                (r < h->rank ? low : high) += recv_counts[r];
+            }
+            const i64 own = h->f_count, total = low + own + high;
+            REQUIRE((u64)total < (1ull << 32), XSB_EINVAL,
+                    "received positions plus the own stream must stay below 2^32 (the map indexes values with 32 bits)");
+            REQUIRE(low + high == 0 || (recv_positions && is_device_ptr(recv_positions)), XSB_EINVAL,
+                    "receive buffer must be device memory");
+            cudaStream_t s = h->stream;
+            const size_t room = (size_t)std::max<i64>(total, 1);
+            Rec *A = static_cast<Rec *>(h->dalloc(sizeof(Rec) * room));
+            write_scalar(h, 2, 0);
+            write_scalar(h, 3, ~0ull);
+            slab_records(s, h->view(), h->m, h->n, h->idx64, h->base, h->fs_slot, own, recv_positions, low, total, A,
+                         h->d_scal + 2, h->d_scal + 3, h->lc);
+            const u64 oob = read_scalar(h, 3);
+            const u64 missing = read_scalar(h, 2);
+            if (oob != ~0ull || missing != 0)
+            {
+                h->dfree(A);
+                if (oob != ~0ull)
+                    throw ApiError(XSB_EBOUNDS,
+                                   "BoundsError: received position " + std::to_string(oob) + " is outside this rank's slab");
+                throw ApiError(XSB_EILLEGAL, std::to_string(missing) + " received positions are not in the frozen pattern");
+            }
+            // foreign own positions carry slot nnz: they sort behind every real slot and stay out of the map
+            const i64 nmap = total - h->fs_foreign;
+            Rec *B = static_cast<Rec *>(h->dalloc(sizeof(Rec) * room));
+            void *ws = h->dalloc(sort_workspace_bytes((u64)total));
+            const SortPlan plan = make_sort_plan(0, ceil_log2(std::max<i64>(h->nnz + 1, 2)));
+            Rec *sorted = radix_sort_records(s, A, B, (u64)total, plan, ws, h->lc, nullptr);
+            h->f_perm = static_cast<u32 *>(h->dalloc(4 * (size_t)std::max<i64>(nmap, 1)));
+            h->f_segstart = static_cast<u32 *>(h->dalloc(4 * (size_t)(h->nnz + 1)));
+            h->f_slot = static_cast<u32 *>(h->dalloc(4 * room));
+            XSB_CUDA(cudaMemsetAsync(h->f_slot, 0xff, 4 * room, s)); // kNoSlot where build_frozen_map writes nothing
+            build_frozen_map(s, sorted, nmap, h->nnz, h->f_perm, h->f_segstart, h->f_slot, h->lc);
+            h->dfree(A);
+            h->dfree(B);
+            h->dfree(ws);
+            h->dfree(h->fs_slot);
+            h->dfree(h->fs_send_pos);
+            h->fs_slot = nullptr;
+            h->fs_send_pos = nullptr;
+            for (int r = 0; r < h->nranks; ++r)
+                h->fs_recv[r] = r == h->rank ? 0 : (i64)recv_counts[r];
+            h->fs_low = low;
+            h->fs_total = total;
+            h->frozen = true;
+            h->fs_state = 2;
+            h->sync();
+        }
+        catch (...)
+        {
+            h->drop_frozen();
+            throw;
+        }
+        return XSB_OK;
+    });
+}
+
+int32_t xsb_frozen_slab_counts(const xsb_matrix *hc, int64_t *send_counts, int64_t *recv_counts)
+{
+    xsb_matrix *h = const_cast<xsb_matrix *>(hc);
+    return guard(h, [&]() -> int32_t {
+        REQUIRE(h, XSB_EINVAL, "NULL handle");
+        REQUIRE(h->nranks > 0, XSB_ESTATE, "not a slab handle");
+        REQUIRE(h->fs_state == 2, XSB_ESTATE, "no frozen slab stream");
+        for (int r = 0; r < h->nranks; ++r)
+        {
+            if (send_counts)
+                send_counts[r] = h->fs_send[r];
+            if (recv_counts)
+                recv_counts[r] = h->fs_recv[r];
+        }
+        return XSB_OK;
+    });
+}
+
+namespace
+{
+void slab_step_check(xsb_matrix *h, int64_t count)
+{
+    slab_freeze_check(h);
+    REQUIRE(h->fs_state == 2, XSB_ESTATE,
+            h->fs_state == 1 ? "the slab freeze is not complete: xsb_freeze_slab_finish first" : "no frozen slab stream");
+    REQUIRE(count == h->f_count, XSB_ESIZE, "value count differs from the frozen stream");
+}
+} // namespace
+
+int32_t xsb_reassemble_slab_pack(xsb_matrix *h, const double *V, int64_t count, double *send_values)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_step_check(h, count);
+        if (h->fs_foreign == 0)
+            return XSB_OK;
+        REQUIRE(V, XSB_EINVAL, "NULL array");
+        REQUIRE(send_values && is_device_ptr(send_values), XSB_EINVAL, "send buffer must be device memory");
+        DevIn dV(h, V, 8 * (size_t)count);
+        slab_pack_values(h->stream, static_cast<const double *>(dV.ptr), h->fs_send_idx, h->fs_foreign, send_values, h->lc);
+        return XSB_OK;
+    });
+}
+
+int32_t xsb_reassemble_slab_values(xsb_matrix *h, const double *V, int64_t count, const double *recv_values, int32_t mode,
+                                   int32_t zero_first)
+{
+    return guard(h, [&]() -> int32_t {
+        slab_step_check(h, count);
+        REQUIRE(mode == XSB_DETERMINISTIC || mode == XSB_FAST, XSB_EINVAL, "unknown summation mode");
+        const i64 nrecv = h->fs_total - h->f_count;
+        REQUIRE(count == 0 || V, XSB_EINVAL, "NULL array");
+        REQUIRE(nrecv == 0 || recv_values, XSB_EINVAL, "NULL receive buffer");
+        DevIn dV(h, V, 8 * (size_t)count), dR(h, recv_values, 8 * (size_t)nrecv);
+        const SlabValues sv{static_cast<const double *>(dR.ptr), (u32)h->fs_low, (u32)h->f_count};
+        const double *v = static_cast<const double *>(dV.ptr);
+        if (mode == XSB_DETERMINISTIC)
+            reassemble_deterministic(h->stream, v, h->f_perm, h->f_segstart, h->nnz, h->nzval, zero_first != 0, h->lc, &sv);
+        else
+        {
+            if (zero_first)
+                zero_values(h->stream, h->nzval, h->nnz, h->lc);
+            reassemble_fast(h->stream, v, h->f_slot, h->fs_total, h->nzval, h->lc, &sv);
+        }
         return XSB_OK;
     });
 }

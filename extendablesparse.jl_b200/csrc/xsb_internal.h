@@ -304,10 +304,38 @@ void count_missing_records(cudaStream_t stream, const Rec *recs, i64 count, cons
 void slots_to_records(cudaStream_t stream, const i64 *slot, i64 count, Rec *out, LaunchCounter &lc);
 void build_frozen_map(cudaStream_t stream, const Rec *sorted, i64 count, i64 nnz, u32 *perm, u32 *segstart, u32 *slot32,
                       LaunchCounter &lc);
+// A stream frozen across column slabs (xsb_freeze_slab*): the map indexes the combined space [received from lower
+// ranks | own stream | received from higher ranks].  Index k < low: recv[k]; low <= k < low + own: V[k - low] (the
+// caller's values, read in place); else recv[k - own].  In the fast map the own positions that other ranks own
+// carry kNoSlot.
+struct SlabValues
+{
+    const double *recv;
+    u32 low, own;
+};
+constexpr u32 kNoSlot = 0xffffffffu;
+// sv == nullptr: plain frozen stream, V indexed by stream position
 void reassemble_deterministic(cudaStream_t stream, const double *V, const u32 *perm, const u32 *segstart, i64 nnz,
-                              double *nzval, bool zero_first, LaunchCounter &lc);
+                              double *nzval, bool zero_first, LaunchCounter &lc, const SlabValues *sv = nullptr);
 void reassemble_fast(cudaStream_t stream, const double *V, const u32 *slot, i64 count, double *nzval,
-                     LaunchCounter &lc);
+                     LaunchCounter &lc, const SlabValues *sv = nullptr);
+// slab freeze, one pass over the stream: global bounds (*d_oob: first bad position), owner, own positions -> slot[k]
+// (nzval slot, -1 when absent: *d_missing), every position -> tags[k] {owner << 32 | k, row | column in the owner's
+// slab << 32} for the stable copy-out of route_count / route_extract (layout with ownershift 32)
+void slab_classify(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64, int base,
+                   const void *I, const void *J, i64 count, i64 *slot, Rec *tags, u64 *d_missing, u64 *d_oob,
+                   LaunchCounter &lc);
+void slab_classify_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64,
+                            int base, const void *dofs, int k, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
+                            u64 *d_oob, LaunchCounter &lc);
+// gathered tags -> stream indices and {row, column} positions
+void slab_split(cudaStream_t stream, const Rec *tags, i64 n, u32 *idx, u64 *where, LaunchCounter &lc);
+// (slot, combined index) records of the combined space; received positions recv[q] = {row, slab column}
+// (*d_oob: first bad q, *d_missing: absent ones); slot nnz = no entry of the map
+void slab_records(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const i64 *own_slot, i64 own,
+                  const void *recv, i64 low, i64 total, Rec *out, u64 *d_missing, u64 *d_oob, LaunchCounter &lc);
+// send[q] = V[idx[q]]
+void slab_pack_values(cudaStream_t stream, const double *V, const u32 *idx, i64 n, double *send, LaunchCounter &lc);
 void mark_dirichlet(cudaStream_t stream, const CscView &csc, i64 n, int idx64, int base, double penalty,
                     unsigned char *marker, LaunchCounter &lc);
 void eliminate_dirichlet(cudaStream_t stream, const CscView &csc, i64 n, int idx64, int base,

@@ -271,16 +271,29 @@ void build_frozen_map(cudaStream_t stream, const Rec *sorted, i64 count, i64 nnz
     XSB_CUDA(cudaGetLastError());
 }
 
+// Where value k of a re-assembly lives.  Plain handles: V[k].  SLAB (a stream frozen across column slabs): k runs
+// over the combined index space [received from lower ranks | own stream | received from higher ranks], whose parts
+// sit in two arrays -- the received values and the caller's V, which is read in place.
+template <bool SLAB>
+__device__ __forceinline__ const double *value_at(const double *V, const SlabValues &sv, u32 k)
+{
+    if constexpr (!SLAB)
+        return V + k;
+    else
+        return k < sv.low ? sv.recv + k : (k - sv.low < sv.own ? V + (k - sv.low) : sv.recv + (k - sv.own));
+}
+
 // nzval[z] = ((nzval[z] + V[p0]) + V[p1]) + ...  in stream order: bit-exact with the reference's in-place CSC-hit
 // updates (extendable.jl:164-166).  One thread per entry walks its piece of the permutation built at freeze time.
 // The gathers of V go through L1: the threads of a block hold consecutive entries (a few dozen neighbouring columns),
 // whose values come from a few short windows of the stream, so the 32-byte sectors of V are shared inside the block
 // and HBM sees every value about once.  ZERO: the entries start from +0.0 instead of the resident value
-// (nonzeros(A) .= 0 fused in: nzval is written, never read).
-template <bool ZERO>
+// (nonzeros(A) .= 0 fused in: nzval is written, never read).  `sv` comes last so that the plain instantiations keep
+// the parameter layout (and the code) they had before slab streams existed.
+template <bool ZERO, bool SLAB>
 __global__ void __launch_bounds__(256)
 reassemble_det_kernel(const double *__restrict__ V, const u32 *__restrict__ perm, const u32 *__restrict__ segstart,
-                      i64 nnz, double *__restrict__ nzval)
+                      i64 nnz, double *__restrict__ nzval, SlabValues sv)
 {
     const i64 stride = (i64)gridDim.x * blockDim.x;
     for (i64 z = (i64)blockIdx.x * blockDim.x + threadIdx.x; z < nnz; z += stride)
@@ -296,46 +309,243 @@ reassemble_det_kernel(const double *__restrict__ V, const u32 *__restrict__ perm
         u32 s = s0;
         for (; s + 2 <= s1; s += 2)
         { // two gathers in flight, folded in order
-            const double v0 = __ldg(V + perm[s]), v1 = __ldg(V + perm[s + 1]);
+            const double v0 = __ldg(value_at<SLAB>(V, sv, perm[s])), v1 = __ldg(value_at<SLAB>(V, sv, perm[s + 1]));
             acc = acc + v0;
             acc = acc + v1;
         }
         if (s < s1)
-            acc = acc + __ldg(V + perm[s]);
+            acc = acc + __ldg(value_at<SLAB>(V, sv, perm[s]));
         nzval[z] = acc;
     }
 }
 
 void reassemble_deterministic(cudaStream_t stream, const double *V, const u32 *perm, const u32 *segstart, i64 nnz,
-                              double *nzval, bool zero_first, LaunchCounter &lc)
+                              double *nzval, bool zero_first, LaunchCounter &lc, const SlabValues *sv)
 {
     if (nnz <= 0)
         return;
     const int blocks = (int)std::min<i64>((nnz + 255) / 256, (i64)kNumSM * 64);
-    if (zero_first)
-        reassemble_det_kernel<true><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval);
+    const SlabValues none{};
+    if (sv && zero_first)
+        reassemble_det_kernel<true, true><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval, *sv);
+    else if (sv)
+        reassemble_det_kernel<false, true><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval, *sv);
+    else if (zero_first)
+        reassemble_det_kernel<true, false><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval, none);
     else
-        reassemble_det_kernel<false><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval);
+        reassemble_det_kernel<false, false><<<blocks, 256, 0, stream>>>(V, perm, segstart, nnz, nzval, none);
     lc.add();
     XSB_CUDA(cudaGetLastError());
 }
 
-// fast mode: one atomic add per insertion through the 4-byte entry -> nzval map, in whatever order the hardware takes
+// fast mode: one atomic add per insertion through the 4-byte entry -> nzval map, in whatever order the hardware takes.
+// SLAB: k runs over the combined index space; the own stream's positions in other ranks' columns carry kNoSlot.
+template <bool SLAB>
 __global__ void __launch_bounds__(256)
 reassemble_fast_kernel(const double *__restrict__ V, const u32 *__restrict__ slot, i64 count,
-                       double *__restrict__ nzval)
+                       double *__restrict__ nzval, SlabValues sv)
 {
     const i64 stride = (i64)gridDim.x * blockDim.x;
     for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < count; k += stride)
-        atomicAdd(nzval + slot[k], V[k]);
+    {
+        if constexpr (!SLAB)
+            atomicAdd(nzval + slot[k], V[k]);
+        else
+        {
+            const u32 z = slot[k];
+            if (z != kNoSlot)
+                atomicAdd(nzval + z, __ldg(value_at<true>(V, sv, (u32)k)));
+        }
+    }
 }
 
 void reassemble_fast(cudaStream_t stream, const double *V, const u32 *slot, i64 count, double *nzval,
-                     LaunchCounter &lc)
+                     LaunchCounter &lc, const SlabValues *sv)
 {
     if (count <= 0)
         return;
-    reassemble_fast_kernel<<<grid_for(count, 256, 32), 256, 0, stream>>>(V, slot, count, nzval);
+    if (sv)
+        reassemble_fast_kernel<true><<<grid_for(count, 256, 32), 256, 0, stream>>>(V, slot, count, nzval, *sv);
+    else
+        reassemble_fast_kernel<false><<<grid_for(count, 256, 32), 256, 0, stream>>>(V, slot, count, nzval, SlabValues{});
+    lc.add();
+    XSB_CUDA(cudaGetLastError());
+}
+
+// ---- frozen streams of slab handles (xsb_freeze_slab*): positions in GLOBAL columns, some owned by other ranks ----
+// One pass over the stream: bounds, owner (KeyLayout::pack, the search the producers use), own positions -> nzval
+// slot, foreign ones -> a routing tag {owner << 32 | stream index, (row, owner-relative column)} that the stable
+// copy-out of xsb_route.cu gathers destination after destination.  Own positions (and bad ones) get tag owner self.
+template <typename Ti, class Pos>
+__global__ void __launch_bounds__(256)
+slab_classify_kernel(const Ti *__restrict__ colptr, const Ti *__restrict__ rowval, Ti base, i64 m, i64 n_global,
+                     KeyLayout Ls, Pos pos, i64 count, i64 *__restrict__ slot, Rec *__restrict__ tags,
+                     u64 *__restrict__ d_missing, u64 *__restrict__ d_oob)
+{
+    const i64 stride = (i64)gridDim.x * blockDim.x;
+    for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < count; k += stride)
+    {
+        i64 i, j;
+        pos.at(k, i, j);
+        i -= base;
+        j -= base;
+        i64 s = -1;
+        u64 owner = (u64)Ls.self, where = 0;
+        if (i < 0 || i >= m || j < 0 || j >= n_global)
+            atomicMin(d_oob, (u64)k);
+        else
+        {
+            const u64 key = Ls.colpart((u64)j);
+            const u64 lc = Ls.col(key);
+            owner = Ls.owner(key);
+            if (owner == (u64)Ls.self)
+            {
+                s = find_slot<Ti>(colptr, rowval, base, i, (i64)lc);
+                if (s < 0)
+                    atomicAdd(d_missing, 1ull);
+            }
+            else
+                where = (u64)i | (lc << 32);
+        }
+        slot[k] = s;
+        Rec r;
+        r.key = (owner << 32) | (u64)k;
+        *reinterpret_cast<u64 *>(&r.val) = where;
+        st_rec(tags + k, r);
+    }
+}
+
+template <typename Ti, class Pos>
+static void launch_classify(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int base,
+                            Pos pos, i64 count, i64 *slot, Rec *tags, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+{
+    if (count <= 0)
+        return;
+    slab_classify_kernel<Ti, Pos><<<grid_for(count, 256), 256, 0, stream>>>(
+        (const Ti *)csc.colptr, (const Ti *)csc.rowval, (Ti)base, m, n_global, Ls, pos, count, slot, tags, d_missing, d_oob);
+    lc.add();
+    XSB_CUDA(cudaGetLastError());
+}
+
+void slab_classify(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64, int base,
+                   const void *I, const void *J, i64 count, i64 *slot, Rec *tags, u64 *d_missing, u64 *d_oob,
+                   LaunchCounter &lc)
+{
+    if (idx64)
+        launch_classify<int64_t>(stream, csc, m, n_global, Ls, base, PosIJ<int64_t>{(const int64_t *)I, (const int64_t *)J},
+                                 count, slot, tags, d_missing, d_oob, lc);
+    else
+        launch_classify<int32_t>(stream, csc, m, n_global, Ls, base, PosIJ<int32_t>{(const int32_t *)I, (const int32_t *)J},
+                                 count, slot, tags, d_missing, d_oob, lc);
+}
+
+void slab_classify_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64,
+                            int base, const void *dofs, int k, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
+                            u64 *d_oob, LaunchCounter &lc)
+{
+    if (idx64)
+        launch_classify<int64_t>(stream, csc, m, n_global, Ls, base, PosElements<int64_t>{(const int64_t *)dofs, (i64)k},
+                                 count, slot, tags, d_missing, d_oob, lc);
+    else
+        launch_classify<int32_t>(stream, csc, m, n_global, Ls, base, PosElements<int32_t>{(const int32_t *)dofs, (i64)k},
+                                 count, slot, tags, d_missing, d_oob, lc);
+}
+
+// the gathered tags -> stream indices (kept for every step) and 8-byte positions {row, owner-relative column}
+__global__ void __launch_bounds__(256)
+slab_split_kernel(const Rec *__restrict__ tags, i64 n, u32 *__restrict__ idx, u64 *__restrict__ where)
+{
+    const i64 stride = (i64)gridDim.x * blockDim.x;
+    for (i64 q = (i64)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride)
+    {
+        const Rec r = tags[q];
+        idx[q] = (u32)r.key;
+        where[q] = *reinterpret_cast<const u64 *>(&r.val);
+    }
+}
+
+void slab_split(cudaStream_t stream, const Rec *tags, i64 n, u32 *idx, u64 *where, LaunchCounter &lc)
+{
+    if (n <= 0)
+        return;
+    slab_split_kernel<<<grid_for(n, 256), 256, 0, stream>>>(tags, n, idx, where);
+    lc.add();
+    XSB_CUDA(cudaGetLastError());
+}
+
+// (slot, combined index) records over [received from lower ranks | own stream | received from higher ranks]: received
+// positions are looked up in the slab, own ones bring the slot found at freeze time; foreign own positions and bad
+// received ones get slot `nnz`, which sorts behind every real slot and stays out of the map
+template <typename Ti>
+__global__ void __launch_bounds__(256)
+slab_records_kernel(const Ti *__restrict__ colptr, const Ti *__restrict__ rowval, Ti base, i64 m, i64 n,
+                    const i64 *__restrict__ own_slot, i64 own, const uint2 *__restrict__ recv, i64 low, i64 total,
+                    i64 nnz, Rec *__restrict__ out, u64 *__restrict__ d_missing, u64 *__restrict__ d_oob)
+{
+    const i64 stride = (i64)gridDim.x * blockDim.x;
+    for (i64 k = (i64)blockIdx.x * blockDim.x + threadIdx.x; k < total; k += stride)
+    {
+        i64 s;
+        if (k >= low && k - low < own)
+        {
+            s = own_slot[k - low];
+            if (s < 0)
+                s = nnz;
+        }
+        else
+        {
+            const i64 q = k < low ? k : k - own;
+            const uint2 p = recv[q];
+            s = nnz;
+            if ((i64)p.x >= m || (i64)p.y >= n)
+                atomicMin(d_oob, (u64)q);
+            else
+            {
+                const i64 f = find_slot<Ti>(colptr, rowval, base, (i64)p.x, (i64)p.y);
+                if (f < 0)
+                    atomicAdd(d_missing, 1ull);
+                else
+                    s = f;
+            }
+        }
+        Rec r;
+        r.key = (u64)s;
+        *reinterpret_cast<u64 *>(&r.val) = (u64)k;
+        st_rec(out + k, r);
+    }
+}
+
+void slab_records(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const i64 *own_slot, i64 own,
+                  const void *recv, i64 low, i64 total, Rec *out, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+{
+    if (total <= 0)
+        return;
+    if (idx64)
+        slab_records_kernel<int64_t><<<grid_for(total, 256), 256, 0, stream>>>(
+            (const int64_t *)csc.colptr, (const int64_t *)csc.rowval, (int64_t)base, m, n, own_slot, own,
+            (const uint2 *)recv, low, total, csc.nnz, out, d_missing, d_oob);
+    else
+        slab_records_kernel<int32_t><<<grid_for(total, 256), 256, 0, stream>>>(
+            (const int32_t *)csc.colptr, (const int32_t *)csc.rowval, (int32_t)base, m, n, own_slot, own,
+            (const uint2 *)recv, low, total, csc.nnz, out, d_missing, d_oob);
+    lc.add();
+    XSB_CUDA(cudaGetLastError());
+}
+
+// per step: the values of the foreign positions, bucket after bucket, in the order of xsb_freeze_slab_prepare
+__global__ void __launch_bounds__(256)
+slab_pack_kernel(const double *__restrict__ V, const u32 *__restrict__ idx, i64 n, double *__restrict__ send)
+{
+    const i64 stride = (i64)gridDim.x * blockDim.x;
+    for (i64 q = (i64)blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride)
+        send[q] = __ldg(V + idx[q]);
+}
+
+void slab_pack_values(cudaStream_t stream, const double *V, const u32 *idx, i64 n, double *send, LaunchCounter &lc)
+{
+    if (n <= 0)
+        return;
+    slab_pack_kernel<<<grid_for(n, 256), 256, 0, stream>>>(V, idx, n, send);
     lc.add();
     XSB_CUDA(cudaGetLastError());
 }

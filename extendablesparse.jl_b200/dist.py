@@ -30,6 +30,7 @@ import torch.distributed as dist
 
 
 _ROUTE_MAGIC = 0x5853425F524F5554  # header word of a fixed-capacity block ("XSB_ROUT", xsb_route.cu)
+_FAILED_WITHOUT_STATUS = 1000  # a rank's freeze failed with an exception that has no library status code
 
 
 def uniform_splits(n: int, world: int) -> List[int]:
@@ -120,6 +121,13 @@ class DistExtendableSparseMatrix:
         self._peer = None  # None: not decided yet; True / False after the first fixed-capacity step
         self._early = False  # exchange_begin() already packed this step
         self.transport_note = ""
+        # values-only re-assembly of a stream frozen across the slabs (freeze_pattern / freeze_elements): the sizes of
+        # the per-step exchange of values, fixed at freeze time (own rank: 0)
+        self._frozen = False
+        self._vcounts_out = None  # per destination rank
+        self._vcounts_in = None   # per source rank
+        self._vsend = None
+        self._vrecv = None
 
     # insertion: global (i,j) on any rank
     def insert_batch(self, I, J, V, flavour=0):
@@ -397,6 +405,129 @@ class DistExtendableSparseMatrix:
             self._nnz_offset, self._nnz_global = sum(per_rank[: self.rank]), sum(per_rank)
             self._changed_any = any(flags)
             self._offsets_pending = None
+            if self._changed_any and self._frozen:
+                # the pattern changed on some rank: the values its frozen stream sends elsewhere no longer fit the
+                # owners' maps, so every rank drops its map (the rank whose pattern changed already has)
+                self.unfreeze()
+
+    # ---- values-only re-assembly of a stream frozen across the slabs ----
+    def _fail_everywhere(self, err):
+        """Collective: every rank learns whether any rank failed; if one did, every rank is left unfrozen and raises
+        (the failing rank its own error)."""
+        codes = torch.zeros(self.world, dtype=torch.int64, device=self.device)
+        if err is not None:
+            # any failure counts, also one that carries no library status (a bad argument caught in Python): the MAX
+            # reduction only sees positive entries
+            code = getattr(err, "code", None)
+            codes[self.rank] = code if isinstance(code, int) and code > 0 else _FAILED_WITHOUT_STATUS
+        dist.all_reduce(codes, op=dist.ReduceOp.MAX, group=self.group)
+        bad = [(r, c) for r, c in enumerate(codes.cpu().tolist()) if c != 0]
+        if not bad:
+            return
+        self.unfreeze()
+        if err is not None:
+            raise err
+        r, c = bad[0]
+        why = "an error without a library status" if c == _FAILED_WITHOUT_STATUS else f"status {c}"
+        raise RuntimeError(f"freezing the slab stream failed on rank {r} ({why}); every rank is left unfrozen")
+
+    def _freeze(self, first):
+        """The collective freeze: `first()` resolves the own positions and returns the positions per owner; the counts
+        and then the foreign positions (8 bytes each) travel all-to-all; finish resolves what arrived."""
+        self.unfreeze()
+        self._resolve_offsets()
+        counts, err = None, None
+        try:
+            counts = first()
+        except Exception as e:  # noqa: BLE001  (reported to every rank)
+            err = e
+        self._fail_everywhere(err)
+        world, rank = self.world, self.rank
+        off = [0 if r == rank else int(c) for r, c in enumerate(counts)]
+        send = torch.empty(max(sum(off), 1), dtype=torch.int64, device=self.device)
+        err = None
+        try:
+            self.h.freeze_slab_prepare(send, sum(off))
+        except Exception as e:  # noqa: BLE001
+            err = e
+        self._fail_everywhere(err)
+        if self.device.type == "cuda":
+            torch.cuda.current_stream(self.device).synchronize()
+        sc = torch.tensor(off, dtype=torch.int64, device=self.device)
+        rc = torch.empty(world, dtype=torch.int64, device=self.device)
+        dist.all_to_all_single(rc, sc, group=self.group)
+        rcounts = [0 if r == rank else int(c) for r, c in enumerate(rc.cpu().tolist())]
+        recv = torch.empty(max(sum(rcounts), 1), dtype=torch.int64, device=self.device)
+        dist.all_to_all_single(recv[: sum(rcounts)], send[: sum(off)], output_split_sizes=rcounts,
+                               input_split_sizes=off, group=self.group)
+        if self.device.type == "cuda":
+            torch.cuda.current_stream(self.device).synchronize()
+        err = None
+        try:
+            self.h.freeze_slab_finish(recv, rcounts)
+        except Exception as e:  # noqa: BLE001
+            err = e
+        self._fail_everywhere(err)
+        self._vcounts_out, self._vcounts_in = off, rcounts
+        self._vsend = torch.empty(max(sum(off), 1), dtype=torch.float64, device=self.device)
+        self._vrecv = torch.empty(max(sum(rcounts), 1), dtype=torch.float64, device=self.device)
+        self._frozen = True
+
+    def freeze_pattern(self, I, J):
+        """Collective: freezes this rank's stream of GLOBAL positions (I[k], J[k]) -- any owner -- for values-only
+        re-assembly.  Every position must already be an entry of its owner's slab.  One rank's error (a position
+        outside the matrix or absent from the pattern) fails the freeze on every rank and leaves every rank unfrozen."""
+        self._freeze(lambda: self.h.freeze_slab(I, J))
+
+    def freeze_elements(self, dofs):
+        """freeze_pattern for the stream insert_elements(dofs, .) stages: reassemble_values then takes the element
+        matrices (ncells, k, k) as they are."""
+        self._freeze(lambda: self.h.freeze_slab_elements(dofs))
+
+    def unfreeze(self):
+        self.h.unfreeze()
+        self._frozen = False
+        self._vcounts_out = self._vcounts_in = None
+
+    def reassemble_values(self, V, mode=0, zero_first=True):
+        """One values-only step: V holds a value per position of this rank's frozen stream.  The values of positions
+        other ranks own go to them with one grouped point-to-point exchange whose sizes were fixed at freeze time, and
+        every slab entry folds its resident value (+0.0 with zero_first) followed by the values of rank 0, 1, ... in
+        each rank's stream order -- the same bits as one matrix re-assembling the rank-ordered concatenation of the
+        streams.  Stream-ordered on the library's stream; the host does not wait for the device."""
+        self._resolve_offsets()
+        if not self._frozen:
+            raise RuntimeError("no frozen stream: freeze_pattern / freeze_elements first")
+        h, world, rank = self.h, self.world, self.rank
+        co, ci = self._vcounts_out, self._vcounts_in
+        if self.device.type == "cuda":
+            if self._lib_stream is None:
+                self._lib_stream = torch.cuda.ExternalStream(h.stream, device=self.device)
+            self._lib_stream.wait_stream(torch.cuda.current_stream(self.device))  # V may come from the current stream
+        h.reassemble_slab_pack(V, self._vsend)
+        ops, spos, rpos = [], 0, 0
+        for p in range(world):
+            if p == rank:
+                continue
+            if co[p] > 0:
+                ops.append(dist.P2POp(dist.isend, self._vsend[spos: spos + co[p]], p, group=self.group))
+            if ci[p] > 0:
+                ops.append(dist.P2POp(dist.irecv, self._vrecv[rpos: rpos + ci[p]], p, group=self.group))
+            spos += co[p]
+            rpos += ci[p]
+        if ops:
+            if self.device.type == "cuda":
+                with torch.cuda.stream(self._lib_stream):
+                    for w in dist.batch_isend_irecv(ops):
+                        w.wait()  # stream-level: the library's stream waits for the transfers, the host does not
+            else:
+                for w in dist.batch_isend_irecv(ops):
+                    w.wait()
+        h.reassemble_slab_values(V, self._vrecv, mode, zero_first)
+        if self.device.type == "cuda" and isinstance(V, torch.Tensor) and V.is_cuda:
+            # the pack and the fold read V on the library's stream, which the host does not wait for: keep V's memory
+            # from being handed to new work on other streams before they are done
+            V.record_stream(self._lib_stream)
 
     @property
     def nnz_offset(self) -> int:

@@ -179,14 +179,17 @@ mutable struct B200Assembler{Tv, Ti <: Integer}
     m::Int
     n::Int
     handle::Ptr{Cvoid}
+    nranks::Int # slab assemblers: ranks and own rank (0, 0: a whole matrix)
+    rank::Int
+    slab::Any # device buffers of a stream frozen across column slabs (freeze_slab!), or nothing
     function B200Assembler{Tv, Ti}(m, n, nparts = 1; device = 0) where {Tv, Ti}
         h = Ref{Ptr{Cvoid}}(C_NULL)
         rc = ccall((:xsb_create, libxsb), Int32,
                    (Int64, Int64, Int32, Int32, Int32, Int32, Int32, Ref{Ptr{Cvoid}}),
                    m, n, XSB_F64, idxcode(Ti), 1, nparts, device, h)
         check(Ptr{Cvoid}(C_NULL), rc)
-        x = new{Tv, Ti}(m, n, h[])
-        finalizer(y -> (y.handle == C_NULL || ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), y.handle);
+        x = new{Tv, Ti}(m, n, h[], 0, 0, nothing)
+        finalizer(y -> (free_slab_buffers!(y); y.handle == C_NULL || ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), y.handle);
                         y.handle = C_NULL), x)
         x
     end
@@ -198,8 +201,8 @@ mutable struct B200Assembler{Tv, Ti <: Integer}
                    (Int64, Int64, Int32, Int32, Ptr{Int64}, Int32, Int32, Int32, Int32, Ref{Ptr{Cvoid}}),
                    m, n, nranks, rank, col_splits, XSB_F64, idxcode(Ti), 1, device, h)
         check(Ptr{Cvoid}(C_NULL), rc)
-        x = new{Tv, Ti}(m, n, h[])
-        finalizer(y -> (y.handle == C_NULL || ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), y.handle);
+        x = new{Tv, Ti}(m, n, h[], nranks, rank, nothing)
+        finalizer(y -> (free_slab_buffers!(y); y.handle == C_NULL || ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), y.handle);
                         y.handle = C_NULL), x)
         x
     end
@@ -337,6 +340,100 @@ function peer_exchange_close!(a::B200Assembler, barrier)
     check(a.handle, ccall((:xsb_peer_exchange_destroy, libxsb), Int32, (Ptr{Cvoid},), a.handle))
     a
 end
+
+# ---- values-only re-assembly of a stream of GLOBAL positions frozen across the column slabs (INTEGRATION.md §4) ----
+# `alltoallv(sendbuf::Ptr, sendcounts::Vector{Int64}, recvbuf::Ptr, recvcounts::Vector{Int64}, itembytes)` is the
+# caller's all-to-all-v over the ranks (e.g. CUDA-aware `MPI.Alltoallv!`): item counts per rank, own rank 0; the
+# buffers are host memory for the counts and device memory for positions and values.
+const libcudart = get(ENV, "XSPARSE_B200_CUDART", "libcudart.so")
+function device_alloc(bytes)
+    p = Ref{Ptr{Cvoid}}(C_NULL)
+    ccall((:cudaMalloc, libcudart), Int32, (Ref{Ptr{Cvoid}}, Csize_t), p, max(bytes, 16)) == 0 ||
+        throw(OutOfMemoryError())
+    p[]
+end
+function free_slab_buffers!(a::B200Assembler)
+    if a.slab !== nothing
+        for p in (a.slab.send, a.slab.recv)
+            ccall((:cudaFree, libcudart), Int32, (Ptr{Cvoid},), p)
+        end
+        a.slab = nothing
+    end
+    a
+end
+
+function freeze_slab_exchange!(a::B200Assembler, send_counts::Vector{Int64}, alltoallv)
+    nranks, rank = a.nranks, a.rank
+    off = [r == rank ? 0 : send_counts[r + 1] for r in 0:nranks-1]
+    recv_counts = zeros(Int64, nranks)
+    ones_ = [r == rank ? 0 : 1 for r in 0:nranks-1]
+    alltoallv(pointer(off), ones_, pointer(recv_counts), ones_, 8)
+    send = device_alloc(8 * sum(off))
+    recv = device_alloc(8 * sum(recv_counts))
+    try
+        check(a.handle, ccall((:xsb_freeze_slab_prepare, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int64),
+                              a.handle, send, sum(off)))
+        alltoallv(send, off, recv, recv_counts, 8)
+        check(a.handle, ccall((:xsb_freeze_slab_finish, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Int64}),
+                              a.handle, recv, recv_counts))
+    catch
+        ccall((:cudaFree, libcudart), Int32, (Ptr{Cvoid},), send)
+        ccall((:cudaFree, libcudart), Int32, (Ptr{Cvoid},), recv)
+        rethrow()
+    end
+    ccall((:cudaFree, libcudart), Int32, (Ptr{Cvoid},), send)
+    ccall((:cudaFree, libcudart), Int32, (Ptr{Cvoid},), recv)
+    # the per-step value buffers: sizes fixed since the freeze
+    a.slab = (send = device_alloc(8 * sum(off)), recv = device_alloc(8 * sum(recv_counts)), off = off,
+              recv_counts = recv_counts)
+    a
+end
+
+"""
+    freeze_slab!(a, I, J, alltoallv)
+
+Collective over the ranks: freezes this rank's stream of GLOBAL positions (any owner) on the slab assembler `a`;
+afterwards every step is `reassemble_slab!(a, V, alltoallv)`.  A rank whose freeze fails throws; the caller
+must make the other ranks give up too (e.g. an all-reduce of the status), every handle is then left unfrozen.
+"""
+function freeze_slab!(a::B200Assembler{Tv, Ti}, I::Vector{Ti}, J::Vector{Ti}, alltoallv) where {Tv, Ti}
+    free_slab_buffers!(a)
+    counts = zeros(Int64, a.nranks)
+    check(a.handle, ccall((:xsb_freeze_slab, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int64, Ptr{Int64}),
+                          a.handle, I, J, length(I), counts))
+    freeze_slab_exchange!(a, counts, alltoallv)
+end
+
+"freeze_slab! for the element loop of insert_elements!: then `reassemble_slab!(a, vec(Aloc), alltoallv)` each step"
+function freeze_slab_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}, alltoallv) where {Tv, Ti}
+    free_slab_buffers!(a)
+    counts = zeros(Int64, a.nranks)
+    check(a.handle, ccall((:xsb_freeze_slab_elements, libxsb), Int32, (Ptr{Cvoid}, Int32, Int64, Ptr{Cvoid}, Ptr{Int64}),
+                          a.handle, size(dofs, 1), size(dofs, 2), dofs, counts))
+    freeze_slab_exchange!(a, counts, alltoallv)
+end
+
+"""
+    reassemble_slab!(a, V, alltoallv; mode = XSB_DETERMINISTIC, zero = true)
+
+One values-only step of a stream frozen with `freeze_slab!`: the values of positions other ranks own leave through
+`alltoallv` with the sizes of the freeze, and every slab entry folds its resident value (+0.0 with `zero`) followed
+by the values of rank 0, 1, ... in each rank's stream order.
+"""
+function reassemble_slab!(a::B200Assembler{Tv}, V::Vector{Tv}, alltoallv; mode = XSB_DETERMINISTIC, zero = true) where {Tv}
+    s = a.slab
+    s === nothing && error("no frozen slab stream: freeze_slab! first")
+    check(a.handle, ccall((:xsb_reassemble_slab_pack, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Ptr{Cvoid}),
+                          a.handle, V, length(V), s.send))
+    ccall((:xsb_synchronize, libxsb), Int32, (Ptr{Cvoid},), a.handle)
+    alltoallv(s.send, s.off, s.recv, s.recv_counts, 8)
+    check(a.handle, ccall((:xsb_reassemble_slab_values, libxsb), Int32,
+                          (Ptr{Cvoid}, Ptr{Cvoid}, Int64, Ptr{Cvoid}, Int32, Int32),
+                          a.handle, V, length(V), s.recv, mode, zero ? 1 : 0))
+    a
+end
+
+export freeze_slab!, freeze_slab_elements!, reassemble_slab!
 
 export peer_exchange!, route_step!, peer_exchange_close!
 export SparseMatrixB200, B200Assembler, pattern_equal, B200ExtendableSparseMatrixCSC, STB200ExtendableSparseMatrixCSC,

@@ -304,6 +304,47 @@ int32_t xsb_reassemble_values(xsb_matrix *h, const void *V, int64_t count, int32
  * entries start from +0.0 and nzval is written, never read (a Newton / time step re-assembles from zero). */
 int32_t xsb_reassemble_values_zeroed(xsb_matrix *h, const void *V, int64_t count, int32_t mode);
 int32_t xsb_unfreeze(xsb_matrix *h);
+/* On slab handles xsb_freeze_pattern / xsb_freeze_elements / xsb_get_values take slab-relative columns and the
+ * rank's own entries only.  A distributed element loop is sharded by elements instead: the interface elements of
+ * every rank write into columns a neighbour owns.  The calls below freeze such a stream -- GLOBAL positions, any
+ * owner -- across the ranks (slab handles only; on a plain handle, or with insertions pending: XSB_ESTATE).
+ * A counted exchange runs once, at freeze time; every step then moves the values of the foreign positions with sizes
+ * fixed since the freeze.
+ *   freeze  xsb_freeze_slab(h, I, J, count, send_counts) or xsb_freeze_slab_elements(h, k, ncells, dofs, send_counts):
+ *             resolves the own positions and counts the foreign ones per owner: send_counts[n_ranks] (host; own rank:
+ *             the positions kept).  count < 2^32 (else XSB_EINVAL); a position outside the matrix: XSB_EBOUNDS naming
+ *             the stream position; an own position absent from the pattern: XSB_EILLEGAL.  The handle is now HALF
+ *             frozen: the re-assembly calls return XSB_ESTATE, and insertions, xsb_flush, xsb_set_csc, xsb_reset and
+ *             xsb_unfreeze drop the half-made freeze.
+ *           xsb_freeze_slab_prepare(h, send_positions, capacity): the foreign positions, destination after destination,
+ *             each bucket in stream order, 8 bytes each {u32 row (0-based), u32 column relative to the owner's slab},
+ *             into device memory; capacity >= their number.
+ *           (caller) exchange the counts, then the positions, all-to-all-v (own rank: nothing).
+ *           xsb_freeze_slab_finish(h, recv_positions, recv_counts): the received buckets, sources ascending, own rank
+ *             left out (recv_counts[own] is ignored); device memory.  Resolves them against the slab's CSC (absent:
+ *             XSB_EILLEGAL, outside the slab: XSB_EBOUNDS) and builds the map.  Received positions plus count must
+ *             stay below 2^32 (XSB_EINVAL).  On any error of the three calls the handle is left unfrozen.
+ *           xsb_frozen_slab_counts(h, send_counts, recv_counts): the sizes of the per-step exchange.
+ *   step    xsb_reassemble_slab_pack(h, V, count, send_values): V holds one value per position of the rank's frozen
+ *             stream (count must match: XSB_ESIZE); the values of the foreign positions go to send_values (device),
+ *             laid out as the positions at prepare.
+ *           (caller) exchange the values with the counts of the freeze (point-to-point, no count on the host).
+ *           xsb_reassemble_slab_values(h, V, count, recv_values, mode, zero_first): folds own and received values into
+ *             the slab's nzval; recv_values laid out as the positions at finish.
+ *   The map indexes the combined space [received from lower ranks | own stream | received from higher ranks]; every
+ *   entry folds its resident value (+0.0 with zero_first), then the values of rank 0, 1, ..., each rank's in its
+ *   stream order.  So rank r's slab equals, bit for bit in XSB_DETERMINISTIC mode, its columns of one plain handle
+ *   that froze the concatenated streams S_0 ++ S_1 ++ ... and re-assembled V_0 ++ V_1 ++ ...  XSB_FAST: one atomic add
+ *   per value.  xsb_reassemble_values[_zeroed] on a handle frozen this way returns XSB_ESTATE; a flush that changes the
+ *   slab's pattern drops the map. */
+int32_t xsb_freeze_slab(xsb_matrix *h, const void *I, const void *J, int64_t count, int64_t *send_counts);
+int32_t xsb_freeze_slab_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs, int64_t *send_counts);
+int32_t xsb_freeze_slab_prepare(xsb_matrix *h, void *send_positions, int64_t capacity);
+int32_t xsb_freeze_slab_finish(xsb_matrix *h, const void *recv_positions, const int64_t *recv_counts);
+int32_t xsb_frozen_slab_counts(const xsb_matrix *h, int64_t *send_counts, int64_t *recv_counts);
+int32_t xsb_reassemble_slab_pack(xsb_matrix *h, const double *V, int64_t count, double *send_values);
+int32_t xsb_reassemble_slab_values(xsb_matrix *h, const double *V, int64_t count, const double *recv_values,
+                                   int32_t mode, int32_t zero_first);
 
 /* y = A*x on the resident CSC (x: n values, y: m values; host or device pointers).  mul!(r,A,x):
  * src/matrix/abstractextendablesparsematrixcsc.jl:170-181 (flush, then the stdlib kernel: columns
