@@ -109,6 +109,7 @@ SIGNATURES = {
     "xsb_insert_batch": (_i32, [_p, _i32, _p, _p, _p, _i64, _i32]),
     "xsb_insert_triplets": (_i32, [_p, _i32, _p, _i64, _i32]),
     "xsb_insert_elements": (_i32, [_p, _i32, _i32, _i64, _p, _p, _i32]),
+    "xsb_insert_elements_rect": (_i32, [_p, _i32, _i32, _i32, _i64, _p, _p, _p, _i32]),
     "xsb_pending": (_i32, [_p, C.POINTER(_i64)]),
     "xsb_flush": (_i32, [_p, _i32, C.POINTER(_i64), C.POINTER(_i32)]),
     "xsb_flush_ex": (_i32, [_p, _i32, _i32, C.POINTER(_i64), C.POINTER(_i32)]),
@@ -117,11 +118,13 @@ SIGNATURES = {
     "xsb_zero_values": (_i32, [_p]),
     "xsb_freeze_pattern": (_i32, [_p, _p, _p, _i64]),
     "xsb_freeze_elements": (_i32, [_p, _i32, _i64, _p]),
+    "xsb_freeze_elements_rect": (_i32, [_p, _i32, _i32, _i64, _p, _p]),
     "xsb_reassemble_values": (_i32, [_p, _p, _i64, _i32]),
     "xsb_reassemble_values_zeroed": (_i32, [_p, _p, _i64, _i32]),
     "xsb_unfreeze": (_i32, [_p]),
     "xsb_freeze_slab": (_i32, [_p, _p, _p, _i64, C.POINTER(_i64)]),
     "xsb_freeze_slab_elements": (_i32, [_p, _i32, _i64, _p, C.POINTER(_i64)]),
+    "xsb_freeze_slab_elements_rect": (_i32, [_p, _i32, _i32, _i64, _p, _p, C.POINTER(_i64)]),
     "xsb_freeze_slab_prepare": (_i32, [_p, _p, _i64]),
     "xsb_freeze_slab_finish": (_i32, [_p, _p, C.POINTER(_i64)]),
     "xsb_frozen_slab_counts": (_i32, [_p, C.POINTER(_i64), C.POINTER(_i64)]),
@@ -362,39 +365,61 @@ class Handle:
             count = len(T)
         self._c(lib().xsb_insert_triplets(self._h, tid, ptr(T), count, flavour))
 
-    def _element_arrays(self, dofs, Aloc=None):
-        """(ncells, k) connectivity in the handle's index type and (ncells, k, k) Float64 element matrices, both
-        C-contiguous: the column-major k x ncells / k x k x ncells arrays of the C ABI (Aloc[c, jl, il] is entry
-        (il, jl) of element c).  numpy arrays are converted, torch tensors (host or device) must already match."""
+    def _dof_array(self, dofs, name):
         if hasattr(dofs, "data_ptr"):
             want = "torch.int64" if self.idx_type == I64 else "torch.int32"
             if str(dofs.dtype) != want:
-                raise TypeError(f"dofs must be {want}")
+                raise TypeError(f"{name} must be {want}")
         else:
             dofs = np.ascontiguousarray(dofs, self.idx_dtype)
         if dofs.ndim != 2:
-            raise ValueError("dofs must have shape (ncells, k)")
-        ncells, k = (int(x) for x in dofs.shape)
+            raise ValueError(f"{name} must have shape (ncells, k)")
+        return dofs
+
+    def _element_arrays(self, dofs, Aloc=None, col_dofs=None):
+        """(ncells, k) connectivity in the handle's index type and (ncells, k, k) Float64 element matrices, both
+        C-contiguous: the column-major k x ncells / k x k x ncells arrays of the C ABI (Aloc[c, jl, il] is entry
+        (il, jl) of element c).  With col_dofs, dofs is the (ncells, kr) row connectivity, col_dofs the (ncells, kc)
+        column connectivity and Aloc has shape (ncells, kc, kr).  numpy arrays are converted, torch tensors (host or
+        device) must already match.  Returns (dofs, col_dofs, Aloc, ncells, kr, kc)."""
+        dofs = self._dof_array(dofs, "dofs")
+        ncells, kr = (int(x) for x in dofs.shape)
+        kc = kr
+        if col_dofs is not None:
+            col_dofs = self._dof_array(col_dofs, "col_dofs")
+            if int(col_dofs.shape[0]) != ncells:
+                raise ValueError(f"col_dofs must have {ncells} rows, one per element, not {int(col_dofs.shape[0])}")
+            kc = int(col_dofs.shape[1])
         if Aloc is not None:
             if hasattr(Aloc, "data_ptr"):
                 if str(Aloc.dtype) != "torch.float64":
                     raise TypeError("Aloc must be torch.float64")
             else:
                 Aloc = np.ascontiguousarray(Aloc, np.float64)
-            if tuple(Aloc.shape) != (ncells, k, k):
-                raise ValueError(f"Aloc must have shape (ncells, k, k) = {(ncells, k, k)}, not {tuple(Aloc.shape)}")
-        return dofs, Aloc, ncells, k
+            if tuple(Aloc.shape) != (ncells, kc, kr):
+                what = "(ncells, k, k)" if col_dofs is None else "(ncells, kc, kr)"
+                raise ValueError(f"Aloc must have shape {what} = {(ncells, kc, kr)}, not {tuple(Aloc.shape)}")
+        return dofs, col_dofs, Aloc, ncells, kr, kc
 
-    def insert_elements(self, dofs, Aloc, flavour=RAW, tid=0):
-        """k*k*ncells calls of an element loop: call k*k*c + k*jl + il is (dofs[c, il], dofs[c, jl], Aloc[c, jl, il])."""
-        dofs, Aloc, ncells, k = self._element_arrays(dofs, Aloc)
-        self._c(lib().xsb_insert_elements(self._h, tid, k, ncells, ptr(dofs), ptr(Aloc), flavour))
+    def insert_elements(self, dofs, Aloc, flavour=RAW, tid=0, col_dofs=None):
+        """k*k*ncells calls of an element loop: call k*k*c + k*jl + il is (dofs[c, il], dofs[c, jl], Aloc[c, jl, il]).
+        With col_dofs (rows and columns from different connectivities, kr and kc dofs per element): call
+        kr*kc*c + kr*jl + il is (dofs[c, il], col_dofs[c, jl], Aloc[c, jl, il])."""
+        dofs, col_dofs, Aloc, ncells, kr, kc = self._element_arrays(dofs, Aloc, col_dofs)
+        if col_dofs is None:
+            self._c(lib().xsb_insert_elements(self._h, tid, kr, ncells, ptr(dofs), ptr(Aloc), flavour))
+        else:
+            self._c(lib().xsb_insert_elements_rect(self._h, tid, kr, kc, ncells, ptr(dofs), ptr(col_dofs), ptr(Aloc),
+                                                   flavour))
 
-    def freeze_elements(self, dofs):
-        """freeze_pattern for the stream insert_elements(dofs, .) stages; reassemble_values(Aloc) then takes the
-        element matrices as they are."""
-        dofs, _, ncells, k = self._element_arrays(dofs)
-        self._c(lib().xsb_freeze_elements(self._h, k, ncells, ptr(dofs)))
+    def freeze_elements(self, dofs, col_dofs=None):
+        """freeze_pattern for the stream insert_elements(dofs, ., col_dofs=col_dofs) stages; reassemble_values(Aloc)
+        then takes the element matrices as they are."""
+        dofs, col_dofs, _, ncells, kr, kc = self._element_arrays(dofs, None, col_dofs)
+        if col_dofs is None:
+            self._c(lib().xsb_freeze_elements(self._h, kr, ncells, ptr(dofs)))
+        else:
+            self._c(lib().xsb_freeze_elements_rect(self._h, kr, kc, ncells, ptr(dofs), ptr(col_dofs)))
 
     def flush(self, mode=DETERMINISTIC, combine=COMBINE_SEED):
         nnz, changed = _i64(0), _i32(0)
@@ -453,11 +478,15 @@ class Handle:
         self._c(lib().xsb_freeze_slab(self._h, ptr(I), ptr(J), count, counts))
         return [int(c) for c in counts]
 
-    def freeze_slab_elements(self, dofs):
-        """freeze_slab for the stream insert_elements(dofs, .) stages ((ncells, k) connectivity)."""
-        dofs, _, ncells, k = self._element_arrays(dofs)
+    def freeze_slab_elements(self, dofs, col_dofs=None):
+        """freeze_slab for the stream insert_elements(dofs, ., col_dofs=col_dofs) stages ((ncells, k) connectivity,
+        or (ncells, kr) rows and (ncells, kc) columns)."""
+        dofs, col_dofs, _, ncells, kr, kc = self._element_arrays(dofs, None, col_dofs)
         counts = self._rank_counts()
-        self._c(lib().xsb_freeze_slab_elements(self._h, k, ncells, ptr(dofs), counts))
+        if col_dofs is None:
+            self._c(lib().xsb_freeze_slab_elements(self._h, kr, ncells, ptr(dofs), counts))
+        else:
+            self._c(lib().xsb_freeze_slab_elements_rect(self._h, kr, kc, ncells, ptr(dofs), ptr(col_dofs), counts))
         return [int(c) for c in counts]
 
     def freeze_slab_prepare(self, send_positions, capacity):

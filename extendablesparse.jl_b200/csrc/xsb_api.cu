@@ -525,6 +525,21 @@ struct DevIn
     ~DevIn() { h->dfree(tmp); }
 };
 
+// the connectivity of an element batch on the device; the square loop's one array moves once
+struct ElementDofs
+{
+    DevIn r, c;
+    ElementBatch batch;
+    ElementDofs(xsb_matrix *h, int32_t kr, int32_t kc, i64 ncells, const void *rdofs, const void *cdofs,
+                const double *Aloc = nullptr)
+        : r(h, rdofs, h->isz() * (size_t)kr * (size_t)ncells),
+          c(h, square(kr, kc, rdofs, cdofs) ? nullptr : cdofs, h->isz() * (size_t)kc * (size_t)ncells),
+          batch{r.ptr, square(kr, kc, rdofs, cdofs) ? r.ptr : c.ptr, Aloc, kr, kc, ncells}
+    {
+    }
+    static bool square(int32_t kr, int32_t kc, const void *rdofs, const void *cdofs) { return rdofs == cdofs && kr == kc; }
+};
+
 struct DevOut
 {
     xsb_matrix *h;
@@ -1236,13 +1251,14 @@ void end_emit(xsb_matrix *h, int32_t tid, int32_t flavour, i64 count)
         h->has_assign = true;
 }
 
-// the limits of an element batch: k in [1, 64]; its k^2 ncells calls stay below 2^63
-i64 element_calls(int32_t k, int64_t ncells)
+// the limits of an element batch: kr, kc in [1, 64]; its kr kc ncells calls stay below 2^63
+i64 element_calls(int32_t kr, int32_t kc, int64_t ncells)
 {
-    REQUIRE(k >= 1 && k <= 64, XSB_EINVAL, "element size k must be in [1, 64]");
+    REQUIRE(kr >= 1 && kr <= 64 && kc >= 1 && kc <= 64, XSB_EINVAL,
+            kr == kc ? "element size k must be in [1, 64]" : "element sizes kr and kc must be in [1, 64]");
     REQUIRE(ncells >= 0, XSB_EINVAL, "negative element count");
-    REQUIRE(ncells <= INT64_MAX / ((i64)k * k), XSB_EINVAL, "k^2 * ncells overflows");
-    return (i64)k * k * ncells;
+    REQUIRE(ncells <= INT64_MAX / ((i64)kr * kc), XSB_EINVAL, kr == kc ? "k^2 * ncells overflows" : "kr * kc * ncells overflows");
+    return (i64)kr * kc * ncells;
 }
 
 // xsb_freeze_pattern / xsb_freeze_elements
@@ -2312,34 +2328,41 @@ int32_t xsb_insert_triplets(xsb_matrix *h, int32_t tid, const xsb_triplet *T, in
 int32_t xsb_insert_elements(xsb_matrix *h, int32_t tid, int32_t k, int64_t ncells, const void *dofs, const double *Aloc,
                             int32_t flavour)
 {
+    return xsb_insert_elements_rect(h, tid, k, k, ncells, dofs, dofs, Aloc, flavour);
+}
+
+int32_t xsb_insert_elements_rect(xsb_matrix *h, int32_t tid, int32_t kr, int32_t kc, int64_t ncells, const void *rdofs,
+                                 const void *cdofs, const double *Aloc, int32_t flavour)
+{
     return guard(h, [&]() -> int32_t {
         REQUIRE(h, XSB_EINVAL, "NULL handle");
         check_tid_flavour(h, tid, flavour);
-        const i64 count = element_calls(k, ncells);
+        const i64 count = element_calls(kr, kc, ncells);
         if (count == 0)
             return XSB_OK;
-        REQUIRE(dofs && Aloc, XSB_EINVAL, "NULL array");
+        REQUIRE(rdofs && cdofs && Aloc, XSB_EINVAL, "NULL array");
         Rec *dst = begin_emit(h, tid, flavour, count);
-        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells), dA(h, Aloc, 8 * (size_t)count);
+        DevIn dA(h, Aloc, 8 * (size_t)count);
+        const ElementDofs ed(h, kr, kc, ncells, rdofs, cdofs, static_cast<const double *>(dA.ptr));
+        const ElementBatch &eb = ed.batch;
         write_scalar(h, 1, ~0ull);
         RunTarget rt;
         u32 chunk0 = 0, pos0 = 0, chunks = 0;
-        const bool grouped = runs_begin(h, tid, count, insert_elements_chunks(k, ncells), &rt, &chunk0, &pos0);
-        const i64 nmax = std::min<i64>(h->m, h->n_global); // a dof is the row and the column of its element's calls
+        const bool grouped = runs_begin(h, tid, count, insert_elements_chunks(kr, kc, ncells), &rt, &chunk0, &pos0);
         if (grouped)
-            chunks = insert_elements_grouped(h->stream, dD.ptr, static_cast<const double *>(dA.ptr), k, ncells, h->idx64,
-                                             h->base, nmax, h->Ls, (u32)tid, (u32)flavour, dst, h->d_scal + 1, h->lc,
-                                             h->stage_flags(tid), rt, chunk0, pos0);
+            chunks = insert_elements_grouped(h->stream, eb, h->idx64, h->base, h->m, h->n_global, h->Ls, (u32)tid,
+                                             (u32)flavour, dst, h->d_scal + 1, h->lc, h->stage_flags(tid), rt, chunk0, pos0);
         else
-            insert_elements(h->stream, dD.ptr, static_cast<const double *>(dA.ptr), k, ncells, h->idx64, h->base, nmax, h->Ls,
-                            (u32)tid, (u32)flavour, dst, h->d_scal + 1, h->lc, h->stage_flags(tid));
+            insert_elements(h->stream, eb, h->idx64, h->base, h->m, h->n_global, h->Ls, (u32)tid, (u32)flavour, dst,
+                            h->d_scal + 1, h->lc, h->stage_flags(tid));
         const u64 bad = read_scalar(h, 1);
         if (bad != ~0ull)
         {
             if (grouped)
                 h->runs.dead = true; // the rejected batch left runs behind: the index is rebuilt at flush time
-            throw ApiError(XSB_EBOUNDS, "BoundsError: element " + std::to_string(bad) +
-                                            " of the batch has a dof outside the matrix; batch rejected");
+            const char *what = ElementDofs::square(kr, kc, rdofs, cdofs) ? "a dof" : (bad & 1u) ? "a column dof" : "a row dof";
+            throw ApiError(XSB_EBOUNDS, "BoundsError: element " + std::to_string(bad >> 1) + " of the batch has " + what +
+                                            " outside the matrix; batch rejected");
         }
         if (h->n_tid > 1 && flavour == XSB_ASSIGN)
             check_mt_assign(h, dst, count);
@@ -2438,16 +2461,22 @@ int32_t xsb_freeze_pattern(xsb_matrix *h, const void *I, const void *J, int64_t 
 
 int32_t xsb_freeze_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs)
 {
+    return xsb_freeze_elements_rect(h, k, k, ncells, dofs, dofs);
+}
+
+int32_t xsb_freeze_elements_rect(xsb_matrix *h, int32_t kr, int32_t kc, int64_t ncells, const void *rdofs,
+                                 const void *cdofs)
+{
     return guard(h, [&]() -> int32_t {
         REQUIRE(h, XSB_EINVAL, "NULL handle");
-        const i64 count = element_calls(k, ncells);
+        const i64 count = element_calls(kr, kc, ncells);
         freeze_check(h, count);
-        REQUIRE(count == 0 || dofs, XSB_EINVAL, "NULL array");
+        REQUIRE(count == 0 || (rdofs && cdofs), XSB_EINVAL, "NULL array");
         h->drop_frozen();
-        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells);
+        ElementDofs ed(h, kr, kc, ncells, rdofs, cdofs);
         return freeze_impl(h, count, [&](i64 *slot) {
-            lookup_slots_elements(h->stream, h->view(), h->m, h->n, h->idx64, h->base, dD.ptr, k, count, slot, h->d_scal + 2,
-                                  h->d_scal + 3, h->lc);
+            lookup_slots_elements(h->stream, h->view(), h->m, h->n, h->idx64, h->base, ed.batch, count, slot,
+                                  h->d_scal + 2, h->d_scal + 3, h->lc);
         });
     });
 }
@@ -2518,15 +2547,21 @@ int32_t xsb_freeze_slab(xsb_matrix *h, const void *I, const void *J, int64_t cou
 
 int32_t xsb_freeze_slab_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs, int64_t *send_counts)
 {
+    return xsb_freeze_slab_elements_rect(h, k, k, ncells, dofs, dofs, send_counts);
+}
+
+int32_t xsb_freeze_slab_elements_rect(xsb_matrix *h, int32_t kr, int32_t kc, int64_t ncells, const void *rdofs,
+                                      const void *cdofs, int64_t *send_counts)
+{
     return guard(h, [&]() -> int32_t {
         slab_freeze_check(h);
-        const i64 count = element_calls(k, ncells);
+        const i64 count = element_calls(kr, kc, ncells);
         freeze_check(h, count);
-        REQUIRE(count == 0 || dofs, XSB_EINVAL, "NULL array");
+        REQUIRE(count == 0 || (rdofs && cdofs), XSB_EINVAL, "NULL array");
         h->drop_frozen();
-        DevIn dD(h, dofs, h->isz() * (size_t)k * (size_t)ncells);
+        ElementDofs ed(h, kr, kc, ncells, rdofs, cdofs);
         return freeze_slab_impl(h, count, send_counts, [&](i64 *slot, Rec *tags) {
-            slab_classify_elements(h->stream, h->view(), h->m, h->n_global, h->Ls, h->idx64, h->base, dD.ptr, k, count,
+            slab_classify_elements(h->stream, h->view(), h->m, h->n_global, h->Ls, h->idx64, h->base, ed.batch, count,
                                    slot, tags, h->d_scal + 2, h->d_scal + 3, h->lc);
         });
     });

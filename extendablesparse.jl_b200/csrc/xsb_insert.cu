@@ -1423,74 +1423,94 @@ void emit_blockrd(cudaStream_t stream, i64 nx, i64 ny, i64 nz, int ns, u64 seed,
 }
 
 // ------------------------------------------------------------------------
-// Element-by-element insertion (test/femtools.jl:45-72 with the caller's mesh): connectivity dofs[k x ncells] and
-// dense element matrices Aloc[k x k x ncells], both column-major.  Call p = k^2 c + k jl + il is
-// (row = dofs[il, c], col = dofs[jl, c], v = Aloc[il, jl, c]): the records of one (element, column) VISIT are k
+// Element-by-element insertion (test/femtools.jl:45-72 with the caller's mesh): row connectivity rdofs[kr x ncells],
+// column connectivity cdofs[kc x ncells] and dense element matrices Aloc[kr x kc x ncells], all column-major (the
+// square loop: kr == kc, rdofs == cdofs).  Call p = kr kc c + kr jl + il is
+// (row = rdofs[il, c], col = cdofs[jl, c], v = Aloc[il, jl, c]): the records of one (element, column) VISIT are kr
 // neighbours in call order.
 //
-// A warp owns a chunk of whole elements (at most EL_VISITS visits).  Grouped (xsb_chunk.cuh): the chunk's visits run
-// through the warp's table with match.any (neighbouring elements share columns) and every visit stands for k
-// records, so a record goes to start[slot] + k x (visits of its column before its own) + il -- stable, also when an
-// element repeats a dof.  A column holds at most EL_VISITS records of a chunk when the elements' dofs are distinct;
-// repeated dofs can pile up more than one run may hold (CH_RUN_MAX): such a column is published as several runs
+// A warp owns a chunk of whole elements (at most EL_VISITS visits and EL_VISITS row dofs).  Grouped (xsb_chunk.cuh):
+// the chunk's visits run through the warp's table with match.any (neighbouring elements share columns) and every
+// visit stands for kr records, so a record goes to start[slot] + kr x (visits of its column before its own) + il --
+// stable, also when an element repeats a dof.  A column holds at most 128 min(kr, kc) records of a chunk; repeated
+// column dofs can pile up more than one run may hold (CH_RUN_MAX): such a column is published as several runs
 // (chunk_publish_split).  Call order (ungrouped): record p goes to p.  Either way the lanes walk the
 // chunk's values in memory order (coalesced 8-byte loads) and store one 16-byte record each; consecutive lanes store
 // consecutive records wherever they belong to one visit, so the stores merge into whole sectors there.
 // ------------------------------------------------------------------------
 constexpr int EL_WARPS = 4;
-constexpr int EL_VISITS = 128; // visits per chunk: records (<= 128 k <= 8192) fit the 16-bit run offsets
+constexpr int EL_VISITS = 128; // visits per chunk: records (<= 128 min(kr, kc) <= 8192) fit the 16-bit run offsets
 constexpr int EL_HB = 8;       // 256 table slots for at most 128 distinct columns
 struct ElWarpSpace
 {
-    u64 ckey[EL_VISITS]; // dof l of the chunk (l = element * k + local node): column half of its keys
-    u64 rkey[EL_VISITS]; // ... and row half
-    u32 vis[EL_VISITS];  // visit l: (slot << 16 | visits of its column before it)
+    u64 ckey[EL_VISITS]; // visit v = element * kc + jl of the chunk: column half of its keys
+    u64 rkey[EL_VISITS]; // row dof l = element * kr + il of the chunk: row half of its keys
+    u32 vis[EL_VISITS];  // visit v: (slot << 16 | visits of its column before it)
     ChunkSpaceT<EL_HB> tab;
 };
 static_assert(ChunkSpaceT<EL_HB>::DMAX >= EL_VISITS, "a chunk's visits must fit the table");
 
-__host__ __device__ __forceinline__ int el_cells_per_chunk(int k) { return EL_VISITS / k; }
+__host__ __device__ __forceinline__ int el_cells_per_chunk(int kr, int kc) { return EL_VISITS / (kr > kc ? kr : kc); }
 
-u32 insert_elements_chunks(int k, i64 ncells)
+u32 insert_elements_chunks(int kr, int kc, i64 ncells)
 {
-    const i64 e = el_cells_per_chunk(k);
+    const i64 e = el_cells_per_chunk(kr, kc);
     return (u32)((ncells + e - 1) / e);
 }
 
+// x / k for x < 128 k: (x * ceil(2^22 / k)) >> 22 is exact there (k <= 64) and stays in 32 bits
+struct DivK
+{
+    u32 inv;
+    __device__ __forceinline__ explicit DivK(u32 k) : inv(((1u << 22) + k - 1u) / k) {}
+    __device__ __forceinline__ u32 operator()(u32 x) const { return (x * inv) >> 22; }
+};
+
 template <typename Ti, bool GROUPED>
 __global__ void __launch_bounds__(EL_WARPS * 32)
-insert_elements_kernel(const Ti *__restrict__ dofs, const double *__restrict__ Aloc, int k, i64 ncells, i64 base, i64 nmax,
-                       KeyLayout L, u32 tid, u32 flavour, Rec *__restrict__ out, u64 *__restrict__ d_err, StageFlags sf,
-                       RunTarget rt, u32 chunk0, u32 pos0)
+insert_elements_kernel(const Ti *__restrict__ rdofs, const Ti *__restrict__ cdofs, const double *__restrict__ Aloc, int kr,
+                       int kc, i64 ncells, i64 base, i64 m, i64 n, KeyLayout L, u32 tid, u32 flavour,
+                       Rec *__restrict__ out, u64 *__restrict__ d_err, StageFlags sf, RunTarget rt, u32 chunk0, u32 pos0)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     ElWarpSpace &sp = reinterpret_cast<ElWarpSpace *>(smem_raw)[warp];
     const u32 chunk = blockIdx.x * EL_WARPS + warp;
-    const i64 per = el_cells_per_chunk(k);
+    const i64 per = el_cells_per_chunk(kr, kc);
     const i64 e0 = (i64)chunk * per;
     if (e0 >= ncells)
         return;
-    const u32 uk = (u32)k;
-    const u32 nvis = (u32)(min(per, ncells - e0) * k); // visits = dofs of the chunk
-    const u32 nrec = nvis * uk;
-    const i64 c0 = e0 * k * k; // position of the chunk's first record (call order)
-    // x / k for x < 128 k (every x below): (x * ceil(2^22 / k)) >> 22 is exact there and stays in 32 bits
-    const u32 kinv = ((1u << 22) + uk - 1u) / uk;
-    auto divk = [&](u32 x) { return (x * kinv) >> 22; };
+    const u32 ukr = (u32)kr, ukc = (u32)kc;
+    const u32 ne = (u32)min(per, ncells - e0);
+    const u32 nvis = ne * ukc; // visits = column dofs of the chunk
+    const u32 nrow = ne * ukr; // row dofs of the chunk
+    const u32 nrec = nvis * ukr;
+    const i64 c0 = e0 * kr * kc; // position of the chunk's first record (call order)
+    // every quotient below has a dividend under 128 x its divisor: p < nrec <= 128 min(kr, kc), v < nvis <= 128
+    const DivK divr(ukr), divc(ukc);
+    // *d_err: 2 x element + (1 for a column dof), so the first offending element wins
     bool foreign = false;
     for (u32 l = lane; l < nvis; l += 32)
     {
-        i64 d = (i64)dofs[e0 * k + l] - base;
-        if (d < 0 || d >= nmax)
+        i64 d = (i64)cdofs[e0 * kc + l] - base;
+        if (d < 0 || d >= n)
         { // BoundsError (sparsematrixcsc.jl:8-10): the batch is rejected, whatever is written for it is dropped
-            atomicMin(d_err, (u64)(e0 + divk(l)));
+            atomicMin(d_err, ((u64)(e0 + divc(l)) << 1) | 1u);
             d = 0;
         }
         const u64 ck = L.colpart((u64)d);
         sp.ckey[l] = ck;
-        sp.rkey[l] = L.rowpart((u64)d, tid, flavour);
         foreign |= sf.flags != nullptr && L.owner(ck) != (u32)L.self;
+    }
+    for (u32 l = lane; l < nrow; l += 32)
+    {
+        i64 d = (i64)rdofs[e0 * kr + l] - base;
+        if (d < 0 || d >= m)
+        {
+            atomicMin(d_err, (u64)(e0 + divr(l)) << 1);
+            d = 0;
+        }
+        sp.rkey[l] = L.rowpart((u64)d, tid, flavour);
     }
     // slab handles: only chunks that hold a column of another rank mark route tiles
     if (!__any_sync(0xffffffffu, foreign))
@@ -1517,27 +1537,27 @@ insert_elements_kernel(const Ti *__restrict__ dofs, const double *__restrict__ A
         }
         __syncwarp();
         if (nrec > CH_RUN_MAX) // warp-uniform
-        {                      // a column holds k x (its visits) records of the chunk
+        {                      // a column holds kr x (its visits) records of the chunk
             bool over = false;
             for (u32 v = lane; v < nvis; v += 32)
-                over |= ((sp.vis[v] & 0xffffu) + 1u) * uk > CH_RUN_MAX;
+                over |= ((sp.vis[v] & 0xffffu) + 1u) * ukr > CH_RUN_MAX;
             split = __any_sync(0xffffffffu, over);
         }
-        chunk_scan(sp.tab, d, lane, uk);
+        chunk_scan(sp.tab, d, lane, ukr);
     }
     const double *src = Aloc + c0;
     Rec *dst = out + c0;
     auto put = [&](u32 p, double val) {
-        const u32 v = divk(p), il = p - v * uk; // visit (dof of the column) and row rank inside it
-        const u32 jl = v - divk(v) * uk;        // the column's local node
+        const u32 v = divr(p), il = p - v * ukr; // visit (element, column dof) and row rank inside it
+        const u32 e = divc(v);                   // the chunk's element
         Rec r;
-        r.key = sp.ckey[v] | sp.rkey[v - jl + il];
+        r.key = sp.ckey[v] | sp.rkey[e * ukr + il];
         r.val = val;
         u32 t = p;
         if (GROUPED)
         {
             const u32 vs = sp.vis[v];
-            t = (u32)sp.tab.start[vs >> 16] + uk * (vs & 0xffffu) + il;
+            t = (u32)sp.tab.start[vs >> 16] + ukr * (vs & 0xffffu) + il;
         }
         st_rec(dst + t, r);
         if (sf.flags != nullptr && L.owner(r.key) != (u32)L.self)
@@ -1558,53 +1578,50 @@ insert_elements_kernel(const Ti *__restrict__ dofs, const double *__restrict__ A
     for (u32 p = p0 + lane; p < nrec; p += 32)
         put(p, __ldcs(src + p));
     if (GROUPED && !split)
-        chunk_publish(sp.tab, rt, chunk0 + chunk, pos0 + (u32)c0, d, true, lane, uk);
+        chunk_publish(sp.tab, rt, chunk0 + chunk, pos0 + (u32)c0, d, true, lane, ukr);
     else if (GROUPED)
-        chunk_publish_split(sp.tab, rt, chunk0 + chunk, pos0 + (u32)c0, d, lane, uk);
+        chunk_publish_split(sp.tab, rt, chunk0 + chunk, pos0 + (u32)c0, d, lane, ukr);
 }
 
 template <typename Ti, bool GROUPED>
-static void launch_insert_elements(cudaStream_t stream, const Ti *dofs, const double *Aloc, int k, i64 ncells, int base,
-                                   i64 nmax, const KeyLayout &L, u32 tid, u32 flavour, Rec *out, u64 *d_err, StageFlags sf,
-                                   const RunTarget &rt, u32 chunk0, u32 pos0, LaunchCounter &lc)
+static void launch_insert_elements(cudaStream_t stream, const ElementBatch &eb, int base, i64 m, i64 n, const KeyLayout &L,
+                                   u32 tid, u32 flavour, Rec *out, u64 *d_err, StageFlags sf, const RunTarget &rt,
+                                   u32 chunk0, u32 pos0, LaunchCounter &lc)
 {
     static FuncAttrOnce once;
     const int smem = (int)(sizeof(ElWarpSpace) * EL_WARPS);
     once.set(insert_elements_kernel<Ti, GROUPED>, smem, true);
-    const u32 chunks = insert_elements_chunks(k, ncells);
+    const u32 chunks = insert_elements_chunks(eb.kr, eb.kc, eb.ncells);
     insert_elements_kernel<Ti, GROUPED><<<(chunks + EL_WARPS - 1) / EL_WARPS, EL_WARPS * 32, smem, stream>>>(
-        dofs, Aloc, k, ncells, (i64)base, nmax, L, tid, flavour, out, d_err, sf, rt, chunk0, pos0);
+        (const Ti *)eb.rdofs, (const Ti *)eb.cdofs, eb.Aloc, eb.kr, eb.kc, eb.ncells, (i64)base, m, n, L, tid, flavour, out,
+        d_err, sf, rt, chunk0, pos0);
     lc.add();
     XSB_CUDA(cudaGetLastError());
 }
 
-void insert_elements(cudaStream_t stream, const void *dofs, const double *Aloc, int k, i64 ncells, int idx64, int base,
-                     i64 nmax, KeyLayout L, u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf)
+void insert_elements(cudaStream_t stream, const ElementBatch &eb, int idx64, int base, i64 m, i64 n, KeyLayout L, u32 tid,
+                     u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf)
 {
-    if (ncells <= 0)
+    if (eb.ncells <= 0)
         return;
     const RunTarget none{};
     if (idx64)
-        launch_insert_elements<int64_t, false>(stream, (const int64_t *)dofs, Aloc, k, ncells, base, nmax, L, tid, flavour,
-                                               out, d_err, sf, none, 0, 0, lc);
+        launch_insert_elements<int64_t, false>(stream, eb, base, m, n, L, tid, flavour, out, d_err, sf, none, 0, 0, lc);
     else
-        launch_insert_elements<int32_t, false>(stream, (const int32_t *)dofs, Aloc, k, ncells, base, nmax, L, tid, flavour,
-                                               out, d_err, sf, none, 0, 0, lc);
+        launch_insert_elements<int32_t, false>(stream, eb, base, m, n, L, tid, flavour, out, d_err, sf, none, 0, 0, lc);
 }
 
-u32 insert_elements_grouped(cudaStream_t stream, const void *dofs, const double *Aloc, int k, i64 ncells, int idx64,
-                            int base, i64 nmax, KeyLayout L, u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc,
-                            StageFlags sf, const RunTarget &rt, u32 chunk0, u32 pos0)
+u32 insert_elements_grouped(cudaStream_t stream, const ElementBatch &eb, int idx64, int base, i64 m, i64 n, KeyLayout L,
+                            u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf,
+                            const RunTarget &rt, u32 chunk0, u32 pos0)
 {
-    if (ncells <= 0)
+    if (eb.ncells <= 0)
         return 0;
     if (idx64)
-        launch_insert_elements<int64_t, true>(stream, (const int64_t *)dofs, Aloc, k, ncells, base, nmax, L, tid, flavour,
-                                              out, d_err, sf, rt, chunk0, pos0, lc);
+        launch_insert_elements<int64_t, true>(stream, eb, base, m, n, L, tid, flavour, out, d_err, sf, rt, chunk0, pos0, lc);
     else
-        launch_insert_elements<int32_t, true>(stream, (const int32_t *)dofs, Aloc, k, ncells, base, nmax, L, tid, flavour,
-                                              out, d_err, sf, rt, chunk0, pos0, lc);
-    return insert_elements_chunks(k, ncells);
+        launch_insert_elements<int32_t, true>(stream, eb, base, m, n, L, tid, flavour, out, d_err, sf, rt, chunk0, pos0, lc);
+    return insert_elements_chunks(eb.kr, eb.kc, eb.ncells);
 }
 
 } // namespace xsb

@@ -259,16 +259,26 @@ u32 emit_blockrd_grouped(cudaStream_t stream, i64 nx, i64 ny, i64 nz, int ns, u6
 u32 emit_p1fem_chunks(i64 nxn, i64 nyn, i64 cz_begin, i64 cz_end);
 u32 emit_p1fem_grouped(cudaStream_t stream, i64 nxn, i64 nyn, i64 nzn, KeyLayout L, u32 tid, u32 flavour, i64 cz_begin,
                        i64 cz_end, Rec *out, LaunchCounter &lc, StageFlags sf, const RunTarget &rt, u32 chunk0, u32 pos0);
-// element-by-element insertion: k x ncells connectivity + k x k x ncells element matrices (column-major) -> the
-// k^2 ncells records of the element loop; nmax = min(rows, columns); *d_err receives the first offending element.
-// insert_elements stores call order, insert_elements_grouped groups chunks of whole elements and returns the chunks
-// appended to the run index (insert_elements_chunks(k, ncells)).
-u32 insert_elements_chunks(int k, i64 ncells);
-void insert_elements(cudaStream_t stream, const void *dofs, const double *Aloc, int k, i64 ncells, int idx64, int base,
-                     i64 nmax, KeyLayout L, u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf);
-u32 insert_elements_grouped(cudaStream_t stream, const void *dofs, const double *Aloc, int k, i64 ncells, int idx64,
-                            int base, i64 nmax, KeyLayout L, u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc,
-                            StageFlags sf, const RunTarget &rt, u32 chunk0, u32 pos0);
+// element-by-element insertion: an element loop given as connectivity and dense element matrices, Julia's
+// column-major arrays (rdofs kr x ncells and cdofs kc x ncells in the handle's index type, Aloc kr x kc x ncells;
+// the square loop passes rdofs == cdofs): call p = kr kc c + kr jl + il is (rdofs[il, c], cdofs[jl, c], Aloc[il, jl, c])
+struct ElementBatch
+{
+    const void *rdofs, *cdofs;
+    const double *Aloc;
+    int kr, kc;
+    i64 ncells;
+};
+// -> the kr kc ncells records of the loop; a row dof must lie below m, a column dof below n.  *d_err receives
+// 2 x (first offending element) + (1 if a column dof is at fault).  insert_elements stores call order,
+// insert_elements_grouped groups chunks of whole elements and returns the chunks appended to the run index
+// (insert_elements_chunks(kr, kc, ncells)).
+u32 insert_elements_chunks(int kr, int kc, i64 ncells);
+void insert_elements(cudaStream_t stream, const ElementBatch &eb, int idx64, int base, i64 m, i64 n, KeyLayout L, u32 tid,
+                     u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf);
+u32 insert_elements_grouped(cudaStream_t stream, const ElementBatch &eb, int idx64, int base, i64 m, i64 n, KeyLayout L,
+                            u32 tid, u32 flavour, Rec *out, u64 *d_err, LaunchCounter &lc, StageFlags sf,
+                            const RunTarget &rt, u32 chunk0, u32 pos0);
 // pointblock (xsb_values.cu): CSC entries -> records of the block pattern; values into the blocks
 void pointblock_emit(cudaStream_t stream, const CscView &csc, i64 n, int idx64, int base, i64 bs, i64 nb,
                      KeyLayout Lb, Rec *out, u64 *d_err, LaunchCounter &lc);
@@ -294,9 +304,9 @@ void fill_index(cudaStream_t stream, void *x, i64 count, int idx64, i64 value, L
 // slot[k] = nz index of (I[k],J[k]) or -1; *d_missing counts the absent ones
 void lookup_slots(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *I,
                   const void *J, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc);
-// the same for the calls of an element loop (dofs: k x ncells, column-major; count = k^2 ncells)
-void lookup_slots_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *dofs,
-                           int k, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc);
+// the same for the calls of an element loop (eb.Aloc unused; count = kr kc ncells)
+void lookup_slots_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base,
+                           const ElementBatch &eb, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc);
 void gather_values(cudaStream_t stream, const double *nzval, const i64 *slot, i64 count, double *out,
                    LaunchCounter &lc);
 void count_missing_records(cudaStream_t stream, const Rec *recs, i64 count, const KeyLayout &L, const CscView &csc,
@@ -326,7 +336,7 @@ void slab_classify(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global,
                    const void *I, const void *J, i64 count, i64 *slot, Rec *tags, u64 *d_missing, u64 *d_oob,
                    LaunchCounter &lc);
 void slab_classify_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64,
-                            int base, const void *dofs, int k, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
+                            int base, const ElementBatch &eb, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
                             u64 *d_oob, LaunchCounter &lc);
 // gathered tags -> stream indices and {row, column} positions
 void slab_split(cudaStream_t stream, const Rec *tags, i64 n, u32 *idx, u64 *where, LaunchCounter &lc);

@@ -90,6 +90,28 @@ template <typename Ti> struct PosElements
         j = (i64)dofs[c * k + jl];
     }
 };
+template <typename Ti> struct PosElementsRect
+{
+    const Ti *rdofs, *cdofs; // kr x ncells and kc x ncells, column-major
+    i64 kr, kc;
+    // call p = kr kc c + kr jl + il is (rdofs[il, c], cdofs[jl, c])
+    __device__ __forceinline__ void at(i64 p, i64 &i, i64 &j) const
+    {
+        const i64 kk = kr * kc, c = p / kk, r = p - c * kk, jl = r / kr;
+        i = (i64)rdofs[c * kr + (r - jl * kr)];
+        j = (i64)cdofs[c * kc + jl];
+    }
+};
+
+// the square loop (one connectivity for rows and columns) reads it through PosElements, anything else through
+// PosElementsRect
+template <typename Ti, class F> static void with_element_pos(const ElementBatch &eb, F &&f)
+{
+    if (eb.rdofs == eb.cdofs && eb.kr == eb.kc)
+        f(PosElements<Ti>{(const Ti *)eb.rdofs, (i64)eb.kr});
+    else
+        f(PosElementsRect<Ti>{(const Ti *)eb.rdofs, (const Ti *)eb.cdofs, (i64)eb.kr, (i64)eb.kc});
+}
 
 template <typename Ti, class Pos>
 __global__ void __launch_bounds__(256)
@@ -139,15 +161,17 @@ void lookup_slots(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx
                                d_missing, d_oob, lc);
 }
 
-void lookup_slots_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, const void *dofs,
-                           int k, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
+void lookup_slots_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base,
+                           const ElementBatch &eb, i64 count, i64 *slot, u64 *d_missing, u64 *d_oob, LaunchCounter &lc)
 {
     if (idx64)
-        launch_lookup<int64_t>(stream, csc, m, n, base, PosElements<int64_t>{(const int64_t *)dofs, (i64)k}, count, slot,
-                               d_missing, d_oob, lc);
+        with_element_pos<int64_t>(eb, [&](auto pos) {
+            launch_lookup<int64_t>(stream, csc, m, n, base, pos, count, slot, d_missing, d_oob, lc);
+        });
     else
-        launch_lookup<int32_t>(stream, csc, m, n, base, PosElements<int32_t>{(const int32_t *)dofs, (i64)k}, count, slot,
-                               d_missing, d_oob, lc);
+        with_element_pos<int32_t>(eb, [&](auto pos) {
+            launch_lookup<int32_t>(stream, csc, m, n, base, pos, count, slot, d_missing, d_oob, lc);
+        });
 }
 
 __global__ void __launch_bounds__(256)
@@ -440,15 +464,17 @@ void slab_classify(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global,
 }
 
 void slab_classify_elements(cudaStream_t stream, const CscView &csc, i64 m, i64 n_global, const KeyLayout &Ls, int idx64,
-                            int base, const void *dofs, int k, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
+                            int base, const ElementBatch &eb, i64 count, i64 *slot, Rec *tags, u64 *d_missing,
                             u64 *d_oob, LaunchCounter &lc)
 {
     if (idx64)
-        launch_classify<int64_t>(stream, csc, m, n_global, Ls, base, PosElements<int64_t>{(const int64_t *)dofs, (i64)k},
-                                 count, slot, tags, d_missing, d_oob, lc);
+        with_element_pos<int64_t>(eb, [&](auto pos) {
+            launch_classify<int64_t>(stream, csc, m, n_global, Ls, base, pos, count, slot, tags, d_missing, d_oob, lc);
+        });
     else
-        launch_classify<int32_t>(stream, csc, m, n_global, Ls, base, PosElements<int32_t>{(const int32_t *)dofs, (i64)k},
-                                 count, slot, tags, d_missing, d_oob, lc);
+        with_element_pos<int32_t>(eb, [&](auto pos) {
+            launch_classify<int32_t>(stream, csc, m, n_global, Ls, base, pos, count, slot, tags, d_missing, d_oob, lc);
+        });
 }
 
 // the gathered tags -> stream indices (kept for every step) and 8-byte positions {row, owner-relative column}

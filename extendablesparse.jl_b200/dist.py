@@ -133,8 +133,8 @@ class DistExtendableSparseMatrix:
     def insert_batch(self, I, J, V, flavour=0):
         self.h.insert_batch(I, J, V, flavour)
 
-    def insert_elements(self, dofs, Aloc, flavour=1):  # XSB_RAW: the element loop's rawupdateindex!
-        self.h.insert_elements(dofs, Aloc, flavour)
+    def insert_elements(self, dofs, Aloc, flavour=1, col_dofs=None):  # XSB_RAW: the element loop's rawupdateindex!
+        self.h.insert_elements(dofs, Aloc, flavour, col_dofs=col_dofs)
 
     def _send_buffer(self, records: int) -> torch.Tensor:
         words = 2 * max(records, 1)
@@ -479,10 +479,10 @@ class DistExtendableSparseMatrix:
         outside the matrix or absent from the pattern) fails the freeze on every rank and leaves every rank unfrozen."""
         self._freeze(lambda: self.h.freeze_slab(I, J))
 
-    def freeze_elements(self, dofs):
-        """freeze_pattern for the stream insert_elements(dofs, .) stages: reassemble_values then takes the element
-        matrices (ncells, k, k) as they are."""
-        self._freeze(lambda: self.h.freeze_slab_elements(dofs))
+    def freeze_elements(self, dofs, col_dofs=None):
+        """freeze_pattern for the stream insert_elements(dofs, ., col_dofs=col_dofs) stages: reassemble_values then
+        takes the element matrices ((ncells, k, k), or (ncells, kc, kr) with col_dofs) as they are."""
+        self._freeze(lambda: self.h.freeze_slab_elements(dofs, col_dofs))
 
     def unfreeze(self):
         self.h.unfreeze()

@@ -237,6 +237,23 @@ function insert_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}, Aloc::Arra
                           a.handle, tid, k, size(dofs, 2), dofs, Aloc, flavour))
 end
 
+"""
+    insert_elements!(a, rowdofs, coldofs, Aloc; flavour = XSB_RAW, tid = 0)
+
+The element loop whose rows and columns come from different connectivities (coupling blocks, rectangular
+operators): for every cell `c`, `for jl, for il`, `rawupdateindex!(A, +, Aloc[il, jl, c], rowdofs[il, c],
+coldofs[jl, c])`.  `rowdofs` is kr x ncells, `coldofs` kc x ncells, `Aloc` kr x kc x ncells.
+"""
+function insert_elements!(a::B200Assembler{Tv, Ti}, rowdofs::Matrix{Ti}, coldofs::Matrix{Ti}, Aloc::Array{Tv, 3};
+                          flavour = XSB_RAW, tid = 0) where {Tv, Ti}
+    kr, kc, ncells = size(rowdofs, 1), size(coldofs, 1), size(rowdofs, 2)
+    size(coldofs, 2) == ncells || throw(DimensionMismatch("rowdofs and coldofs must have the same number of cells"))
+    size(Aloc) == (kr, kc, ncells) || throw(DimensionMismatch("size(Aloc) must be (kr, kc, ncells)"))
+    check(a.handle, ccall((:xsb_insert_elements_rect, libxsb), Int32,
+                          (Ptr{Cvoid}, Int32, Int32, Int32, Int64, Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Cvoid}, Int32),
+                          a.handle, tid, kr, kc, ncells, rowdofs, coldofs, Aloc, flavour))
+end
+
 "flush! + sparse(A): two-phase -- query nnz, allocate Julia arrays, fetch (ownership stays with Julia)"
 function fetch!(a::B200Assembler{Tv, Ti}, mode = XSB_DETERMINISTIC) where {Tv, Ti}
     nnz = Ref{Int64}(0); changed = Ref{Int32}(0)
@@ -259,6 +276,12 @@ end
 function freeze_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}) where {Tv, Ti}
     check(a.handle, ccall((:xsb_freeze_elements, libxsb), Int32, (Ptr{Cvoid}, Int32, Int64, Ptr{Cvoid}),
                           a.handle, size(dofs, 1), size(dofs, 2), dofs))
+end
+"freeze! for the element loop of insert_elements!(a, rowdofs, coldofs, Aloc)"
+function freeze_elements!(a::B200Assembler{Tv, Ti}, rowdofs::Matrix{Ti}, coldofs::Matrix{Ti}) where {Tv, Ti}
+    size(coldofs, 2) == size(rowdofs, 2) || throw(DimensionMismatch("rowdofs and coldofs must have the same number of cells"))
+    check(a.handle, ccall((:xsb_freeze_elements_rect, libxsb), Int32, (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Cvoid}, Ptr{Cvoid}),
+                          a.handle, size(rowdofs, 1), size(coldofs, 1), size(rowdofs, 2), rowdofs, coldofs))
 end
 function reassemble!(a::B200Assembler{Tv}, V::Vector{Tv}; mode = XSB_DETERMINISTIC, zero = true) where {Tv}
     # zero = true: nonzeros(A) .= 0 and the re-assembly as ONE pass over nzval (xsb_reassemble_values_zeroed)
@@ -410,6 +433,17 @@ function freeze_slab_elements!(a::B200Assembler{Tv, Ti}, dofs::Matrix{Ti}, allto
     counts = zeros(Int64, a.nranks)
     check(a.handle, ccall((:xsb_freeze_slab_elements, libxsb), Int32, (Ptr{Cvoid}, Int32, Int64, Ptr{Cvoid}, Ptr{Int64}),
                           a.handle, size(dofs, 1), size(dofs, 2), dofs, counts))
+    freeze_slab_exchange!(a, counts, alltoallv)
+end
+
+"freeze_slab! for the element loop of insert_elements!(a, rowdofs, coldofs, Aloc)"
+function freeze_slab_elements!(a::B200Assembler{Tv, Ti}, rowdofs::Matrix{Ti}, coldofs::Matrix{Ti}, alltoallv) where {Tv, Ti}
+    size(coldofs, 2) == size(rowdofs, 2) || throw(DimensionMismatch("rowdofs and coldofs must have the same number of cells"))
+    free_slab_buffers!(a)
+    counts = zeros(Int64, a.nranks)
+    check(a.handle, ccall((:xsb_freeze_slab_elements_rect, libxsb), Int32,
+                          (Ptr{Cvoid}, Int32, Int32, Int64, Ptr{Cvoid}, Ptr{Cvoid}, Ptr{Int64}),
+                          a.handle, size(rowdofs, 1), size(coldofs, 1), size(rowdofs, 2), rowdofs, coldofs, counts))
     freeze_slab_exchange!(a, counts, alltoallv)
 end
 

@@ -115,12 +115,13 @@ class ExtendableSparseMatrix:
         self._ship(tid)
         self._h.insert_batch(I, J, V, flavour, tid)
 
-    def insert_elements(self, dofs, Aloc, flavour=capi.RAW, tid=0):
+    def insert_elements(self, dofs, Aloc, flavour=capi.RAW, tid=0, col_dofs=None):
         """Element loop (test/femtools.jl:45-72): for every element c, for jl, for il,
         rawupdateindex!(A, +, Aloc[c, jl, il], dofs[c, il], dofs[c, jl]) (or the `flavour`'s call).
-        dofs (ncells, k), 1-based; Aloc (ncells, k, k)."""
+        dofs (ncells, k), 1-based; Aloc (ncells, k, k).  With col_dofs (ncells, kc) the columns come from col_dofs:
+        rawupdateindex!(A, +, Aloc[c, jl, il], dofs[c, il], col_dofs[c, jl]), dofs (ncells, kr), Aloc (ncells, kc, kr)."""
         self._ship(tid)
-        self._h.insert_elements(dofs, Aloc, flavour, tid)
+        self._h.insert_elements(dofs, Aloc, flavour, tid, col_dofs=col_dofs)
 
     # -- flush!/sparse/nnz/reset!
     def flush(self):

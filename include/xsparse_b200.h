@@ -189,6 +189,17 @@ int32_t xsb_insert_triplets(xsb_matrix *h, int32_t tid, const xsb_triplet *T, in
  * grouping settings like the emitters: whole elements are grouped by column while they are staged. */
 int32_t xsb_insert_elements(xsb_matrix *h, int32_t tid, int32_t k, int64_t ncells, const void *dofs, const double *Aloc,
                             int32_t flavour);
+/* The element loop whose rows and columns come from different connectivities: coupling blocks of multi-field
+ * problems (test space != trial space, e.g. the pressure-velocity block of Stokes), rectangular operators (P0 x P1
+ * divergence, interpolation between meshes).  Julia's column-major arrays again:
+ *   rdofs kr x ncells, cdofs kc x ncells (idx_type, index_base), Aloc kr x kc x ncells Float64.
+ * Call p = kr*kc*c + kr*jl + il is (row = rdofs[il,c], col = cdofs[jl,c], v = Aloc[il,jl,c]) -- the order of
+ * xsb_insert_elements, whose calls are these with kr = kc = k and rdofs = cdofs = dofs.  The result equals
+ * xsb_insert_batch of the expanded stream bit for bit, as for the square loop.  1 <= kr, kc <= 64, else XSB_EINVAL.
+ * A row dof must lie in the m rows, a column dof in the n_global columns; one outside rejects the whole batch with
+ * XSB_EBOUNDS, and the message names the first offending element and whether a row or a column dof is at fault. */
+int32_t xsb_insert_elements_rect(xsb_matrix *h, int32_t tid, int32_t kr, int32_t kc, int64_t ncells,
+                                 const void *rdofs, const void *cdofs, const double *Aloc, int32_t flavour);
 
 /* Number of staged insertions (an upper bound of nnznew(A), genericextendable...:21). */
 int32_t xsb_pending(const xsb_matrix *h, int64_t *count);
@@ -296,6 +307,10 @@ int32_t xsb_freeze_pattern(xsb_matrix *h, const void *I, const void *J, int64_t 
 /* xsb_freeze_pattern for the stream xsb_insert_elements(h, ., k, ncells, dofs, ., .) would stage: the element
  * loop's positions from its connectivity alone; errors as xsb_freeze_pattern (XSB_EBOUNDS names the call). */
 int32_t xsb_freeze_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs);
+/* xsb_freeze_elements for the stream xsb_insert_elements_rect(h, ., kr, kc, ncells, rdofs, cdofs, ., .) would stage;
+ * xsb_reassemble_values[_zeroed](h, Aloc, kr*kc*ncells, mode) then takes Aloc unchanged. */
+int32_t xsb_freeze_elements_rect(xsb_matrix *h, int32_t kr, int32_t kc, int64_t ncells, const void *rdofs,
+                                 const void *cdofs);
 /* nzval[slot(k)] += V[k] for the frozen stream; deterministic mode folds every entry's values in stream order,
  * starting from the resident value (bit-exact with the in-place CSC-hit updates); fast mode is one atomic add
  * per insertion through the 4-byte entry -> nzval map. */
@@ -304,7 +319,7 @@ int32_t xsb_reassemble_values(xsb_matrix *h, const void *V, int64_t count, int32
  * entries start from +0.0 and nzval is written, never read (a Newton / time step re-assembles from zero). */
 int32_t xsb_reassemble_values_zeroed(xsb_matrix *h, const void *V, int64_t count, int32_t mode);
 int32_t xsb_unfreeze(xsb_matrix *h);
-/* On slab handles xsb_freeze_pattern / xsb_freeze_elements / xsb_get_values take slab-relative columns and the
+/* On slab handles xsb_freeze_pattern / xsb_freeze_elements[_rect] / xsb_get_values take slab-relative columns and the
  * rank's own entries only.  A distributed element loop is sharded by elements instead: the interface elements of
  * every rank write into columns a neighbour owns.  The calls below freeze such a stream -- GLOBAL positions, any
  * owner -- across the ranks (slab handles only; on a plain handle, or with insertions pending: XSB_ESTATE).
@@ -339,6 +354,9 @@ int32_t xsb_unfreeze(xsb_matrix *h);
  *   slab's pattern drops the map. */
 int32_t xsb_freeze_slab(xsb_matrix *h, const void *I, const void *J, int64_t count, int64_t *send_counts);
 int32_t xsb_freeze_slab_elements(xsb_matrix *h, int32_t k, int64_t ncells, const void *dofs, int64_t *send_counts);
+/* the first step of the slab freeze for the stream of xsb_insert_elements_rect; then _prepare and _finish as above */
+int32_t xsb_freeze_slab_elements_rect(xsb_matrix *h, int32_t kr, int32_t kc, int64_t ncells, const void *rdofs,
+                                      const void *cdofs, int64_t *send_counts);
 int32_t xsb_freeze_slab_prepare(xsb_matrix *h, void *send_positions, int64_t capacity);
 int32_t xsb_freeze_slab_finish(xsb_matrix *h, const void *recv_positions, const int64_t *recv_counts);
 int32_t xsb_frozen_slab_counts(const xsb_matrix *h, int64_t *send_counts, int64_t *recv_counts);
