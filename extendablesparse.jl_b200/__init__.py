@@ -5,10 +5,10 @@ through the repo-root shim `xsparse_b200` (import xsparse_b200).
 """
 from . import capi  # noqa: F401
 from .capi import (  # noqa: F401
-    ASSIGN, COMBINE_ADD, COMBINE_SEED, DETERMINISTIC, FAST, I32, I64, RAW, UPDATE, Handle, XsbBoundsError, XsbError,
+    ASSIGN, COMBINE_ADD, COMBINE_SEED, DETERMINISTIC, FAST, I32, I64, OP_ADD, OP_SUB, RAW, UPDATE, Handle, XsbBoundsError, XsbError,
     XsbIllegalError, XsbSizeError,
 )
 from .matrix import (  # noqa: F401
-    ExtendableSparseMatrix, MTExtendableSparseMatrix, fdrand, flush, nnz, pointblock, rawupdateindex, reset, sparse,
+    ExtendableSparseMatrix, MTExtendableSparseMatrix, dropzeros, fdrand, flush, nnz, pointblock, rawupdateindex, reset, sparse,
     updateindex,
 )

@@ -24,6 +24,7 @@ DETERMINISTIC, FAST = 0, 1
 COMBINE_SEED, COMBINE_ADD = 0, 1
 STRATEGY_AUTO, STRATEGY_FULLSORT = 0, 1
 GROUPING_AUTO, GROUPING_OFF, GROUPING_ON = 0, 1, 2
+OP_ADD, OP_SUB = 0, 1
 
 
 class XsbError(RuntimeError):
@@ -134,6 +135,8 @@ SIGNATURES = {
     "xsb_eliminate_dirichlet": (_i32, [_p, _p]),
     "xsb_pattern_hash": (_i32, [_p, C.POINTER(_u64)]),
     "xsb_pattern_equal": (_i32, [_p, _p, C.POINTER(_i32)]),
+    "xsb_add": (_i32, [_p, _p, _i32, C.POINTER(_p)]),
+    "xsb_dropzeros": (_i32, [_p, C.POINTER(_i64), C.POINTER(_i32)]),
     "xsb_pointblock": (_i32, [_p, _i32, C.POINTER(_p)]),
     "xsb_block_size": (_i32, [_p, C.POINTER(_i32)]),
     "xsb_fetch_blocks": (_i32, [_p, _p]),
@@ -577,6 +580,24 @@ class Handle:
         v = _i32(0)
         self._c(lib().xsb_pattern_equal(self._h, other._h, C.byref(v)))
         return bool(v.value)
+
+    def add(self, other: "Handle", op=OP_ADD) -> "Handle":
+        """A + B (op=OP_ADD) or A - B (op=OP_SUB) of two flushed matrices: SparseArrays' map(+/-, A, B) on the
+        device, entries equal to zero not stored.  Returns a new plain handle, a full assembly target."""
+        out = _p()
+        self._c(lib().xsb_add(self._h, other._h, int(op), C.byref(out)))
+        hc = Handle.__new__(Handle)
+        hc._h = out
+        hc.m, hc.n, hc.n_global, hc.col_begin = self.m, self.n, self.n, 0
+        hc.idx_type, hc.index_base, hc.n_tid, hc.device = self.idx_type, self.index_base, 1, self.device
+        hc.idx_dtype = self.idx_dtype
+        return hc
+
+    def dropzeros(self):
+        """dropzeros!(A) in place on the device: (nnz, pattern changed)."""
+        nnz, changed = _i64(0), _i32(0)
+        self._c(lib().xsb_dropzeros(self._h, C.byref(nnz), C.byref(changed)))
+        return nnz.value, bool(changed.value)
 
     def emit_fdrand(self, nx, ny=1, nz=1, seed=20240717, ones=False, flavour=UPDATE, tid=0, l_range=None):
         if l_range is None:

@@ -2835,6 +2835,130 @@ int32_t xsb_pattern_equal(xsb_matrix *a, xsb_matrix *b, int32_t *equal_out)
     });
 }
 
+namespace {
+// rowval / nzval of `nnz` entries in one store from the handle's cache, as the flush lays them out
+void *alloc_store(xsb_matrix *h, i64 nnz, size_t *bytes, void **rowval, double **nzval)
+{
+    const size_t rv_bytes = (h->isz() * (size_t)nnz + 15) & ~(size_t)15;
+    *bytes = rv_bytes + 8 * (size_t)nnz;
+    unsigned char *st = static_cast<unsigned char *>(h->dalloc(*bytes));
+    *rowval = st;
+    *nzval = reinterpret_cast<double *>(st + rv_bytes);
+    return st;
+}
+
+void check_result_nnz(const xsb_matrix *h, u64 nnz)
+{
+    REQUIRE(h->idx64 || nnz + (u64)h->base <= (u64)INT32_MAX, XSB_EINVAL,
+            "the result has " + std::to_string(nnz) + " entries, more than Int32 indices can address");
+}
+} // namespace
+
+int32_t xsb_add(xsb_matrix *a, xsb_matrix *b, int32_t op, xsb_matrix **out)
+{
+    if (out)
+        *out = nullptr;
+    if (!a || !b || !out)
+    {
+        g_err = "NULL argument";
+        return XSB_EINVAL;
+    }
+    // lock both handles in address order (two threads adding the same pair the other way round must not deadlock)
+    xsb_matrix *first = a < b ? a : b, *second = a < b ? b : a;
+    std::lock_guard<std::recursive_mutex> l1(first->mu), l2(second->mu);
+    return guard(a, [&]() -> int32_t {
+        REQUIRE(op == XSB_OP_ADD || op == XSB_OP_SUB, XSB_EINVAL, "op must be XSB_OP_ADD or XSB_OP_SUB");
+        REQUIRE(a->nranks == 0 && b->nranks == 0, XSB_ESTATE, "+ and - work on whole matrices, not on column slabs");
+        REQUIRE(a->block_size == 0 && b->block_size == 0, XSB_ESTATE, "+ and - do not take a pointblock result");
+        REQUIRE(a->pending() == 0 && b->pending() == 0, XSB_ESTATE, "flush! both matrices first");
+        REQUIRE(a->m == b->m && a->n == b->n, XSB_ESIZE,
+                "DimensionMismatch: dimensions must match: a has dims (" + std::to_string(a->m) + ", " +
+                    std::to_string(a->n) + "), b has dims (" + std::to_string(b->m) + ", " + std::to_string(b->n) + ")");
+        REQUIRE(a->idx64 == b->idx64 && a->base == b->base, XSB_EINVAL, "A and B must share index type and base");
+        REQUIRE(a->device == b->device, XSB_EINVAL, "A and B must live on the same device");
+        xsb_matrix *c = nullptr;
+        const int32_t rc = create_impl(a->m, a->n, 0, 0, nullptr, XSB_F64, a->idx64 ? XSB_I64 : XSB_I32, a->base, 1,
+                                       a->device, &c);
+        if (rc != XSB_OK)
+            throw ApiError(rc, "+/-: " + g_err);
+        try
+        {
+            a->sync(); // A and B are read on C's stream
+            b->sync();
+            const CscView va = a->view(), vb = b->view();
+            const int alg = op == XSB_OP_ADD ? kAlgAdd : kAlgSub;
+            void *ws = c->dalloc(merge_workspace_bytes(va.nnz, vb.nnz));
+            merge_count(c->stream, alg, va, &vb, a->n, a->idx64, a->base, ws, c->lc);
+            XSB_CUDA(cudaMemcpyAsync(c->h_scal, ws, sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+            c->sync();
+            const u64 nnz = c->h_scal[0];
+            check_result_nnz(c, nnz);
+            c->dfree(c->csc_store);
+            c->csc_store = alloc_store(c, (i64)nnz, &c->csc_store_bytes, &c->rowval, &c->nzval);
+            merge_write(c->stream, alg, va, &vb, a->n, a->idx64, a->base, ws, c->colptr, c->rowval, c->nzval, c->lc);
+            c->nnz = (i64)nnz;
+            c->dfree(ws);
+            c->sync();
+        }
+        catch (...)
+        {
+            xsb_destroy(c);
+            XSB_CUDA(cudaSetDevice(a->device));
+            throw;
+        }
+        *out = c;
+        return XSB_OK;
+    });
+}
+
+int32_t xsb_dropzeros(xsb_matrix *h, int64_t *nnz_out, int32_t *pattern_changed)
+{
+    return guard(h, [&]() -> int32_t {
+        REQUIRE(h, XSB_EINVAL, "NULL handle");
+        REQUIRE(h->pending() == 0, XSB_ESTATE, "staged insertions are pending: flush first");
+        REQUIRE(h->block_size == 0, XSB_ESTATE, "dropzeros! does not take a pointblock result");
+        const CscView v = h->view();
+        void *ws = h->dalloc(merge_workspace_bytes(v.nnz, 0));
+        try
+        {
+            merge_count(h->stream, kAlgKeep, v, nullptr, h->n, h->idx64, h->base, ws, h->lc);
+            XSB_CUDA(cudaMemcpyAsync(h->h_scal, ws, sizeof(u64), cudaMemcpyDeviceToHost, h->stream));
+            h->sync();
+            const i64 nnz = (i64)h->h_scal[0];
+            if (nnz != h->nnz)
+            {
+                void *colptr = h->dalloc(h->isz() * (size_t)(h->n + 1));
+                size_t bytes = 0;
+                void *rowval = nullptr;
+                double *nzval = nullptr;
+                void *store = alloc_store(h, nnz, &bytes, &rowval, &nzval);
+                merge_write(h->stream, kAlgKeep, v, nullptr, h->n, h->idx64, h->base, ws, colptr, rowval, nzval, h->lc);
+                h->dfree(h->colptr);
+                h->dfree(h->csc_store);
+                h->colptr = colptr;
+                h->csc_store = store;
+                h->csc_store_bytes = bytes;
+                h->rowval = rowval;
+                h->nzval = nzval;
+                h->drop_frozen(); // the frozen maps (plain or slab), a half-made slab freeze and the csr_map
+                h->sync();
+            }
+            h->dfree(ws);
+            if (nnz_out)
+                *nnz_out = nnz;
+            if (pattern_changed)
+                *pattern_changed = nnz != v.nnz ? 1 : 0;
+            h->nnz = nnz;
+        }
+        catch (...)
+        {
+            h->dfree(ws);
+            throw;
+        }
+        return XSB_OK;
+    });
+}
+
 int32_t xsb_pointblock(xsb_matrix *h, int32_t blocksize, xsb_matrix **out)
 {
     if (out)

@@ -354,6 +354,23 @@ void pattern_hash(cudaStream_t stream, const CscView &csc, i64 n, int idx64, u64
 void pattern_diff(cudaStream_t stream, const CscView &a, int idx64a, int basea, const CscView &b, int idx64b, int baseb,
                   i64 n, u64 *d_diff, LaunchCounter &lc);
 
+// ---- xsb_algebra.cu
+// C = A + B, A - B (SparseArrays' map(op, A, B): an entry of C is stored unless it == 0) and dropzeros! (kAlgKeep:
+// A's entries that are not +-0.0, bits unchanged; b unused).  Both CSCs sorted by (column, row), same n, index type
+// and base.  merge_count leaves C's nnz at ((u64 *)ws)[0]; merge_write then fills colptr_out (n + 1) and
+// rowval_out / nzval_out (that many entries) in the same index type and base.
+enum : int
+{
+    kAlgAdd = 0,
+    kAlgSub = 1,
+    kAlgKeep = 2
+};
+size_t merge_workspace_bytes(i64 nnz_a, i64 nnz_b);
+void merge_count(cudaStream_t stream, int op, const CscView &a, const CscView *b, i64 n, int idx64, int base, void *ws,
+                 LaunchCounter &lc);
+void merge_write(cudaStream_t stream, int op, const CscView &a, const CscView *b, i64 n, int idx64, int base,
+                 const void *ws, void *colptr_out, void *rowval_out, double *nzval_out, LaunchCounter &lc);
+
 // ---- xsb_mul.cu
 size_t csr_map_bytes(i64 m, i64 nnz);
 void build_csr_map(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, Rec *tags_a, Rec *tags_b,

@@ -529,6 +529,19 @@ class DistExtendableSparseMatrix:
             # from being handed to new work on other streams before they are done
             V.record_stream(self._lib_stream)
 
+    def dropzeros(self):
+        """Collective dropzeros!: every rank removes the stored +-0.0 of its own slab (no entries move between ranks),
+        then one all-gather refreshes nnz_offset / nnz_global and whether any rank's pattern changed; if one did,
+        every rank unfreezes, as after a flush.  Returns (local nnz, pattern changed on any rank)."""
+        self._resolve_offsets()
+        nnz, changed = self.h.dropzeros()
+        mine = torch.tensor([nnz, int(changed)], dtype=torch.int64, device=self.device)
+        allv = torch.empty(2 * self.world, dtype=torch.int64, device=self.device)
+        work = dist.all_gather_into_tensor(allv, mine, group=self.group, async_op=True)
+        self._offsets_pending = (work, allv, mine)
+        self._resolve_offsets()
+        return nnz, self._changed_any
+
     @property
     def nnz_offset(self) -> int:
         """Entries owned by lower ranks: the shift from the slab's colptr to the global one."""

@@ -34,6 +34,7 @@ const XSB_F64, XSB_I32, XSB_I64 = Int32(0), Int32(0), Int32(1)
 const XSB_UPDATE, XSB_RAW, XSB_ASSIGN = Int32(0), Int32(1), Int32(2)
 const XSB_DETERMINISTIC, XSB_FAST = Int32(0), Int32(1)
 const XSB_COMBINE_SEED, XSB_COMBINE_ADD = Int32(0), Int32(1)
+const XSB_OP_ADD, XSB_OP_SUB = Int32(0), Int32(1)
 
 const CHUNK = 1 << 16
 
@@ -206,6 +207,13 @@ mutable struct B200Assembler{Tv, Ti <: Integer}
                         y.handle = C_NULL), x)
         x
     end
+    # takes ownership of a plain handle the library returned (the result of + and -)
+    function B200Assembler{Tv, Ti}(m, n, handle::Ptr{Cvoid}) where {Tv, Ti}
+        x = new{Tv, Ti}(m, n, handle, 0, 0, nothing)
+        finalizer(y -> (y.handle == C_NULL || ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), y.handle);
+                        y.handle = C_NULL), x)
+        x
+    end
 end
 
 function set_csc!(a::B200Assembler{Tv, Ti}, csc::SparseMatrixCSC{Tv, Ti}) where {Tv, Ti}
@@ -316,6 +324,29 @@ function pointblock(a::B200Assembler{Tv, Ti}, blocksize::Integer) where {Tv, Ti}
     finally
         ccall((:xsb_destroy, libxsb), Int32, (Ptr{Cvoid},), hb[])
     end
+end
+
+"""
+    a + b, a - b -> B200Assembler
+
+SparseArrays' `+` / `-` of the two flushed matrices (src/matrix/abstractextendablesparsematrixcsc.jl: flush
+both, then `map(+/-, A, B)`), computed on the device: entries equal to zero are not stored.  The result is a
+new assembler on `a`'s device with its own handle: insert!, fetch!, freeze! and mul work on it.
+"""
+function add_sub(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}, op) where {Tv, Ti}
+    hc = Ref{Ptr{Cvoid}}(C_NULL)
+    check(a.handle, ccall((:xsb_add, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Int32, Ref{Ptr{Cvoid}}),
+                          a.handle, b.handle, op, hc))
+    B200Assembler{Tv, Ti}(a.m, a.n, hc[])
+end
+Base.:+(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}) where {Tv, Ti} = add_sub(a, b, XSB_OP_ADD)
+Base.:-(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}) where {Tv, Ti} = add_sub(a, b, XSB_OP_SUB)
+
+"dropzeros!(a): the stored +-0.0 of the flushed matrix removed in place on the device (a slab: its own columns)"
+function SparseArrays.dropzeros!(a::B200Assembler)
+    nnz = Ref{Int64}(0); changed = Ref{Int32}(0)
+    check(a.handle, ccall((:xsb_dropzeros, libxsb), Int32, (Ptr{Cvoid}, Ref{Int64}, Ref{Int32}), a.handle, nnz, changed))
+    a
 end
 
 # the drop-in aliases, mirroring src/ExtendableSparse.jl:35-39

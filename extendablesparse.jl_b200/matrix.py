@@ -8,6 +8,7 @@ mutators is dropped):
     rawupdateindex(A, op, v, i, j[, tid])             extendable.jl:181-197, genericmt...:87-99
     A[i, j] = v ; A[i, j]                             extendable.jl:205-238
     pointblock(A, blocksize)                          extendable.jl:292-318
+    A + B ; A - B ; dropzeros(A)                      abstractextendablesparsematrixcsc.jl
     flush(A) ; sparse(A) ; nnz(A) ; reset(A)          extendable.jl:248-272
     MTExtendableSparseMatrix(m, n, nparts)            src/ExtendableSparse.jl:35-39, genericmt...:1-114
 
@@ -167,13 +168,31 @@ class ExtendableSparseMatrix:
         self._h.zero_values()
 
     def dropzeros(self):
-        """dropzeros!(A): stdlib pass over the flushed CSC (abstractextendable...:110), done on the host."""
-        cp, rv, nz = self.csc()
-        keep = nz != 0
-        cols = np.repeat(np.arange(self.n), np.diff(cp))
-        cp2 = np.concatenate([[1], 1 + np.cumsum(np.bincount(cols[keep], minlength=self.n))]).astype(np.int64)
-        self._h.set_csc(cp2, np.ascontiguousarray(rv[keep]), np.ascontiguousarray(nz[keep]))
+        """dropzeros!(A) (abstractextendablesparsematrixcsc.jl:110): the stored +-0.0 removed on the device, in place."""
+        self.flush()
+        _, changed = self._h.dropzeros()
+        self.pattern_changes += int(changed)
         return self
+
+    def _combine(self, other, op):
+        if not isinstance(other, ExtendableSparseMatrix):
+            return NotImplemented
+        self.flush()
+        other.flush()
+        hc = self._h.add(other._h, op)
+        C = ExtendableSparseMatrix.__new__(ExtendableSparseMatrix)
+        C._h, C.m, C.n, C.mode = hc, self.m, self.n, self.mode
+        C._buf = [_HostBuffer()]
+        C.pattern_changes = 0
+        return C
+
+    def __add__(self, other):
+        """A + B (abstractextendablesparsematrixcsc.jl: flush both, then SparseArrays' +): a new matrix."""
+        return self._combine(other, capi.OP_ADD)
+
+    def __sub__(self, other):
+        """A - B: a new matrix."""
+        return self._combine(other, capi.OP_SUB)
 
     def mark_dirichlet(self, penalty=1.0e20):
         self.flush()
@@ -229,6 +248,10 @@ def rawupdateindex(A, op, v, i, j, *tid):
 
 def pointblock(A, blocksize):
     return A.pointblock(blocksize)
+
+
+def dropzeros(A):
+    return A.dropzeros()
 
 
 def flush(A):

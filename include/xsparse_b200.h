@@ -388,6 +388,33 @@ int32_t xsb_pattern_hash(xsb_matrix *h, uint64_t *hash_out);
  * comparing fingerprints. */
 int32_t xsb_pattern_equal(xsb_matrix *a, xsb_matrix *b, int32_t *equal_out);
 
+/* ------------------------------------------------------------------ */
+/* pattern-changing operations on flushed matrices                     */
+/* ------------------------------------------------------------------ */
+/* A + B and A - B: src/matrix/abstractextendablesparsematrixcsc.jl (flush both, then SparseArrays'
+ * map(+/-, A, B)).  Column by column over the sorted rows of both: a row in both gives f(a, b), a row
+ * in A only f(a, 0.0), a row in B only f(0.0, b), and the result is stored unless it == 0 (so +-0.0 are
+ * dropped, NaN is kept, explicit zeros of the inputs disappear).  Every value is one IEEE add or
+ * subtract; NaN results carry x86-64's bits (the first NaN operand, quieted; Inf - Inf is the negative
+ * default NaN), as the reference computes them on its hosts.
+ * Returns a NEW plain handle *out = C with one partition and A's device, index type and base: a full
+ * assembly target (insert, flush, freeze, mul).  Its CSC is built on the device.  The caller destroys it.
+ * a == b is allowed (A - A is empty).  Pending inserts on either, a slab handle or a pointblock result:
+ * XSB_ESTATE; different sizes: XSB_ESIZE (DimensionMismatch); different index type, base or device, an
+ * unknown op, or a result nnz the index type cannot hold: XSB_EINVAL.  On any error *out is NULL and A
+ * and B are unchanged. */
+#define XSB_OP_ADD 0
+#define XSB_OP_SUB 1
+int32_t xsb_add(xsb_matrix *a, xsb_matrix *b, int32_t op, xsb_matrix **out);
+
+/* dropzeros!(A): src/matrix/abstractextendablesparsematrixcsc.jl:110 (fkeep! with !iszero): removes
+ * the stored +-0.0 in place, order and the other values' bits unchanged.  *pattern_changed = 1 exactly
+ * when an entry was dropped; only then are the frozen map (plain or slab), the row-major view of xsb_mul
+ * and a half-made slab freeze dropped, so a dropzeros that drops nothing leaves a frozen handle frozen.
+ * Plain and slab handles (each rank filters its own slab, no communication).  Pending inserts or a
+ * pointblock result: XSB_ESTATE. */
+int32_t xsb_dropzeros(xsb_matrix *h, int64_t *nnz_out, int32_t *pattern_changed);
+
 /* pointblock(A, blocksize): src/matrix/extendable.jl:292-318 (feeds PointBlockILUZeroPreconditioner,
  * src/factorizations/iluzero.jl:61-71).  Returns a NEW handle *out holding the nblock x nblock block
  * matrix Ab, nblock = n / blocksize: its CSC pattern is read with xsb_nnz / xsb_fetch_csc, its values
