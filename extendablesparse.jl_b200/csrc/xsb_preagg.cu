@@ -8,7 +8,7 @@
 // elements (P1-FEM: 120 insertions per cube hit 46 entries), so 2.5-4x fewer records leave the
 // kernel.  The partial sums are then grouped and folded per column like any other records; the
 // value of an entry becomes a sum of partial sums instead of the left fold in insertion order
-// (<= 1e-14 relative, include/xsparse_b200.h XSB_FAST) and the pattern is unchanged:
+// (within gamma(N-1) * sum|x| of the exact sum, include/xsparse_b200.h XSB_FAST) and the pattern is unchanged:
 //   rawupdateindex! always creates, updateindex! creates unless every value it saw was zero
 //   (sparsematrixlnk.jl:212,223,239) -- a window whose records create nothing emits nothing.
 // Not used when A[i,j] = v records are staged (assignment does not commute).

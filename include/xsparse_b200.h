@@ -74,7 +74,11 @@ extern "C" {
 
 /* summation modes */
 #define XSB_DETERMINISTIC 0 /* left fold in insertion order: bit-exact with the reference   */
-#define XSB_FAST 1          /* summation order free: <= 1e-14 relative (f64), pattern bit-exact.  xsb_flush: duplicates
+#define XSB_FAST 1          /* summation order free, pattern bit-exact.  Each entry is within gamma(N-1) * sum|x| of
+                               the exact sum of its N contributions x (resident value included), gamma(k) = k u /
+                               (1 - k u), u = 2^-53; exact (and so equal to XSB_DETERMINISTIC up to the sign of a zero
+                               result) whenever every partial sum is representable, e.g. integers or one common power
+                               of two.  No relative bound holds once contributions cancel.  xsb_flush: duplicates
                                may be accumulated per chunk of the stream before the per-column merge (off unless
                                xsb_set_preaggregation; otherwise the exact merge runs); xsb_reassemble_values: one
                                atomic add per insertion instead of the ordered per-entry fold */
@@ -488,7 +492,10 @@ int32_t xsb_set_grouping(xsb_matrix *h, int32_t grouping);
 /* XSB_FAST flushes only (ignored otherwise, and when A[i,j]=v records are staged): fold the staged
  * stream inside windows of 512 insertions first -- the reference's accumulate-on-insert
  * (src/matrix/sparsematrixlnk.jl:210-253) -- so that fewer records are grouped.  Pattern unchanged,
- * values <= 1e-14 relative, summation order not reproducible from run to run.  Off by default:
+ * each value within gamma(N-1) * sum|x| of the exact sum of its N contributions (XSB_FAST), summation
+ * order not reproducible from run to run.  Streams of fewer than 4096 staged records are not folded;
+ * a handle stops trying after two flushes in a row whose windows kept more than 3/4 of the records,
+ * until xsb_set_preaggregation is called again.  Off by default:
  * on B200 it only pays when the windows shrink the stream more than about 3x (DESIGN.md section 5). */
 int32_t xsb_set_preaggregation(xsb_matrix *h, int32_t enable);
 /* Grouping at insertion (default on): the kernels behind xsb_insert_batch / xsb_insert_triplets / xsb_emit_* bring
