@@ -9,8 +9,8 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libxsparse_b200.so")
-SOURCES = ["xsb_sort.cu", "xsb_flush.cu", "xsb_colfold.cu", "xsb_group.cu", "xsb_runs.cu", "xsb_preagg.cu", "xsb_route.cu", "xsb_insert.cu", "xsb_values.cu", "xsb_mul.cu", "xsb_algebra.cu", "xsb_api.cu"]
-HEADERS = ["xsb_common.cuh", "xsb_internal.h", "xsb_fold.cuh", "xsb_group_count.cuh", "xsb_chunk.cuh", os.path.join("..", "..", "include", "xsparse_b200.h")]
+SOURCES = ["xsb_sort.cu", "xsb_flush.cu", "xsb_colfold.cu", "xsb_group.cu", "xsb_runs.cu", "xsb_preagg.cu", "xsb_route.cu", "xsb_insert.cu", "xsb_values.cu", "xsb_mul.cu", "xsb_algebra.cu", "xsb_spgemm.cu", "xsb_api.cu"]
+HEADERS = ["xsb_common.cuh", "xsb_internal.h", "xsb_fold.cuh", "xsb_group_count.cuh", "xsb_chunk.cuh", "xsb_x86nan.cuh", os.path.join("..", "..", "include", "xsparse_b200.h")]
 
 NVCC_FLAGS = [
     "-O3",

@@ -136,6 +136,7 @@ SIGNATURES = {
     "xsb_pattern_hash": (_i32, [_p, C.POINTER(_u64)]),
     "xsb_pattern_equal": (_i32, [_p, _p, C.POINTER(_i32)]),
     "xsb_add": (_i32, [_p, _p, _i32, C.POINTER(_p)]),
+    "xsb_matmul": (_i32, [_p, _p, C.POINTER(_p)]),
     "xsb_dropzeros": (_i32, [_p, C.POINTER(_i64), C.POINTER(_i32)]),
     "xsb_pointblock": (_i32, [_p, _i32, C.POINTER(_p)]),
     "xsb_block_size": (_i32, [_p, C.POINTER(_i32)]),
@@ -589,6 +590,19 @@ class Handle:
         hc = Handle.__new__(Handle)
         hc._h = out
         hc.m, hc.n, hc.n_global, hc.col_begin = self.m, self.n, self.n, 0
+        hc.idx_type, hc.index_base, hc.n_tid, hc.device = self.idx_type, self.index_base, 1, self.device
+        hc.idx_dtype = self.idx_dtype
+        return hc
+
+    def matmul(self, other: "Handle") -> "Handle":
+        """A * B of two flushed matrices: SparseArrays' spmatmul on the device (structural pattern, each entry the
+        left fold in ascending k of the products).  Returns a new plain self.m x other.n handle, a full assembly
+        target."""
+        out = _p()
+        self._c(lib().xsb_matmul(self._h, other._h, C.byref(out)))
+        hc = Handle.__new__(Handle)
+        hc._h = out
+        hc.m, hc.n, hc.n_global, hc.col_begin = self.m, other.n, other.n, 0
         hc.idx_type, hc.index_base, hc.n_tid, hc.device = self.idx_type, self.index_base, 1, self.device
         hc.idx_dtype = self.idx_dtype
         return hc

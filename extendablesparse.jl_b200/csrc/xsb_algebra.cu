@@ -10,6 +10,7 @@
 // and emits nothing.  Three passes: count (kept entries per block), scan (block offsets), write (rowval, nzval
 // and the colptr of every non-empty column); a last pass fills the colptr of the empty columns.
 #include "xsb_internal.h"
+#include "xsb_x86nan.cuh"
 
 namespace xsb {
 namespace {
@@ -17,24 +18,6 @@ namespace {
 constexpr int kAlgThreads = 256;
 constexpr int kAlgItems = 8;
 constexpr i64 kAlgTile = (i64)kAlgThreads * kAlgItems;
-
-// One IEEE add or subtract, NaN results with the bits x86-64 gives them (the first NaN operand, quieted;
-// Inf - Inf is the negative default NaN): nzval is compared bit for bit with the reference's host arithmetic.
-__device__ __forceinline__ double quiet(double x)
-{
-    return __longlong_as_double(__double_as_longlong(x) | 0x0008000000000000ll);
-}
-template <int OP> __device__ __forceinline__ double apply(double a, double b)
-{
-    const double r = OP == kAlgSub ? __dsub_rn(a, b) : __dadd_rn(a, b);
-    if (r == r)
-        return r;
-    if (a != a)
-        return quiet(a);
-    if (b != b)
-        return quiet(b);
-    return __longlong_as_double((long long)0xfff8000000000000ull);
-}
 
 template <typename Ti, int OP> struct Operands
 {

@@ -2911,6 +2911,81 @@ int32_t xsb_add(xsb_matrix *a, xsb_matrix *b, int32_t op, xsb_matrix **out)
     });
 }
 
+int32_t xsb_matmul(xsb_matrix *a, xsb_matrix *b, xsb_matrix **out)
+{
+    if (out)
+        *out = nullptr;
+    if (!a || !b || !out)
+    {
+        g_err = "NULL argument";
+        return XSB_EINVAL;
+    }
+    // lock both handles in address order (two threads computing A * B and B * A at once must not deadlock)
+    xsb_matrix *first = a < b ? a : b, *second = a < b ? b : a;
+    std::lock_guard<std::recursive_mutex> l1(first->mu), l2(second->mu);
+    return guard(a, [&]() -> int32_t {
+        REQUIRE(a->nranks == 0 && b->nranks == 0, XSB_ESTATE, "* works on whole matrices, not on column slabs");
+        REQUIRE(a->block_size == 0 && b->block_size == 0, XSB_ESTATE, "* does not take a pointblock result");
+        REQUIRE(a->pending() == 0 && b->pending() == 0, XSB_ESTATE, "flush! both matrices first");
+        REQUIRE(a->n == b->m, XSB_ESIZE,
+                "DimensionMismatch: matrix A has dimensions (" + std::to_string(a->m) + ", " + std::to_string(a->n) +
+                    "), matrix B has dimensions (" + std::to_string(b->m) + ", " + std::to_string(b->n) + ")");
+        REQUIRE(a->idx64 == b->idx64 && a->base == b->base, XSB_EINVAL, "A and B must share index type and base");
+        REQUIRE(a->device == b->device, XSB_EINVAL, "A and B must live on the same device");
+        REQUIRE(a->m < (1ll << 32) - 1 && b->n < (1ll << 32), XSB_EINVAL,
+                "A * B needs A to have fewer than 2^32 - 1 rows and B fewer than 2^32 columns");
+        xsb_matrix *c = nullptr;
+        const int32_t rc = create_impl(a->m, b->n, 0, 0, nullptr, XSB_F64, a->idx64 ? XSB_I64 : XSB_I32, a->base, 1,
+                                       a->device, &c);
+        if (rc != XSB_OK)
+            throw ApiError(rc, "*: " + g_err);
+        try
+        {
+            a->sync(); // A and B are read on C's stream
+            b->sync();
+            Spgemm g{};
+            g.a = a->view();
+            g.b = b->view();
+            g.m = a->m;
+            g.n = b->n;
+            g.idx64 = a->idx64;
+            g.base = a->base;
+            g.ws = c->dalloc(spgemm_workspace_bytes(g.n));
+            spgemm_classify(c->stream, g, c->lc);
+            XSB_CUDA(cudaMemcpyAsync(c->h_scal, g.ws, 5 * sizeof(u64), cudaMemcpyDeviceToHost, c->stream));
+            c->sync();
+            std::copy(c->h_scal, c->h_scal + 4, g.bins);
+            g.tiles = c->h_scal[4];
+            REQUIRE(g.tiles < (1ull << 32), XSB_EINVAL, "A * B: more than 2^32 row tiles");
+            g.tile_ws = c->dalloc(spgemm_tiles_bytes(g.tiles));
+            spgemm_count(c->stream, g, c->colptr, c->lc);
+            XSB_CUDA(cudaMemcpyAsync(c->h_scal, static_cast<u64 *>(g.ws) + 5, sizeof(u64), cudaMemcpyDeviceToHost,
+                                     c->stream));
+            XSB_CUDA(cudaMemcpyAsync(c->h_scal + 1, static_cast<u64 *>(g.ws) + 12, 4 * sizeof(u64),
+                                     cudaMemcpyDeviceToHost, c->stream));
+            c->sync();
+            const u64 nnz = c->h_scal[0];
+            std::copy(c->h_scal + 1, c->h_scal + 5, g.umax);
+            check_result_nnz(c, nnz);
+            c->dfree(c->csc_store);
+            c->csc_store = alloc_store(c, (i64)nnz, &c->csc_store_bytes, &c->rowval, &c->nzval);
+            spgemm_write(c->stream, g, c->colptr, c->rowval, c->nzval, c->lc);
+            c->nnz = (i64)nnz;
+            c->dfree(g.tile_ws);
+            c->dfree(g.ws);
+            c->sync();
+        }
+        catch (...)
+        {
+            xsb_destroy(c);
+            XSB_CUDA(cudaSetDevice(a->device));
+            throw;
+        }
+        *out = c;
+        return XSB_OK;
+    });
+}
+
 int32_t xsb_dropzeros(xsb_matrix *h, int64_t *nnz_out, int32_t *pattern_changed)
 {
     return guard(h, [&]() -> int32_t {

@@ -371,6 +371,31 @@ void merge_count(cudaStream_t stream, int op, const CscView &a, const CscView *b
 void merge_write(cudaStream_t stream, int op, const CscView &a, const CscView *b, i64 n, int idx64, int base,
                  const void *ws, void *colptr_out, void *rowval_out, double *nzval_out, LaunchCounter &lc);
 
+// ---- xsb_spgemm.cu
+// C = A * B (SparseArrays' spmatmul): the structural pattern, and per entry the left fold in ascending k of the
+// separately rounded products a * b, the first one assigned.  A is m x k, B k x n, both sorted by (column, row),
+// same index type and base; m < 2^32 - 1, n < 2^32.  spgemm_classify leaves at ((u64 *)ws)[0..5) the columns of
+// the three warp-table bins and of the tiled bin, then the number of row tiles; the caller copies them into
+// bins / tiles and allocates tile_ws.  spgemm_count fills colptr_out (n + 1) and leaves nnz(C) at
+// ((u64 *)ws)[5] and at ((u64 *)ws)[12..16) the largest u(j) per bin that spgemm_write sizes its tables by (the
+// caller copies them into umax); spgemm_write then fills rowval_out / nzval_out (that many entries).
+struct Spgemm
+{
+    CscView a, b;
+    i64 m, n;
+    int idx64, base;
+    void *ws;      // spgemm_workspace_bytes(n)
+    void *tile_ws; // spgemm_tiles_bytes(tiles)
+    u64 bins[4], tiles;
+    u64 umax[4];
+};
+size_t spgemm_workspace_bytes(i64 n);
+size_t spgemm_tiles_bytes(u64 tiles);
+void spgemm_classify(cudaStream_t stream, const Spgemm &g, LaunchCounter &lc);
+void spgemm_count(cudaStream_t stream, const Spgemm &g, void *colptr_out, LaunchCounter &lc);
+void spgemm_write(cudaStream_t stream, const Spgemm &g, const void *colptr, void *rowval_out, double *nzval_out,
+                  LaunchCounter &lc);
+
 // ---- xsb_mul.cu
 size_t csr_map_bytes(i64 m, i64 nnz);
 void build_csr_map(cudaStream_t stream, const CscView &csc, i64 m, i64 n, int idx64, int base, Rec *tags_a, Rec *tags_b,

@@ -342,6 +342,20 @@ end
 Base.:+(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}) where {Tv, Ti} = add_sub(a, b, XSB_OP_ADD)
 Base.:-(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}) where {Tv, Ti} = add_sub(a, b, XSB_OP_SUB)
 
+"""
+    a * b -> B200Assembler
+
+SparseArrays' `*` of the two flushed matrices (src/matrix/abstractextendablesparsematrixcsc.jl: flush both, then
+`spmatmul`), computed on the device: the structural pattern, each entry the left fold in ascending k of the products.
+The result is a new `a.m × b.n` assembler on `a`'s device with its own handle: insert!, fetch!, freeze! and mul work
+on it.
+"""
+function Base.:*(a::B200Assembler{Tv, Ti}, b::B200Assembler{Tv, Ti}) where {Tv, Ti}
+    hc = Ref{Ptr{Cvoid}}(C_NULL)
+    check(a.handle, ccall((:xsb_matmul, libxsb), Int32, (Ptr{Cvoid}, Ptr{Cvoid}, Ref{Ptr{Cvoid}}), a.handle, b.handle, hc))
+    B200Assembler{Tv, Ti}(a.m, b.n, hc[])
+end
+
 "dropzeros!(a): the stored +-0.0 of the flushed matrix removed in place on the device (a slab: its own columns)"
 function SparseArrays.dropzeros!(a::B200Assembler)
     nnz = Ref{Int64}(0); changed = Ref{Int32}(0)

@@ -9,6 +9,7 @@ mutators is dropped):
     A[i, j] = v ; A[i, j]                             extendable.jl:205-238
     pointblock(A, blocksize)                          extendable.jl:292-318
     A + B ; A - B ; dropzeros(A)                      abstractextendablesparsematrixcsc.jl
+    A @ B (A * B of two matrices) ; A @ x             abstractextendablesparsematrixcsc.jl
     flush(A) ; sparse(A) ; nnz(A) ; reset(A)          extendable.jl:248-272
     MTExtendableSparseMatrix(m, n, nparts)            src/ExtendableSparse.jl:35-39, genericmt...:1-114
 
@@ -150,6 +151,12 @@ class ExtendableSparseMatrix:
         return self._h.mul(np.ascontiguousarray(x, np.float64))
 
     def __matmul__(self, x):
+        """A @ B with a matrix B: flush both, then SparseArrays' A * B on the device, a new matrix.  A @ x with a
+        vector: mul."""
+        if isinstance(x, ExtendableSparseMatrix):
+            self.flush()
+            x.flush()
+            return self._result(self._h.matmul(x._h), self.m, x.n)
         return self.mul(x)
 
     @property
@@ -179,9 +186,12 @@ class ExtendableSparseMatrix:
             return NotImplemented
         self.flush()
         other.flush()
-        hc = self._h.add(other._h, op)
+        return self._result(self._h.add(other._h, op), self.m, self.n)
+
+    def _result(self, hc, m, n):
+        """A new one-partition matrix around the handle of an A + B, A - B or A * B."""
         C = ExtendableSparseMatrix.__new__(ExtendableSparseMatrix)
-        C._h, C.m, C.n, C.mode = hc, self.m, self.n, self.mode
+        C._h, C.m, C.n, C.mode = hc, m, n, self.mode
         C._buf = [_HostBuffer()]
         C.pattern_changes = 0
         return C

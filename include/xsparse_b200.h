@@ -411,6 +411,21 @@ int32_t xsb_pattern_equal(xsb_matrix *a, xsb_matrix *b, int32_t *equal_out);
 #define XSB_OP_SUB 1
 int32_t xsb_add(xsb_matrix *a, xsb_matrix *b, int32_t op, xsb_matrix **out);
 
+/* A * B: src/matrix/abstractextendablesparsematrixcsc.jl (flush both, then SparseArrays' spmatmul).  For
+ * every column j of B, its entries (k, b) in stored order and, for each, A[:, k]'s entries (i, a) give the
+ * products a * b (A's value first); the first product of row i is assigned, every later one added
+ * (acc = acc + p).  So C[:, j] stores the union of the rows of A[:, k] over the k stored in B[:, j] (explicit
+ * zeros of A or B still create entries, nothing is dropped), and each value is the left fold in ascending k of
+ * separately rounded products (a first product of -0.0 stays -0.0).  NaN results carry x86-64's bits, as for
+ * xsb_add (0 * Inf and Inf - Inf give the negative default NaN).  C is A.m x B.n.
+ * Returns a NEW plain handle *out = C with one partition and A's device, index type and base: a full
+ * assembly target (insert, flush, freeze, mul, add).  Its CSC is built on the device; the products are never
+ * stored.  The caller destroys it.  a == b is allowed (A * A).  Pending inserts on either, a slab handle or a
+ * pointblock result: XSB_ESTATE; A.n != B.m: XSB_ESIZE (DimensionMismatch); different index type, base or
+ * device, A with 2^32 - 1 rows or more, B with 2^32 columns or more, or a result nnz the index type cannot
+ * hold: XSB_EINVAL.  On any error *out is NULL and A and B are unchanged. */
+int32_t xsb_matmul(xsb_matrix *a, xsb_matrix *b, xsb_matrix **out);
+
 /* dropzeros!(A): src/matrix/abstractextendablesparsematrixcsc.jl:110 (fkeep! with !iszero): removes
  * the stored +-0.0 in place, order and the other values' bits unchanged.  *pattern_changed = 1 exactly
  * when an entry was dropped; only then are the frozen map (plain or slab), the row-major view of xsb_mul
