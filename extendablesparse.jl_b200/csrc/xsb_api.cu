@@ -1,6 +1,7 @@
 // xsb_api.cu -- the C ABI of libxsparse_b200 (include/xsparse_b200.h): handle, device
 // memory, staging buffers and the flush pipeline that strings the kernels together.
 #include "../../include/xsparse_b200.h"
+#include "xsb_fold.cuh"
 #include "xsb_internal.h"
 
 #include <chrono>
@@ -715,7 +716,7 @@ bool runs_flush(xsb_matrix *h, StageTimer *tp, int64_t *nnz_out)
     double *new_nzval = reinterpret_cast<double *>(store + rv_bytes);
     const u64 avg = (u64)count / (u64)std::max<i64>(1, h->n);
     const u32 maxlen = (u32)std::max<u64>(1024, 8 * avg);
-    int level = h->fold_hint ? runs_level_for(h->fold_hint) : (nnz_old > 0 ? runs_level_for((u32)std::min<i64>(64, 2 * nnz_old / std::max<i64>(1, h->n) + 4))
+    int level = h->fold_hint ? fold_level_for(h->fold_hint) : (nnz_old > 0 ? fold_level_for((u32)std::min<i64>(64, 2 * nnz_old / std::max<i64>(1, h->n) + 4))
                                                                            : (avg < 14 ? 0 : (avg < 40 ? 2 : 3)));
     i64 nnz_new = -1;
     bool ok = false;
@@ -739,7 +740,7 @@ bool runs_flush(xsb_matrix *h, StageTimer *tp, int64_t *nnz_out)
         }
         if ((redo & 6u) || level >= 3)
             break; // a very long column, or one too rich for the largest table
-        level = std::max(level + 1, maxd > 0 ? runs_level_for(maxd) : 0); // the next table shape
+        level = std::max(level + 1, maxd > 0 ? fold_level_for(maxd) : 0); // the next table shape
     }
     if (tp)
         tp->end(s, &StageTimes::fold);

@@ -273,14 +273,14 @@ template <> struct WarpSpace<true>
 
 template <> struct WarpSpace<false>
 {
-    ColFold st[CF_H];
+    RunFold st[CF_H];
     double val[CF_PIECE];
     u32 meta[CF_PIECE];
     u32 key[CF_H];
     u32 ccnt[32];
     unsigned short cnt[CF_H];
     unsigned short cand[CF_H];
-    __device__ __forceinline__ void init_slot(u32 s) { st[s] = ColFold(); }
+    __device__ __forceinline__ void init_slot(u32 s) { st[s] = RunFold(); }
     __device__ __forceinline__ void note(u32, bool, u32, bool) {}
     __device__ __forceinline__ void put(u32 pos, double v, u32 m)
     {
@@ -291,7 +291,7 @@ template <> struct WarpSpace<false>
     {
         if (o0 < o1)
         {
-            ColFold f = st[s];
+            RunFold f = st[s];
             for (; o0 < o1; ++o0)
             {
                 const u32 m = meta[o0];
@@ -302,7 +302,7 @@ template <> struct WarpSpace<false>
     }
     __device__ __forceinline__ bool settle(u32 s)
     {
-        ColFold f = st[s];
+        RunFold f = st[s];
         f.finish();
         st[s].acc = f.acc;
         return f.exists;
@@ -609,109 +609,44 @@ colfold_kernel(const Rec *__restrict__ sorted, KeyLayout L, int combine, u32 chu
 // ------------------------------------------------------------------------
 // one THREAD per column (plain += streams: one partition, no assign flavour, old values seed)
 // ------------------------------------------------------------------------
-// Thread k walks the records of non-empty column k in stream order.  Its accumulators live in
-// shared memory, in a private open-addressing table laid out slot-major ([slot][lane]) so that a
-// lane only ever touches its own bank: no conflicts whatever the slots are.  A table slot holds
-// (row << HBITS | accumulator index); the accumulators are numbered in order of first appearance.
-// Every record is one probe and one add: the exact left fold of the reference's
-// accumulate-on-insert (src/matrix/sparsematrixlnk.jl:210-253) with the list walk replaced by the
-// hash probe.  At the end the slots of the existing entries are insertion-sorted by row in place
-// (src/matrix/sparsematrixlnk.jl:339) and the entries parked at the column's offset.
+// Thread k walks the records of non-empty column k in stream order and folds them through ThreadFold
+// (xsb_fold.cuh), the fold of the grouped-chunk merge; the existing entries are then sorted by row
+// (src/matrix/sparsematrixlnk.jl:339) and parked at the column's offset or written to the new CSC.
 //
-// Three table sizes (16/12, 32/24, 64/48 slots/accumulators) trade occupancy against capacity: a
-// column with more distinct rows than the table takes is appended to `next` (the next size, or the
-// warp-per-column kernel); columns longer than maxlen go straight to `longlist` (warp kernel).
+// The table shapes trade occupancy against capacity: a column with more distinct rows than the table takes
+// is appended to `next` (the next shape, or the warp-per-column kernel); columns longer than maxlen go
+// straight to `longlist` (warp kernel).
 constexpr int CT_WARPS = 4;
 #ifndef XSB_CT_U
 #define XSB_CT_U 2
 #endif
 constexpr int CT_U = XSB_CT_U; // 32-byte record pairs per step (the next step is prefetched)
-constexpr u32 CT_EMPTY = 0xffffffffu;
+// blocks per SM (launch bound: registers) for table shape HBITS
+template <int HBITS> constexpr int ct_blocks() { return HBITS == 4 ? 8 : (HBITS == 6 ? 2 : 5); }
 
-// Table shapes, smallest first.  The template argument is the number of hash bits, except 15 = the
-// 5-bit table with 16 instead of 24 accumulators: a P1 tetrahedral mesh has at most 15 rows per column,
-// and the smaller accumulator array lets 5 instead of 4 blocks share an SM.
-//   shape  4: 16 slots / 12 accumulators     shape 15: 32 / 16     shape 5: 32 / 24     shape 6: 64 / 32
-template <int HBITS> struct CtShape
-{
-    static constexpr int HB = HBITS == 15 ? 5 : HBITS;
-    static constexpr int H = 1 << HB;
-    static constexpr int D = HBITS == 6 ? 32 : (HBITS == 5 ? 24 : (HBITS == 15 ? 16 : 12));
-    static constexpr int kBlocks = HBITS == 4 ? 8 : (HBITS == 6 ? 2 : 5); // launch bound (registers)
-    // table words + accumulators + row of every accumulator (first-appearance order)
-    static constexpr size_t kBytesPerWarp = 32 * (sizeof(u32) * H + (sizeof(double) + sizeof(u32)) * D);
-};
-
-// Folds the records [cstart, cend) of one column.  Returns the number of existing entries j, their
-// (row << HBITS | accumulator) words sorted in key[0 .. j), or -1 if the table is too small.
-// d_out = distinct rows seen.
+// Folds the records [cstart, cend) of one column into f (f.ovf: the table is too small).  The entries of the
+// resident CSC are the first records of their column (stable sort or grouping) and have distinct rows: they
+// seed in a loop of their own, so that the walk below inlines ThreadFold::apply alone (fdrand 200^3, B200 at 1000 W:
+// 1.26 -> 1.15 ms for the fold kernel); the walk then reads the first staged record once more.
 template <int HBITS>
-__device__ __forceinline__ int ct_fold_column(const Rec *__restrict__ sorted, u32 cstart, u32 cend, int low,
-                                              u32 rowmask, u32 *key, double *acc, u32 *rows, u32 &d_out)
+__device__ __forceinline__ void ct_fold_column(const Rec *__restrict__ sorted, u32 cstart, u32 cend, int low,
+                                               u32 rowmask, ThreadFold<HBITS, false> &f)
 {
-    constexpr int H = CtShape<HBITS>::H;
-    constexpr int HB = CtShape<HBITS>::HB;
-    constexpr u32 D = CtShape<HBITS>::D;
-#pragma unroll
-    for (int s = 0; s < H; ++s)
-        key[s * 32] = CT_EMPTY;
-
-    u32 d = 0;       // accumulators in use
-    u32 pending = 0; // of which not (yet) existing: only updateindex! of a zero touched them
-    u64 exmask = 0;  // accumulator i holds an existing entry
-    bool ovf = false;
-    auto apply = [&](const Rec &r) {
-        const u32 row = (u32)(r.key >> low) & rowmask;
-        const double v = r.val;
-        u32 s = (row * 0x9E3779B1u) >> (32 - HB);
-        for (;;)
-        {
-            const u32 kk = key[s * 32];
-            const u32 x = kk ^ (row << HB);
-            if (x < D)
-            { // same row (an empty slot reads as index H-1 >= D): x is the accumulator
-                acc[x * 32] = acc[x * 32] + v;
-                if (pending)
-                {
-                    const u32 fl = (u32)r.key & 3u;
-                    if (!((exmask >> x) & 1ull) && ((fl != FL_UPDATE) | (v != 0.0)))
-                    {
-                        exmask |= 1ull << x;
-                        --pending;
-                    }
-                }
-                return;
-            }
-            if (kk == CT_EMPTY)
-            {
-                if (d >= D)
-                {
-                    ovf = true;
-                    return;
-                }
-                const u32 fl = (u32)r.key & 3u;
-                key[s * 32] = (row << HB) | d;
-                rows[d * 32] = row;
-                // a run starts from +0.0 (sparsematrixlnk.jl:225) unless the resident CSC value
-                // seeds it (extendable.jl:165-166); updateindex! of a zero creates nothing (:212,223)
-                acc[d * 32] = (fl == FL_OLD) ? v : 0.0 + v;
-                if ((fl != FL_UPDATE) | (v != 0.0))
-                    exmask |= 1ull << d;
-                else
-                    ++pending;
-                ++d;
-                return;
-            }
-            s = (s + 1) & (H - 1);
-        }
-    };
-
+    f.init();
+    u32 p = cstart;
+    for (; p < cend && !f.ovf; ++p)
+    {
+        const Rec r = sorted[p];
+        if (((u32)r.key & 3u) != FL_OLD)
+            break;
+        f.seed((u32)(r.key >> low) & rowmask, r.val);
+    }
+    auto fold = [&](const Rec &r) { f.apply((u32)(r.key >> low) & rowmask, r.val, (u32)r.key & 3u); };
     // A lane streams its own column: every load instruction of the warp touches 32 different
     // lines, so the L1 sees one request per lane.  256-bit loads (two records per request, 32-byte
     // aligned: the records of an odd start and an odd end go alone) halve that.
-    u32 p = cstart;
     if ((p & 1u) && p < cend)
-        apply(sorted[p++]);
+        fold(sorted[p++]);
     const Rec *col = sorted + p;
     const u32 npair = (cend - p) >> 1;
     const u32 nfull = npair / CT_U;
@@ -723,7 +658,7 @@ __device__ __forceinline__ int ct_fold_column(const Rec *__restrict__ sorted, u3
             nxt[i] = ld_pair_stream(col + 2 * i);
     }
     u32 g = 0;
-    for (; g < nfull && !ovf; ++g)
+    for (; g < nfull && !f.ovf; ++g)
     {
         RecPair cur[CT_U];
 #pragma unroll
@@ -738,57 +673,27 @@ __device__ __forceinline__ int ct_fold_column(const Rec *__restrict__ sorted, u3
 #pragma unroll
         for (int i = 0; i < CT_U; ++i)
         {
-            if (!ovf)
-                apply(cur[i].a);
-            if (!ovf)
-                apply(cur[i].b);
+            if (!f.ovf)
+                fold(cur[i].a);
+            if (!f.ovf)
+                fold(cur[i].b);
         }
     }
-    for (u32 q = p + 2 * nfull * CT_U; q < cend && !ovf; ++q)
-        apply(sorted[q]);
-    d_out = ovf ? D + 1 : d;
-    if (ovf)
-        return -1;
-    // ---- existing entries as (row << HBITS | accumulator) words, insertion-sorted by row into the
-    // (no longer needed) table.  They are taken in order of first appearance, which an assembly
-    // stream visits nearly in row order: few shifts (src/matrix/sparsematrixlnk.jl:339 sorts here too).
-    u32 j = 0;
-    for (u32 i = 0; i < d; ++i)
-    {
-        if (!((exmask >> i) & 1ull))
-            continue;
-        const u32 kk = (rows[i * 32] << HB) | i;
-        u32 q = j;
-        while (q > 0)
-        {
-            const u32 prev = key[(q - 1) * 32];
-            if (prev < kk)
-                break;
-            key[q * 32] = prev;
-            --q;
-        }
-        key[q * 32] = kk;
-        ++j;
-    }
-    return (int)j;
+    for (u32 q = p + 2 * nfull * CT_U; q < cend && !f.ovf; ++q)
+        fold(sorted[q]);
 }
 
 template <int HBITS, bool LIST>
-__global__ void __launch_bounds__(CT_WARPS * 32, CtShape<HBITS>::kBlocks)
+__global__ void __launch_bounds__(CT_WARPS * 32, ct_blocks<HBITS>())
 colthread_kernel(const Rec *__restrict__ sorted, int low, int rowbits, u32 maxlen, const u32 *__restrict__ nzcol,
                  const u32 *__restrict__ nzstart, const u64 *__restrict__ totals, Rec *__restrict__ tmp,
                  u32 *__restrict__ colcount, const u32 *__restrict__ src, const u32 *__restrict__ src_count,
                  u32 *__restrict__ next, u32 *__restrict__ next_count, u32 *__restrict__ longlist,
                  u32 *__restrict__ long_count, u32 *__restrict__ maxd)
 {
-    constexpr int H = CtShape<HBITS>::H;
-    constexpr u32 D = CtShape<HBITS>::D;
+    typedef ThreadFold<HBITS, false> Fold;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double *acc = reinterpret_cast<double *>(smem_raw) + warp * (D * 32) + lane; // accumulator i: acc[i * 32]
-    u32 *key = reinterpret_cast<u32 *>(smem_raw + (size_t)CT_WARPS * D * 32 * sizeof(double)) + warp * (H * 32) + lane;
-    u32 *rows = reinterpret_cast<u32 *>(smem_raw + (size_t)CT_WARPS * 32 * (D * sizeof(double) + H * sizeof(u32))) +
-                warp * (D * 32) + lane;
     const u32 rowmask = (1u << rowbits) - 1u;
     const u64 K = LIST ? (u64)*src_count : totals[1];
     const u64 step = LIST ? (u64)gridDim.x * (CT_WARPS * 32) : ~0ull >> 1;
@@ -801,38 +706,37 @@ colthread_kernel(const Rec *__restrict__ sorted, int low, int rowbits, u32 maxle
             longlist[atomicAdd(long_count, 1u)] = k;
             continue;
         }
-        u32 d;
-        const int j = ct_fold_column<HBITS>(sorted, cstart, cend, low, rowmask, key, acc, rows, d);
-        if (j < 0)
+        Fold f(smem_raw, CT_WARPS, warp, lane);
+        ct_fold_column<HBITS>(sorted, cstart, cend, low, rowmask, f);
+        if (f.ovf)
         {
             next[atomicAdd(next_count, 1u)] = k;
-            if (d > ld_relaxed_u32(maxd))
-                atomicMax(maxd, d);
+            if (Fold::D + 1 > ld_relaxed_u32(maxd))
+                atomicMax(maxd, Fold::D + 1);
             continue;
         }
+        const int j = f.finish();
         Rec *dst = tmp + cstart;
         for (int e = 0; e < j; ++e)
         {
-            const u32 pk = key[e * 32];
+            const u32 pk = f.key[e * 32];
             Rec o;
-            o.key = (u64)(pk >> CtShape<HBITS>::HB);
-            o.val = acc[(pk & (H - 1)) * 32];
+            o.key = (u64)(pk >> Fold::HB);
+            o.val = f.acc[(pk & (Fold::H - 1)) * 32];
             st_rec(dst + e, o);
         }
         colcount[nzcol[k]] = (u32)j;
-        if (d > ld_relaxed_u32(maxd))
-            atomicMax(maxd, d);
+        if (f.d > ld_relaxed_u32(maxd))
+            atomicMax(maxd, f.d);
     }
 }
 
 // The same fold writing the final CSC in ONE pass: the entries of column k go to
-// rowval/nzval[sum of the entry counts of the columns before k ...], that sum coming from a block
-// scan plus a decoupled look-back over the block totals (blocks are dispatched in index order).
+// rowval/nzval[sum of the entry counts of the columns before k ...] (column_offset).
 // A column that needs another table size or the warp kernel raises *d_redo; the caller then runs
 // the parking path (colthread_kernel + compact) instead.
-
 template <int HBITS, typename Ti>
-__global__ void __launch_bounds__(CT_WARPS * 32, CtShape<HBITS>::kBlocks)
+__global__ void __launch_bounds__(CT_WARPS * 32, ct_blocks<HBITS>())
 colthread_direct_kernel(const Rec *__restrict__ sorted, int low, int rowbits, u32 maxlen,
                         const u32 *__restrict__ nzcol, const u32 *__restrict__ nzstart,
                         const u64 *__restrict__ totals, i64 ncols, Ti base, Ti *__restrict__ rowval,
@@ -840,115 +744,42 @@ colthread_direct_kernel(const Rec *__restrict__ sorted, int low, int rowbits, u3
                         u32 *__restrict__ ticket, u64 *__restrict__ d_nnz, u32 *__restrict__ d_redo,
                         u32 *__restrict__ maxd)
 {
-    constexpr int H = CtShape<HBITS>::H;
-    constexpr u32 D = CtShape<HBITS>::D;
-    constexpr u32 full = 0xffffffffu;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ u32 s_wsum[CT_WARPS];
     __shared__ u64 s_prefix;
     __shared__ u32 s_bid;
-    // blocks take their columns in the order they START (ticket), so a block only ever waits for
-    // blocks that are already running: the look-back cannot starve whatever the dispatch order
+    // the look-back of column_offset needs the blocks to take their columns in the order they start
     if (threadIdx.x == 0)
         s_bid = atomicAdd(ticket, 1u);
     __syncthreads();
     const u32 bid = s_bid;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double *acc = reinterpret_cast<double *>(smem_raw) + warp * (D * 32) + lane;
-    u32 *key = reinterpret_cast<u32 *>(smem_raw + (size_t)CT_WARPS * D * 32 * sizeof(double)) + warp * (H * 32) + lane;
-    u32 *rows = reinterpret_cast<u32 *>(smem_raw + (size_t)CT_WARPS * 32 * (D * sizeof(double) + H * sizeof(u32))) +
-                warp * (D * 32) + lane;
+    ThreadFold<HBITS, false> f(smem_raw, CT_WARPS, warp, lane);
     const u32 rowmask = (1u << rowbits) - 1u;
     const u64 K = totals[1];
     const u64 k = (u64)bid * (CT_WARPS * 32) + threadIdx.x;
     int j = 0;
-    u32 cstart = 0;
     if (k < K && ld_relaxed_u32(d_redo) == 0u)
     {
-        cstart = nzstart[k];
-        const u32 cend = nzstart[k + 1];
+        const u32 cstart = nzstart[k], cend = nzstart[k + 1];
         if (cend - cstart > maxlen)
             atomicOr(d_redo, 2u);
         else
         {
-            u32 d;
-            j = ct_fold_column<HBITS>(sorted, cstart, cend, low, rowmask, key, acc, rows, d);
-            if (j < 0)
-            { // bit 2: not even the largest table takes this column
+            ct_fold_column<HBITS>(sorted, cstart, cend, low, rowmask, f);
+            const u32 d = f.ovf ? f.D + 1 : f.d;
+            if (f.ovf) // bit 2: not even the largest table takes this column
                 atomicOr(d_redo, HBITS == 6 ? 5u : 1u);
-                j = 0;
-            }
+            else
+                j = f.finish();
             if (d > ld_relaxed_u32(maxd))
                 atomicMax(maxd, d);
         }
     }
-    // ---- entries before this column: warp scan, block scan, look-back over the blocks
-    u32 incl = (u32)j;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1)
-    {
-        const u32 t = __shfl_up_sync(full, incl, o);
-        if (lane >= o)
-            incl += t;
-    }
-    if (lane == 31)
-        s_wsum[warp] = incl;
-    __syncthreads();
-    u32 wpre = 0, btotal = 0;
-#pragma unroll
-    for (int w = 0; w < CT_WARPS; ++w)
-    {
-        const u32 c = s_wsum[w];
-        if (w < warp)
-            wpre += c;
-        btotal += c;
-    }
-    if (warp == 0)
-    {
-        const u64 prefix = warp_lookback(status, bid, (u64)btotal, lane);
-        if (lane == 0)
-            s_prefix = prefix;
-    }
-    __syncthreads();
+    const u64 o0 = column_offset<CT_WARPS>(j, status, bid, s_wsum, &s_prefix, lane, warp);
     if (k >= K)
         return;
-    const u64 o0 = s_prefix + wpre + (incl - (u32)j);
-    // 256-bit stores where the destination is 32-byte aligned (rowval and nzval separately: their
-    // bases differ): a lane writes its own run, so every store instruction costs one request per lane
-    {
-        Ti *rv = rowval + o0;
-        auto row_at = [&](int e) { return (Ti)(key[e * 32] >> CtShape<HBITS>::HB) + base; };
-        constexpr int V = 32 / (int)sizeof(Ti);
-        int e = 0;
-        for (; e < j && (reinterpret_cast<uintptr_t>(rv + e) & 31u); ++e)
-            rv[e] = row_at(e);
-        for (; e + V <= j; e += V)
-        {
-            if (sizeof(Ti) == 8)
-                st_v4_u64(rv + e, (u64)row_at(e), (u64)row_at(e + 1), (u64)row_at(e + 2), (u64)row_at(e + 3));
-            else
-            {
-                const u64 w0 = (u64)(u32)row_at(e) | ((u64)(u32)row_at(e + 1) << 32);
-                const u64 w1 = (u64)(u32)row_at(e + 2) | ((u64)(u32)row_at(e + 3) << 32);
-                const u64 w2 = (u64)(u32)row_at(e + 4) | ((u64)(u32)row_at(e + 5) << 32);
-                const u64 w3 = (u64)(u32)row_at(e + 6) | ((u64)(u32)row_at(e + 7) << 32);
-                st_v4_u64(rv + e, w0, w1, w2, w3);
-            }
-        }
-        for (; e < j; ++e)
-            rv[e] = row_at(e);
-    }
-    {
-        double *nv = nzval + o0;
-        auto val_at = [&](int e) { return (u64)__double_as_longlong(acc[(key[e * 32] & (H - 1)) * 32]); };
-        int e = 0;
-        for (; e < j && (reinterpret_cast<uintptr_t>(nv + e) & 31u); ++e)
-            nv[e] = __longlong_as_double((long long)val_at(e));
-        for (; e + 4 <= j; e += 4)
-            st_v4_u64(nv + e, val_at(e), val_at(e + 1), val_at(e + 2), val_at(e + 3));
-        for (; e < j; ++e)
-            nv[e] = __longlong_as_double((long long)val_at(e));
-    }
+    f.store(j, base, rowval + o0, nzval + o0);
     // colptr of this column and of the empty columns right before it
     const i64 c1 = (i64)nzcol[k];
     const i64 c0 = k ? (i64)nzcol[k - 1] + 1 : 0;
@@ -1107,7 +938,7 @@ struct CtArgs
 };
 template <int HBITS, bool LIST> void launch_colthread_t(cudaStream_t stream, unsigned blocks, const CtArgs &a)
 {
-    constexpr size_t smem = CT_WARPS * CtShape<HBITS>::kBytesPerWarp;
+    constexpr size_t smem = CT_WARPS * FoldShape<HBITS>::kBytesPerWarp;
     static FuncAttrOnce once;
     once.set(colthread_kernel<HBITS, LIST>, (int)smem, true);
     colthread_kernel<HBITS, LIST><<<blocks, CT_WARPS * 32, smem, stream>>>(
@@ -1209,7 +1040,7 @@ void launch_direct_t(cudaStream_t stream, unsigned blocks, const Rec *sorted, in
                      const u32 *nzcol, const u32 *nzstart, const u64 *totals, i64 ncols, i64 base, void *rowval,
                      double *nzval, void *colptr, u64 *status, u32 *ticket, u64 *d_nnz, u32 *d_redo, u32 *maxd)
 {
-    constexpr size_t smem = CT_WARPS * CtShape<HBITS>::kBytesPerWarp;
+    constexpr size_t smem = CT_WARPS * FoldShape<HBITS>::kBytesPerWarp;
     static FuncAttrOnce once;
     once.set(colthread_direct_kernel<HBITS, Ti>, (int)smem, true);
     colthread_direct_kernel<HBITS, Ti><<<blocks, CT_WARPS * 32, smem, stream>>>(
@@ -1261,9 +1092,9 @@ void colfold_direct(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
     if (timer)
         timer->begin(stream);
     const u64 avg = nrec / std::max<u64>(1, kmax);
-    const int level = hint_maxd ? (hint_maxd <= 12 ? 0 : (hint_maxd <= 24 ? 1 : 2)) : (avg < 14 ? 0 : (avg < 40 ? 1 : 2));
-    // 13..16 distinct rows in the previous flush (P1 FEM: 15): the 32-slot table with 16 accumulators
-    const bool slim = level == 1 && hint_maxd != 0 && hint_maxd <= 16;
+    // table shape (level 0..3 = shapes 4, 15, 5, 6): what the previous flush of this handle needed, else the mean
+    // column length
+    const int level = hint_maxd ? fold_level_for(hint_maxd) : (avg < 14 ? 0 : (avg < 40 ? 2 : 3));
     const u32 maxlen = (u32)std::max<u64>(256, 6 * avg);
 #define XSB_DIRECT(HB, TI)                                                                                              \
     launch_direct_t<HB, TI>(stream, blocks, sorted, L.low, L.rowbits, maxlen, nzcol, nzstart, totals, ncols, base,      \
@@ -1272,9 +1103,9 @@ void colfold_direct(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
     {
         if (level == 0)
             XSB_DIRECT(4, int64_t);
-        else if (slim)
-            XSB_DIRECT(15, int64_t);
         else if (level == 1)
+            XSB_DIRECT(15, int64_t);
+        else if (level == 2)
             XSB_DIRECT(5, int64_t);
         else
             XSB_DIRECT(6, int64_t);
@@ -1283,9 +1114,9 @@ void colfold_direct(cudaStream_t stream, const Rec *sorted, u64 nrec, KeyLayout 
     {
         if (level == 0)
             XSB_DIRECT(4, int32_t);
-        else if (slim)
-            XSB_DIRECT(15, int32_t);
         else if (level == 1)
+            XSB_DIRECT(15, int32_t);
+        else if (level == 2)
             XSB_DIRECT(5, int32_t);
         else
             XSB_DIRECT(6, int32_t);

@@ -7,6 +7,7 @@
 // Reference counterpart: Base.:+(lnk,csc) src/matrix/sparsematrixlnk.jl:294-383 (gather,
 // sort, 3-way merge per column) and the accumulate-on-insert of :210-253; multi-partition
 // semantics of Base.sum(Vector{SparseMatrixDILNKC},csc) src/matrix/sparsematrixdilnkc.jl:397-435.
+#include "xsb_fold.cuh"
 #include "xsb_internal.h"
 
 namespace xsb {
@@ -63,94 +64,6 @@ constexpr int RD_OVER = 64;
 constexpr u64 RS_LOCAL = 1ull << 62;
 constexpr u64 RS_INCL = 2ull << 62;
 constexpr u64 RS_VALUE = (1ull << 62) - 1ull;
-
-// Insertion-order fold of one run of equal (col,row): the semantics of the three
-// insert flavours (sparsematrixlnk.jl:178-253) behind the CSC-hit router
-// (extendable.jl:159-218), per partition buffer, then partitions summed in tid
-// order with the first one copied (sparse! combine, sparsematrixdilnkc.jl:416-432).
-struct RunFold
-{
-    bool seeded = false, has_old = false, exists = false, pexists = false;
-    double old = 0.0, acc = 0.0, pacc = 0.0;
-    u32 ptid = 0xffffffffu;
-
-    __device__ __forceinline__ void commit()
-    {
-        if (pexists)
-        {
-            if (exists)
-                acc = acc + pacc;
-            else
-            {
-                acc = pacc;
-                exists = true;
-            }
-            pexists = false;
-        }
-    }
-    __device__ __forceinline__ void apply(u32 fl, u32 tid, double v, int combine)
-    {
-        if (fl == FL_OLD)
-        {
-            if (combine == 0)
-            {
-                seeded = true;
-                exists = true;
-                acc = v;
-            }
-            else
-            {
-                has_old = true;
-                old = v;
-            }
-            return;
-        }
-        if (seeded)
-        { // entry already in the CSC: in-place op, extendable.jl:164-166 / :210-212
-            acc = (fl == FL_ASSIGN) ? v : acc + v;
-            return;
-        }
-        if (tid != ptid)
-        {
-            commit();
-            ptid = tid;
-        }
-        if (fl == FL_RAW)
-        {
-            pacc = pexists ? pacc + v : 0.0 + v;
-            pexists = true;
-        }
-        else if (fl == FL_UPDATE)
-        {
-            if (pexists)
-                pacc = pacc + v;
-            else if (v != 0.0)
-            {
-                pexists = true;
-                pacc = 0.0 + v;
-            }
-        }
-        else
-        { // FL_ASSIGN
-            if (pexists)
-                pacc = v;
-            else if (v != 0.0)
-            {
-                pexists = true;
-                pacc = v;
-            }
-        }
-    }
-    __device__ __forceinline__ void finish()
-    {
-        commit();
-        if (has_old)
-        { // csc.nzval + lnk.nzval, sparsematrixlnk.jl:363
-            acc = exists ? old + acc : old;
-            exists = true;
-        }
-    }
-};
 
 // Order-preserving compaction ranks for flags laid out as (step i, thread): returns the
 // exclusive rank of every set flag and the total.  s_cnt/s_off hold RD_IPT*RD_WARPS words.

@@ -197,7 +197,6 @@ void chunk_sort(cudaStream_t stream, Rec *buf, u64 r0, u64 r1, const RunTarget &
 size_t runs_workspace_bytes(u64 npairs, i64 ncols);
 void runs_bucket(cudaStream_t stream, const RunTarget &rt, u32 nchunks, u32 npairs, i64 ncols, const KeyLayout &L,
                  RunRegions reg, void *workspace, LaunchCounter &lc);
-int runs_level_for(u32 maxd);
 void runs_fold(cudaStream_t stream, const Rec *buf, const KeyLayout &L, i64 ncols, int idx64, int base, const CscView &old,
                void *workspace, u32 npairs, int level, u32 maxlen, void *rowval_out, double *nzval_out, void *colptr_out,
                u64 *d_nnz, u32 *d_redo, u32 *d_maxd, bool first_try, bool has_assign, LaunchCounter &lc);

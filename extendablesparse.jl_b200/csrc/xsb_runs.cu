@@ -22,6 +22,7 @@
 // HBM traffic of a flush: 16 B per staged record (read once) + the old CSC read once + the new CSC
 // written once + 20 B per (chunk, column) pair -- SURVEY.md 8(d)'s algorithmic bytes plus the pairs.
 #include "xsb_chunk.cuh"
+#include "xsb_fold.cuh"
 #include "xsb_internal.h"
 
 namespace xsb {
@@ -239,187 +240,38 @@ run_bucket_kernel(const uint2 *__restrict__ chunkinfo, const u32 *__restrict__ c
 // ------------------------------------------------------------------------
 // one THREAD per column: merge the column of the resident CSC with the column's runs
 // ------------------------------------------------------------------------
-constexpr u32 RF_EMPTY = 0xffffffffu;
-
-// Table shapes, smallest first.  The template argument is the number of hash bits, except 15 = the
-// 5-bit table with 16 instead of 24 accumulators (a P1 tetrahedral mesh has at most 15 rows per column).
-//   shape  4: 16 slots / 12 accumulators     shape 15: 32 / 16     shape 5: 32 / 24     shape 6: 64 / 32
-template <int HBITS> struct RfShape
+// Launch shape of the merge kernel for table shape HBITS (xsb_fold.cuh): warps per block; blocks per SM that shared
+// memory and the register file allow.  The largest shape takes 544 B of shared memory per thread: one-warp blocks
+// fit 12 warps per SM where four-warp blocks fit 8 (measured on the block reaction-diffusion system: 2.65 -> 2.34 ms;
+// the small shapes lose with tiny blocks).  The 32/16 shape takes 272 B per thread: five blocks of five warps = 25
+// warps per SM (four-warp blocks: 24).
+template <int HBITS> struct RfLaunch
 {
-    static constexpr int HB = HBITS == 15 ? 5 : HBITS;
-    static constexpr int H = 1 << HB;
-    static constexpr int D = HBITS == 6 ? 32 : (HBITS == 5 ? 24 : (HBITS == 15 ? 16 : 12));
-    // warps per block; blocks per SM that shared memory and the register file allow.  The largest shape takes
-    // 544 B of shared memory per thread: one-warp blocks fit 12 warps per SM where four-warp blocks fit 8
-    // (measured on the block reaction-diffusion system: 2.65 -> 2.34 ms; the small shapes lose with tiny blocks).
-    // The 32/16 shape takes 272 B per thread: five blocks of five warps = 25 warps per SM (four-warp blocks: 24).
     static constexpr int kWarps = HBITS == 6 ? 1 : (HBITS == 15 ? 5 : 4);
     static constexpr int kBlocks = HBITS == 4 ? 8 : (HBITS == 6 ? 12 : 5);
-    static constexpr size_t kBytesPerWarp = 32 * (sizeof(u32) * H + (sizeof(double) + 1) * D);
-};
-
-// The fold state of one column.  A table slot holds (row << HB | accumulator index); accumulators are
-// numbered in order of first appearance.  Flavour semantics (single partition): src/matrix/sparsematrixlnk.jl
-// :178-253 behind the CSC-hit router src/matrix/extendable.jl:159-218.
-template <int HBITS, bool ASSIGN> struct ThreadFold
-{
-    static constexpr int H = RfShape<HBITS>::H;
-    static constexpr int HB = RfShape<HBITS>::HB;
-    static constexpr u32 D = RfShape<HBITS>::D;
-    u32 *key;    // [slot * 32]
-    double *acc; // [i * 32]
-    unsigned char *ord; // [i * 32]: table slot of accumulator i (its row = key >> HB)
-    u32 d = 0;       // accumulators in use
-    u32 pending = 0; // of which not (yet) existing: only updateindex! / setindex! of a zero touched them
-    u32 exmask = 0;  // accumulator i holds an existing entry (D <= 32)
-    bool ovf = false;
-
-    __device__ __forceinline__ void init()
-    {
-#pragma unroll
-        for (int s = 0; s < H; ++s)
-            key[s * 32] = RF_EMPTY;
-    }
-    // slot of `row`: x = its accumulator, or x >= D with s the empty slot where the probe ended (an empty slot reads
-    // as index H-1 >= D).  One loop with one exit: the lanes of a warp leave it together before they touch an accumulator.
-    __device__ __forceinline__ u32 find(u32 row, u32 &s) const
-    {
-        const u32 tag = row << HB;
-        s = (row * 0x9E3779B1u) >> (32 - HB);
-        for (;;)
-        {
-            const u32 kk = key[s * 32];
-            const u32 x = kk ^ tag;
-            if (x < D || kk == RF_EMPTY)
-                return x;
-            s = (s + 1) & (H - 1);
-        }
-    }
-    // an entry of the resident CSC seeds its accumulator (extendable.jl:164-166); old rows are distinct
-    __device__ __forceinline__ void seed(u32 row, double v)
-    {
-        u32 s;
-        find(row, s);
-        if (d >= D)
-        {
-            ovf = true;
-            return;
-        }
-        key[s * 32] = (row << HB) | d;
-        ord[d * 32] = (unsigned char)s;
-        acc[d * 32] = v;
-        exmask |= 1u << d;
-        ++d;
-    }
-    // one staged insertion (update / rawupdate / assign flavour)
-    __device__ __forceinline__ void apply(u32 row, double v, u32 fl)
-    {
-        u32 s;
-        u32 x = find(row, s);
-        if (x >= D)
-        { // first insertion of this row: a new accumulator at +0.0 (sparsematrixlnk.jl:225), not an entry yet
-            if (d >= D)
-            {
-                ovf = true;
-                return;
-            }
-            x = d++;
-            key[s * 32] = (row << HB) | x;
-            ord[x * 32] = (unsigned char)s;
-            acc[x * 32] = 0.0;
-            ++pending;
-        }
-        if (ASSIGN && fl == FL_ASSIGN)
-        { // A[i,j] = v: overwrites; creates only if v != 0 (sparsematrixlnk.jl:184-199)
-            const bool ex = (exmask >> x) & 1u;
-            if (ex | (v != 0.0))
-            {
-                acc[x * 32] = v;
-                if (!ex)
-                {
-                    exmask |= 1u << x;
-                    --pending;
-                }
-            }
-            return;
-        }
-        acc[x * 32] = acc[x * 32] + v;
-        if (pending)
-        { // rawupdateindex! always creates the entry, updateindex! only with v != 0 (sparsematrixlnk.jl:212,223,239)
-            if (!((exmask >> x) & 1u) && ((fl != FL_UPDATE) | (v != 0.0)))
-            {
-                exmask |= 1u << x;
-                --pending;
-            }
-        }
-    }
-    // existing entries as (row << HB | accumulator) words, sorted by row into key[0 .. j).  All words are read into
-    // registers first (the table is overwritten), ordered there by a bitonic network -- no branch, no
-    // memory traffic, the same instruction stream for every lane whatever its column looks like -- and written back.
-    __device__ __forceinline__ int finish()
-    {
-        constexpr int N = D <= 16 ? 16 : 32;
-        u32 a[N];
-#pragma unroll
-        for (int i = 0; i < N; ++i)
-        {
-            a[i] = 0xffffffffu;
-            if ((u32)i < D && (u32)i < d && ((exmask >> i) & 1u))
-                a[i] = key[(u32)ord[i * 32] * 32]; // (row << HB) | i
-        }
-#pragma unroll
-        for (int k = 2; k <= N; k <<= 1) // bitonic network: every index below is a compile-time constant
-#pragma unroll
-            for (int jj = k >> 1; jj > 0; jj >>= 1)
-#pragma unroll
-                for (int i = 0; i < N; ++i)
-                {
-                    const int l = i ^ jj;
-                    if (l > i)
-                    {
-                        const u32 lo_ = min(a[i], a[l]), hi_ = max(a[i], a[l]);
-                        a[i] = (i & k) == 0 ? lo_ : hi_;
-                        a[l] = (i & k) == 0 ? hi_ : lo_;
-                    }
-                }
-        const int j = __popc(exmask);
-#pragma unroll
-        for (int i = 0; i < N; ++i)
-            if (i < H && i < j)
-                key[i * 32] = a[i];
-        return j;
-    }
 };
 
 template <int HBITS, typename Ti, bool ASSIGN>
-__global__ void __launch_bounds__(RfShape<HBITS>::kWarps * 32, RfShape<HBITS>::kBlocks)
+__global__ void __launch_bounds__(RfLaunch<HBITS>::kWarps * 32, RfLaunch<HBITS>::kBlocks)
 runfold_kernel(const Rec *__restrict__ buf, int low, int rowbits, u32 maxlen, const u32 *__restrict__ pstart,
                u64 *__restrict__ bucket, const Ti *__restrict__ old_colptr, const Ti *__restrict__ old_rowval,
                const double *__restrict__ old_nzval, i64 ncols, Ti base, Ti *__restrict__ rowval,
                double *__restrict__ nzval, Ti *__restrict__ colptr, u64 *__restrict__ status, u32 *__restrict__ ticket,
                u64 *__restrict__ d_nnz, u32 *__restrict__ d_redo, u32 *__restrict__ maxd)
 {
-    typedef RfShape<HBITS> Shape;
-    constexpr int RF_WARPS = Shape::kWarps;
-    constexpr int H = Shape::H;
-    constexpr int HB = Shape::HB;
-    constexpr u32 D = Shape::D;
-    constexpr u32 full = 0xffffffffu;
+    constexpr int RF_WARPS = RfLaunch<HBITS>::kWarps;
+    constexpr u32 D = FoldShape<HBITS>::D;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     __shared__ u32 s_wsum[RF_WARPS];
     __shared__ u64 s_prefix;
     __shared__ u32 s_bid;
-    // blocks take their columns in the order they START (ticket), so a block only ever waits for
-    // blocks that are already running: the look-back cannot starve whatever the dispatch order
+    // the look-back of column_offset needs the blocks to take their columns in the order they start
     if (threadIdx.x == 0)
         s_bid = atomicAdd(ticket, 1u);
     __syncthreads();
     const u32 bid = s_bid;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    ThreadFold<HBITS, ASSIGN> f;
-    f.acc = reinterpret_cast<double *>(smem_raw) + warp * (D * 32) + lane;
-    f.key = reinterpret_cast<u32 *>(smem_raw + (size_t)RF_WARPS * D * 32 * sizeof(double)) + warp * (H * 32) + lane;
-    f.ord = smem_raw + (size_t)RF_WARPS * 32 * (D * sizeof(double) + H * sizeof(u32)) + warp * (D * 32) + lane;
+    ThreadFold<HBITS, ASSIGN> f(smem_raw, RF_WARPS, warp, lane);
     const u32 rowmask = (1u << rowbits) - 1u;
     const i64 k = (i64)bid * (RF_WARPS * 32) + threadIdx.x;
     int j = 0;           // entries of this column in the new matrix
@@ -602,37 +454,9 @@ runfold_kernel(const Rec *__restrict__ buf, int low, int rowbits, u32 maxlen, co
             }
         }
     }
-    // ---- entries before this column: warp scan, block scan, look-back over the blocks
-    u32 incl = (u32)j;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1)
-    {
-        const u32 t = __shfl_up_sync(full, incl, o);
-        if (lane >= o)
-            incl += t;
-    }
-    if (lane == 31)
-        s_wsum[warp] = incl;
-    __syncthreads();
-    u32 wpre = 0, btotal = 0;
-#pragma unroll
-    for (int w = 0; w < RF_WARPS; ++w)
-    {
-        const u32 c = s_wsum[w];
-        if (w < warp)
-            wpre += c;
-        btotal += c;
-    }
-    if (warp == 0)
-    {
-        const u64 prefix = warp_lookback(status, bid, (u64)btotal, lane);
-        if (lane == 0)
-            s_prefix = prefix;
-    }
-    __syncthreads();
+    const u64 o0 = column_offset<RF_WARPS>(j, status, bid, s_wsum, &s_prefix, lane, warp);
     if (k >= ncols)
         return;
-    const u64 o0 = s_prefix + wpre + (incl - (u32)j);
     colptr[k] = (Ti)o0 + base;
     if (k == ncols - 1)
     {
@@ -652,42 +476,7 @@ runfold_kernel(const Rec *__restrict__ buf, int low, int rowbits, u32 maxlen, co
         }
         return;
     }
-    // 256-bit stores where the destination is 32-byte aligned (rowval and nzval separately: their
-    // bases differ): a lane writes its own run, so every store instruction costs one request per lane
-    {
-        Ti *rv = rowval + o0;
-        auto row_at = [&](int e) { return (Ti)(f.key[e * 32] >> HB) + base; };
-        constexpr int V = 32 / (int)sizeof(Ti);
-        int e = 0;
-        for (; e < j && (reinterpret_cast<uintptr_t>(rv + e) & 31u); ++e)
-            rv[e] = row_at(e);
-        for (; e + V <= j; e += V)
-        {
-            if (sizeof(Ti) == 8)
-                st_v4_u64(rv + e, (u64)row_at(e), (u64)row_at(e + 1), (u64)row_at(e + 2), (u64)row_at(e + 3));
-            else
-            {
-                const u64 w0 = (u64)(u32)row_at(e) | ((u64)(u32)row_at(e + 1) << 32);
-                const u64 w1 = (u64)(u32)row_at(e + 2) | ((u64)(u32)row_at(e + 3) << 32);
-                const u64 w2 = (u64)(u32)row_at(e + 4) | ((u64)(u32)row_at(e + 5) << 32);
-                const u64 w3 = (u64)(u32)row_at(e + 6) | ((u64)(u32)row_at(e + 7) << 32);
-                st_v4_u64(rv + e, w0, w1, w2, w3);
-            }
-        }
-        for (; e < j; ++e)
-            rv[e] = row_at(e);
-    }
-    {
-        double *nv = nzval + o0;
-        auto val_at = [&](int e) { return (u64)__double_as_longlong(f.acc[(f.key[e * 32] & (H - 1)) * 32]); };
-        int e = 0;
-        for (; e < j && (reinterpret_cast<uintptr_t>(nv + e) & 31u); ++e)
-            nv[e] = __longlong_as_double((long long)val_at(e));
-        for (; e + 4 <= j; e += 4)
-            st_v4_u64(nv + e, val_at(e), val_at(e + 1), val_at(e + 2), val_at(e + 3));
-        for (; e < j; ++e)
-            nv[e] = __longlong_as_double((long long)val_at(e));
-    }
+    f.store(j, base, rowval + o0, nzval + o0);
 }
 
 // ------------------------------------------------------------------------
@@ -811,8 +600,8 @@ void launch_runfold_t(cudaStream_t stream, unsigned blocks, const Rec *buf, int 
                       const u32 *pstart, u64 *bucket, const CscView &old, i64 ncols, i64 base, void *rowval, double *nzval,
                       void *colptr, u64 *status, u32 *ticket, u64 *d_nnz, u32 *d_redo, u32 *maxd)
 {
-    constexpr int RF_WARPS = RfShape<HBITS>::kWarps;
-    constexpr size_t smem = RF_WARPS * RfShape<HBITS>::kBytesPerWarp;
+    constexpr int RF_WARPS = RfLaunch<HBITS>::kWarps;
+    constexpr size_t smem = RF_WARPS * FoldShape<HBITS>::kBytesPerWarp;
     static FuncAttrOnce once;
     once.set(runfold_kernel<HBITS, Ti, ASSIGN>, (int)smem, true);
     const bool has_old = old.nnz > 0;
@@ -833,9 +622,9 @@ void runs_fold(cudaStream_t stream, const Rec *buf, const KeyLayout &L, i64 ncol
     u32 *pstart = reinterpret_cast<u32 *>(ws + l.off_pstart);
     u64 *bucket = reinterpret_cast<u64 *>(ws + l.off_bucket);
     u64 *status = reinterpret_cast<u64 *>(ws + l.off_fstatus);
-    const unsigned tpb = 32u * (unsigned)(level == 3 ? RfShape<6>::kWarps
-                                                      : (level == 2 ? RfShape<5>::kWarps
-                                                                    : (level == 1 ? RfShape<15>::kWarps : RfShape<4>::kWarps)));
+    const unsigned tpb = 32u * (unsigned)(level == 3 ? RfLaunch<6>::kWarps
+                                                      : (level == 2 ? RfLaunch<5>::kWarps
+                                                                    : (level == 1 ? RfLaunch<15>::kWarps : RfLaunch<4>::kWarps)));
     const unsigned blocks = (unsigned)(((u64)ncols + tpb - 1) / tpb);
     u32 *ticket = reinterpret_cast<u32 *>(status + blocks + 1);
     if (!first_try) // look-back words + ticket were cleared with the bucket workspace the first time
@@ -880,8 +669,5 @@ void runs_fold(cudaStream_t stream, const Rec *buf, const KeyLayout &L, i64 ncol
     lc.add();
     XSB_CUDA(cudaGetLastError());
 }
-
-// table shape for columns with at most `maxd` distinct rows
-int runs_level_for(u32 maxd) { return maxd <= 12 ? 0 : (maxd <= 16 ? 1 : (maxd <= 24 ? 2 : 3)); }
 
 } // namespace xsb

@@ -819,6 +819,30 @@ def test_hash_fold_groups_of_columns(xsb, oracle):
             h.flush()
             assert h.flush_stats()["column_path"] in ((2,) if grouping == xsb.capi.GROUPING_OFF else (2, 3, 4))
             assert_csc_equal(h.fetch_csc_numpy(), A.csc())
+    # plain adds (one partition, update / raw) take the thread-per-column fold: columns of exactly 12, 13, 16, 17,
+    # 24, 25, 32 and 33 distinct rows, the edges of its table shapes.  Alone, the second flush picks the shape from
+    # the first one's distinct rows; among many short columns the smallest shape comes first and hands on the rest.
+    edges = [12, 13, 16, 17, 24, 25, 32, 33]
+    for dist in [[d] * 40 for d in edges] + [edges * 5 + [2] * 600]:
+        ne = len(dist)
+        Je = np.repeat(np.arange(1, ne + 1), 3 * np.array(dist))
+        Ie = np.concatenate([np.tile(rng.choice(m, d, replace=False) + 1, 3) for d in dist])
+        Ve = rng.standard_normal(len(Je))
+        Ve[rng.random(len(Je)) < 0.1] = 0.0
+        perm = rng.permutation(len(Je))
+        Ie, Je, Ve = Ie[perm], Je[perm], Ve[perm]
+        A = oracle.OracleExt(m, ne)
+        h = xsb.Handle(m, ne)
+        h.set_grouping(xsb.capi.GROUPING_OFF)
+        for rnd in range(2):
+            for q, idx in enumerate(np.array_split(np.arange(len(Je)), 4)):
+                fl, ofl = ((xsb.UPDATE, oracle.UPDATE), (xsb.RAW, oracle.RAW))[q % 2]
+                A.insert_batch(Ie[idx], Je[idx], Ve[idx] * (rnd + 1), ofl)
+                h.insert_batch(Ie[idx], Je[idx], Ve[idx] * (rnd + 1), fl)
+            A.flush()
+            h.flush()
+            assert h.flush_stats()["column_path"] == 2
+            assert_csc_equal(h.fetch_csc_numpy(), A.csc())
 
 
 # ---------------------------------------------------------------- two-pass grouping by column
